@@ -6,7 +6,7 @@ the sm_100a step kernel through the C ABI (hlynr_step), actions resident in HBM.
 (desynchronised by a fused rollout) before the warm-up, so the timed ticks run at the steady-state rate of
 finished episodes and in-kernel auto-resets (`done_episodes_per_step`, `episode_stats`).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--envs-per-gpu 1048576]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--envs-per-gpu 1048576] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, envs sharded by global id, no
                                                            per-step communication; one NCCL all-reduce of the
                                                            episode-statistics block per rollout, inside the
@@ -304,12 +304,13 @@ def timed_ticks(ctx, sim, pool, K, W, collective=True, graph=False):
     t0 = time.perf_counter()
     e0.record()
     done = 0
+    last = None
     if sg is not None:
         while done + T <= K:
-            sg.replay()
+            last = sg.replay()
             done += T
     for k in range(done, K):
-        sim.step(pool[k % 4], want_terminal_obs=False)
+        last = sim.step(pool[k % 4], want_terminal_obs=False)
     t_issue = time.perf_counter() - t0
     stats_t = sim.stats_tensor()  # one stats all-reduce per rollout (NVLink); tiny, latency-bound
     if ctx.world > 1 and collective:
@@ -320,7 +321,24 @@ def timed_ticks(ctx, sim, pool, K, W, collective=True, graph=False):
     ms = e0.elapsed_time(e1)
     return {"ms": ms, "ms_max": ctx.max_over_ranks(ms) if collective else ms, "launches": sim.launch_count() - launches0,
             "stats": stats_t.cpu().numpy().tolist(), "window": (t0, t1), "host_issue_ms": t_issue * 1e3,
-            "graph_ticks": T if sg is not None else 0}
+            "graph_ticks": T if sg is not None else 0, "last_outputs": last}
+
+
+DUMP_MAX_ROWS = 1 << 18   # 2^18 envs x 124 B = 32.5 MB of .npy files
+
+
+def dump_outputs(out_dir, outputs, first_env):
+    """Writes what the last timed step returned to its caller (obs, reward, terminated, truncated of every env of this rank) as
+    float32 .npy files, plus the global env id of every row.  Above DUMP_MAX_ROWS envs, a fixed seeded sample of the rows
+    (the same rows in every run with the same --envs-per-gpu) keeps the files under 64 MB."""
+    obs, reward, terminated, truncated = (t.cpu().numpy() for t in outputs[:4])
+    n = obs.shape[0]
+    rows = np.arange(n) if n <= DUMP_MAX_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ROWS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "env_id.npy"), (rows + first_env).astype(np.float64))
 
 
 def config_line(ctx, workload, n, K, W, precision, peak):
@@ -380,7 +398,13 @@ def main():
     ap.add_argument("--rollout-steps", type=int, default=24, help="n_steps of the extra on-device PPO rollout-collection measurement (0 = skip)")
     ap.add_argument("--rollout-envs", type=int, default=131072)
     ap.add_argument("--post-steps", type=int, default=200, help="steps of the extra step + frame-stack/normalise measurement (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline's last timed step (rank 0) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none to write")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -404,6 +428,8 @@ def main():
     if rank == 0:
         sampler.start()
     head = timed_ticks(ctx, sim, pool, K, W)
+    if args.dump_outputs and rank == 0:   # before any further step overwrites the output buffers
+        dump_outputs(args.dump_outputs, head["last_outputs"], rank * n)
     total_ms = head["ms_max"]
     clock_windows, clock_note = [head["window"]], None
     if rank == 0 and sampler.proc and sampler.count_between(*head["window"]) < 3:

@@ -24,7 +24,10 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in DEPS)
 
 
-def build(force=False, verbose=False):
+def build(force=False, verbose=False, report=False):
+    """report=True (`python -m hlynr_intercept_b200.build --report`) rewrites csrc/ptxas_report.txt: registers / spills / smem
+    per kernel, kept in git.  Off by default: nvcc's output depends on where the checkout sits (anonymous-namespace kernel names
+    carry a hash of the source path), so an ordinary build that wrote it would modify a committed file."""
     if not force and not needs_build():
         return SO
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
@@ -32,12 +35,16 @@ def build(force=False, verbose=False):
     res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + res.stdout)
-    with open(os.path.join(HERE, "csrc", "ptxas_report.txt"), "w") as f:   # registers / spills / smem per kernel (kept in git)
-        f.write("".join(l for l in res.stdout.splitlines(True) if "Compile time" not in l))
+    if report:   # source paths relative to the checkout
+        out = res.stdout.replace(os.path.dirname(HERE) + os.sep, "")
+        with open(os.path.join(HERE, "csrc", "ptxas_report.txt"), "w") as f:
+            f.write("".join(l for l in out.splitlines(True) if "Compile time" not in l))
     if verbose:
         print(res.stdout)
     return SO
 
 
 if __name__ == "__main__":
-    build(force=True, verbose=True)
+    import sys
+
+    build(force=True, verbose=True, report="--report" in sys.argv[1:])
