@@ -47,6 +47,9 @@ HD double sub(double a, double b) { return __dsub_rn(a, b); }
 // motivated it (profiles/r02_b_fp64_*) shows 3729 instructions per env-step of 165 KB straight-line code with `no_instruction`
 // (instruction-cache misses) as the top stall reason.  Every divisor on the path is positive and finite (guards are at the call
 // sites, as in the reference).  -DHLYNR_F64_EXACT_DIV restores __ddiv_rn.
+// The final product is __dmul_rn like every operation of this section: a plain `*` may be contracted with an addition that follows
+// it into an FMA, and whether the compiler does so depends on the code around the call: with a plain `*` the FT_V2OFF and the
+// generic step kernels of this build left the missile state of cfg2 different in the last bits (tests/test_kernel_variants.py).
 HD double drcp(double b) {
     double r;
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(b));
@@ -58,7 +61,7 @@ HD double drcp(double b) {
 #ifdef HLYNR_F64_EXACT_DIV
 HD double dvd(double a, double b) { return __ddiv_rn(a, b); }
 #else
-HD double dvd(double a, double b) { return a * drcp(b); }
+HD double dvd(double a, double b) { return __dmul_rn(a, drcp(b)); }
 #endif
 #if defined(HLYNR_F64_EXACT_DIV) || defined(HLYNR_F64_EXACT_SQRT)
 HD double sqr(double a) { return __dsqrt_rn(a); }

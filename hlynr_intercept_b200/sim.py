@@ -111,7 +111,7 @@ class HlynrSim:
 
     def rollout(self, k_steps, actions=None, want_obs=True):
         """k fused ticks in one launch (state in registers).  actions: None = in-kernel random policy, or a float32
-        cuda tensor [k,N,6].  Returns (obs_after_last_tick, reward_sum[N], done_count[N])."""
+        cuda tensor [k,N,6].  Returns (obs_after_last_tick[N,obs_dim] or None, reward_sum[N], done_count[N])."""
         t = self._torch
         o = self._alloc_out()
         if not hasattr(self, "_rsum"):

@@ -274,7 +274,7 @@ int hlynr_set_done_list(hlynr_t* sim, HlynrDoneRecord* records_dev, int32_t* cou
 /* k fused ticks in ONE launch with the state held in registers between ticks.
  *   actions_dev  float[k,N,6] or NULL = in-kernel random actions U(-1,1)^6 from the Philox
  *                stream (synthetic random-policy rollouts)
- *   obs_dev      float[N,26]: observation after the last tick (or NULL)
+ *   obs_dev      float[N,obs_dim] (option "obs_dim", 26 by default): observation after the last tick (or NULL)
  *   reward_sum_dev float[N] or NULL: sum of the k rewards;  done_count_dev int32[N] or NULL */
 int hlynr_rollout(hlynr_t* sim, int k_steps, const float* actions_dev, float* obs_dev,
                   float* reward_sum_dev, int32_t* done_count_dev, void* stream);
