@@ -224,23 +224,33 @@ __device__ __forceinline__ uint32_t relu_bf16x2(uint64_t v) {   // {lo, hi} fp32
 
 // bias + LayerNorm + ReLU epilogue of one hidden layer: TMEM accumulators -> bf16 A operand of the next GEMM.
 // Two warps share a row quarter: warp w and w + 4 read TMEM lanes 32 * (w % 4) ..., each over half of the N columns.
-// The arithmetic runs on packed fp32 pairs (3.5 instead of 8.5 floating-point instructions per element over the two passes).
-// one 32-column chunk of pass 1: x = v + b, accumulate the sum and the sum of squares (packed fp32 pairs)
-__device__ __forceinline__ void stats_chunk(const uint32_t (&v)[32], const float4 (&b)[8], uint64_t& s2, uint64_t& ss2) {
+// The arithmetic runs on packed fp32 pairs (4 instead of 9.5 floating-point instructions per element over the two passes).
+// one 32-column chunk of pass 1: x = v + b - k with k the part's shift {-k, -k} = nk2, accumulate the sum and the sum of squares
+// (packed fp32 pairs).  The shift keeps the sums small when a row has a large common mean: E[x^2] - mean^2 in fp32 loses
+// (mean / std)^2 * 2^-24 of the variance, 20 % at mean / std = 1000.
+__device__ __forceinline__ void stats_chunk(const uint32_t (&v)[32], const float4 (&b)[8], uint64_t nk2, uint64_t& s2, uint64_t& ss2) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-        const uint64_t x0 = add2(pk2u(v[4 * j], v[4 * j + 1]), pk2(b[j].x, b[j].y)), x1 = add2(pk2u(v[4 * j + 2], v[4 * j + 3]), pk2(b[j].z, b[j].w));
+        const uint64_t x0 = add2(add2(pk2u(v[4 * j], v[4 * j + 1]), pk2(b[j].x, b[j].y)), nk2);
+        const uint64_t x1 = add2(add2(pk2u(v[4 * j + 2], v[4 * j + 3]), pk2(b[j].z, b[j].w)), nk2);
         s2 = add2(s2, add2(x0, x1));
         ss2 = fma2(x0, x0, fma2(x1, x1, ss2));
     }
 }
-__device__ __forceinline__ void stats_chunk16(const uint32_t (&v)[16], const float4 (&b)[4], uint64_t& s2, uint64_t& ss2) {
+__device__ __forceinline__ void stats_chunk16(const uint32_t (&v)[16], const float4 (&b)[4], uint64_t nk2, uint64_t& s2, uint64_t& ss2) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-        const uint64_t x0 = add2(pk2u(v[4 * j], v[4 * j + 1]), pk2(b[j].x, b[j].y)), x1 = add2(pk2u(v[4 * j + 2], v[4 * j + 3]), pk2(b[j].z, b[j].w));
+        const uint64_t x0 = add2(add2(pk2u(v[4 * j], v[4 * j + 1]), pk2(b[j].x, b[j].y)), nk2);
+        const uint64_t x1 = add2(add2(pk2u(v[4 * j + 2], v[4 * j + 3]), pk2(b[j].z, b[j].w)), nk2);
         s2 = add2(s2, add2(x0, x1));
         ss2 = fma2(x0, x0, fma2(x1, x1, ss2));
     }
+}
+// Chan's merge of two column parts of n columns each: (mean, M2 = sum of squared deviations from the mean).  Symmetric in a and b
+// up to exact operations, so every thread that merges the same two parts gets the same bits.
+__device__ __forceinline__ float2 chan_merge(float2 a, float2 b, float n) {
+    const float d = a.x - b.x;
+    return make_float2((a.x + b.x) * 0.5f, (a.y + b.y) + d * d * (0.5f * n));
 }
 // one 16-column chunk of pass 2: y = ((v + b) * rstd - mean * rstd) * gamma + beta, ReLU fused into the bf16 conversion, two
 // 16-byte chunks of the swizzled K-major A operand
@@ -260,7 +270,7 @@ __device__ __forceinline__ void norm_chunk(const uint32_t (&v)[16], const float4
 
 // bias + LayerNorm + ReLU epilogue of one hidden layer: TMEM accumulators -> bf16 A operand of the next GEMM.
 // Two warps share a row quarter: warp w and w + 4 read TMEM lanes 32 * (w % 4) ..., each over half of the N columns.
-// The arithmetic runs on packed fp32 pairs (3.5 instead of 8.5 floating-point instructions per element over the two passes), and
+// The arithmetic runs on packed fp32 pairs (4 instead of 9.5 floating-point instructions per element over the two passes), and
 // the TMEM loads are double-buffered in registers: the load of chunk i + 1 is in flight while chunk i is processed (a TMEM round
 // trip per chunk, exposed at 2 warps per scheduler, was most of the epilogue's time: profiles/r02_c_policy_phases.log).
 template <int N>
@@ -271,6 +281,8 @@ __device__ __forceinline__ void layer_epilogue(uint32_t lane_addr, uint32_t a_ba
     static_assert(HALF % 64 == 0, "two 32-column chunks per iteration");
     const int cbeg = half * HALF;
     uint64_t s2 = pk2(0.f, 0.f), ss2 = pk2(0.f, 0.f);
+    float k = 0.f;                    // the part's shift: its first column's v + b
+    uint64_t nk2 = pk2(0.f, 0.f);
     if constexpr (PARTS == 2) {
         uint32_t va[32], vb[32];
         tmem_ld32(lane_addr + (uint32_t)cbeg, va);
@@ -280,13 +292,14 @@ __device__ __forceinline__ void layer_epilogue(uint32_t lane_addr, uint32_t a_ba
 #pragma unroll
             for (int j = 0; j < 8; ++j) b[j] = __ldg(reinterpret_cast<const float4*>(bias + c0) + j);
             tmem_wait_ld32(va);
+            if (c0 == cbeg) { k = __uint_as_float(va[0]) + b[0].x; nk2 = pk2(-k, -k); }
             tmem_ld32(lane_addr + (uint32_t)(c0 + 32), vb);           // in flight while chunk A is summed
-            stats_chunk(va, b, s2, ss2);
+            stats_chunk(va, b, nk2, s2, ss2);
 #pragma unroll
             for (int j = 0; j < 8; ++j) b[j] = __ldg(reinterpret_cast<const float4*>(bias + c0 + 32) + j);
             tmem_wait_ld32(vb);
             if (c0 + 64 < cbeg + HALF) tmem_ld32(lane_addr + (uint32_t)(c0 + 64), va);
-            stats_chunk(vb, b, s2, ss2);
+            stats_chunk(vb, b, nk2, s2, ss2);
         }
     } else {   // 18 warps share the register file (96 per thread): 16-column chunks
         uint32_t va[16], vb[16];
@@ -297,36 +310,35 @@ __device__ __forceinline__ void layer_epilogue(uint32_t lane_addr, uint32_t a_ba
 #pragma unroll
             for (int j = 0; j < 4; ++j) b[j] = __ldg(reinterpret_cast<const float4*>(bias + c0) + j);
             tmem_wait_ld16(va);
+            if (c0 == cbeg) { k = __uint_as_float(va[0]) + b[0].x; nk2 = pk2(-k, -k); }
             tmem_ld16(lane_addr + (uint32_t)(c0 + 16), vb);
-            stats_chunk16(va, b, s2, ss2);
+            stats_chunk16(va, b, nk2, s2, ss2);
 #pragma unroll
             for (int j = 0; j < 4; ++j) b[j] = __ldg(reinterpret_cast<const float4*>(bias + c0 + 16) + j);
             tmem_wait_ld16(vb);
             if (c0 + 32 < cbeg + HALF) tmem_ld16(lane_addr + (uint32_t)(c0 + 32), va);
-            stats_chunk16(vb, b, s2, ss2);
+            stats_chunk16(vb, b, nk2, s2, ss2);
         }
     }
     float s_lo, s_hi, q_lo, q_hi;
     upk2(s2, s_lo, s_hi); upk2(ss2, q_lo, q_hi);
-    const float s = s_lo + s_hi, ss = q_lo + q_hi;
-    float mean, var;
+    const float s = s_lo + s_hi, ss = q_lo + q_hi, ms = s * (1.0f / HALF);
+    const float2 part = make_float2(k + ms, fmaxf(fmaf(-s, ms, ss), 0.f));   // the part's (mean, M2)
+    float2 all;
     if (PARTS == 2) {
-        stats[half][row] = make_float2(s, ss);
-        asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");   // the two halves of every row have published their sums
-        const float2 o = stats[half ^ 1][row];
-        mean = (s + o.x) * (1.0f / N);
-        var = fmaxf((ss + o.y) * (1.0f / N) - mean * mean, 0.f);   // biased variance, as nn.LayerNorm
+        stats[half][row] = part;
+        asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");   // the two halves of every row have published their statistics
+        all = chan_merge(stats[0][row], stats[1][row], (float)HALF);
     } else {
-        // four parts through the same 2 KiB (224 of the 227 KiB are operands and weight ring): parts 2, 3 hand their sums to parts
-        // 0, 1, which publish the pair sums; everybody adds the two pair sums in the same order
-        if (half >= 2) stats[half - 2][row] = make_float2(s, ss);
+        // four parts through the same 2 KiB (224 of the 227 KiB are operands and weight ring): parts 2, 3 hand their statistics to
+        // parts 0, 1, which publish the merged pairs; everybody merges the two pairs in the same order
+        if (half >= 2) stats[half - 2][row] = part;
         asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
-        if (half < 2) { const float2 o = stats[half][row]; stats[half][row] = make_float2(s + o.x, ss + o.y); }
+        if (half < 2) stats[half][row] = chan_merge(part, stats[half][row], (float)HALF);
         asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory");
-        const float2 p0 = stats[0][row], p1 = stats[1][row];
-        mean = (p0.x + p1.x) * (1.0f / N);
-        var = fmaxf((p0.y + p1.y) * (1.0f / N) - mean * mean, 0.f);
+        all = chan_merge(stats[0][row], stats[1][row], (float)(2 * HALF));
     }   // (the next layer's writes come after a_ready / acc_ready, which every epilogue thread passes first)
+    const float mean = all.x, var = all.y * (1.0f / N);   // biased variance, as nn.LayerNorm
     const float rstd = rsqrtf(var + eps);
     const uint64_t rstd2 = pk2(rstd, rstd), shift2 = pk2(-mean * rstd, -mean * rstd);
     {
@@ -555,6 +567,22 @@ __global__ void pack_bf16_kernel(const float* __restrict__ src, int rows, int k_
     const int r = i / k_dst, c = i - r * k_dst;
     dst[i] = __float2bfloat16_rn((r < rows && c < k_src) ? src[(size_t)r * k_src + c] : 0.f);
 }
+// dst = src - mean(src), one block of 256 threads.  LayerNorm is shift invariant, so this changes nothing but the rounding: a
+// common offset of a layer's bias is taken out once here instead of riding through every row's fp32 epilogue, where it would cost
+// (offset / std) * 2^-24 of each normalised value (b_i - mean(b) is exact whenever b_i and the mean are within a factor 2).
+__global__ void copy_centred_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int n) {
+    __shared__ double part[256];
+    double s = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) s += src[i];
+    part[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 128; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) part[threadIdx.x] += part[threadIdx.x + w];
+        __syncthreads();
+    }
+    const float m = (float)(part[0] / n);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = src[i] - m;
+}
 __global__ void copy_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int n, int n_dst) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n_dst) dst[i] = i < n ? src[i] : 0.f;
@@ -668,9 +696,10 @@ int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, voi
     CK(cudaMemsetAsync(p->wh, 0, sizeof(__nv_bfloat16) * HEAD_N * H3, st));
     pack(w->wa, ACT, H3, p->wh, ACT, H3);                 // rows 0-5: action_net
     pack(w->wv, 1, H3, p->wh + (size_t)ACT * H3, 1, H3);  // row 6: value_net
-    vec(w->b1, H1, VEC_B1, H1); vec(w->ln1_g, H1, VEC_G1, H1); vec(w->ln1_b, H1, VEC_BE1, H1);
-    vec(w->b2, H2, VEC_B2, H2); vec(w->ln2_g, H2, VEC_G2, H2); vec(w->ln2_b, H2, VEC_BE2, H2);
-    vec(w->b3, H3, VEC_B3, H3); vec(w->ln3_g, H3, VEC_G3, H3); vec(w->ln3_b, H3, VEC_BE3, H3);
+    auto centred = [&](const float* src, int n, int off) { copy_centred_f32_kernel<<<1, 256, 0, st>>>(src, p->vec + off, n); };
+    centred(w->b1, H1, VEC_B1); vec(w->ln1_g, H1, VEC_G1, H1); vec(w->ln1_b, H1, VEC_BE1, H1);
+    centred(w->b2, H2, VEC_B2); vec(w->ln2_g, H2, VEC_G2, H2); vec(w->ln2_b, H2, VEC_BE2, H2);
+    centred(w->b3, H3, VEC_B3); vec(w->ln3_g, H3, VEC_G3, H3); vec(w->ln3_b, H3, VEC_BE3, H3);
     CK(cudaMemsetAsync(p->vec + VEC_BH, 0, sizeof(float) * 16, st));
     vec(w->ba, ACT, VEC_BH, ACT); vec(w->bv, 1, VEC_BH + ACT, 1);
     vec(w->log_std, ACT, VEC_LS, 8);

@@ -115,6 +115,10 @@ class FusedActorCritic:
                                       "with LayerNorm + ReLU (train_flat_ppo.py:410); other shapes run through torch")
         if tuple(net.action_net.weight.shape) != (6, 256) or tuple(net.value_net.weight.shape) != (1, 256):
             raise NotImplementedError("action_net must be Linear(256, 6) and value_net Linear(256, 1)")
+        if any(m.weight is None or m.bias is None for m in lns):
+            raise NotImplementedError("the fused forward needs LayerNorms with affine parameters (elementwise_affine=True, bias=True)")
+        if len({float(m.eps) for m in lns}) != 1:   # the kernel applies one eps to all three LayerNorms
+            raise NotImplementedError(f"the fused forward needs one LayerNorm eps for all layers, got {[m.eps for m in lns]}")
         return lins, lns
 
     def sync_weights(self):

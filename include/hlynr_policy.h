@@ -67,7 +67,7 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
                          float* actions_dev, float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev,
                          uint64_t seed, uint64_t counter, int deterministic, void* stream);
 
-/* Options.  "cluster": CTAs per thread-block cluster, 1, 2 (default) or 4: the CTAs of a cluster share every weight tile through
+/* Options.  "cluster": CTAs per thread-block cluster, 1 (default), 2 or 4: the CTAs of a cluster share every weight tile through
  * TMA multicast, which divides the L2 -> SM weight traffic (the kernel's bottleneck without it) by the cluster size. */
 int hlynr_policy_set_option(hlynr_policy_t* p, const char* name, int64_t value);
 
