@@ -19,13 +19,13 @@ EXPORTS = [
     "hlynr_debug_draws", "hlynr_launch_count", "hlynr_set_option", "hlynr_set_done_list", "hlynr_done_records_host",
     "hlynr_ring_period", "hlynr_note_replayed_ticks", "hlynr_tick_count", "hlynr_pinned_done", "hlynr_host_done_buffer",
     # include/hlynr_post.h
-    "hlynr_post_create", "hlynr_post_destroy", "hlynr_post_obs_dim", "hlynr_post_obs_target", "hlynr_post_reset",
+    "hlynr_post_create", "hlynr_post_create_frames", "hlynr_post_destroy", "hlynr_post_obs_dim", "hlynr_post_obs_target", "hlynr_post_reset",
     "hlynr_post_step", "hlynr_post_original", "hlynr_post_normalize", "hlynr_post_get_stats", "hlynr_post_set_stats",
     "hlynr_post_check_sums", "hlynr_post_launch_count", "hlynr_post_note_replayed_steps",
     # include/hlynr_rollout.h
     "hlynr_bootstrap_timeouts", "hlynr_gae",
     # include/hlynr_policy.h
-    "hlynr_policy_create", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
+    "hlynr_policy_create", "hlynr_policy_create_dim", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
 ]
 
 
@@ -83,6 +83,7 @@ def load(build_if_missing=True):
     L.hlynr_done_records_host.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_int32)]
     dbl, pd = C.c_double, C.POINTER(C.c_double)
     L.hlynr_post_create.argtypes = [i64, i32, i32, dbl, dbl, dbl, C.POINTER(vp)]
+    L.hlynr_post_create_frames.argtypes = [i64, i32, i32, i32, dbl, dbl, dbl, C.POINTER(vp)]
     L.hlynr_post_destroy.argtypes = [vp]
     L.hlynr_post_destroy.restype = None
     L.hlynr_post_obs_dim.argtypes = [vp, C.POINTER(i32)]
@@ -102,6 +103,7 @@ def load(build_if_missing=True):
     L.hlynr_bootstrap_timeouts.argtypes = [vp, vp, vp, C.c_int32, vp, C.c_double, vp, i32, vp]
     L.hlynr_gae.argtypes = [vp, vp, vp, vp, vp, i64, i64, C.c_double, C.c_double, vp, vp, i32, vp]
     L.hlynr_policy_create.argtypes = [i32, C.POINTER(vp)]
+    L.hlynr_policy_create_dim.argtypes = [i32, i32, C.POINTER(vp)]
     L.hlynr_policy_destroy.argtypes = [vp]
     L.hlynr_policy_destroy.restype = None
     L.hlynr_policy_set_weights.argtypes = [vp, C.POINTER(abi.HlynrPolicyWeights), vp]

@@ -2,7 +2,8 @@
 //
 // Network = the reference's policy (rl_system/scripts/train_flat_ppo.py:37-85 CustomMLP as SB3 features extractor, :419-429
 // net_arch=[] so action_net / value_net sit directly on the 256 features):
-//     x[104] -> Linear 512 -> LayerNorm -> ReLU -> Linear 512 -> LayerNorm -> ReLU -> Linear 256 -> LayerNorm -> ReLU -> f[256]
+//     x[in_dim] -> Linear 512 -> LayerNorm -> ReLU -> Linear 512 -> LayerNorm -> ReLU -> Linear 256 -> LayerNorm -> ReLU -> f[256]
+//     (in_dim = 104 = 4 stacked 26-D frames by default; any width 1-256, e.g. 68 = 4 stacked 17-D frames)
 //     mean = action_net(f) [6], V = value_net(f) [1], a = mean + exp(log_std) * eps, log pi(a)
 //
 // One persistent CTA per SM walks over 128-row tiles.  Per tile the activations never leave the SM:
@@ -42,14 +43,14 @@ extern "C" int hlynr_internal_fail(const char* fmt, ...);  // hlynr_capi.cu: set
 namespace {
 
 constexpr int IN = HLYNR_POLICY_IN, H1 = HLYNR_POLICY_H1, H2 = HLYNR_POLICY_H2, H3 = HLYNR_POLICY_H3, ACT = HLYNR_POLICY_ACT;
-constexpr int IN_PAD = 128;      // K of the first GEMM padded to two 64-wide K blocks (zeros)
+constexpr int IN_PAD = 128;      // K of the first GEMM at in_dim = 104, padded to two 64-wide K blocks (zeros)
 constexpr int HEAD_N = 16;       // action_net (6 rows) + value_net (1 row) + zero rows: the smallest UMMA N for M = 128
 constexpr int BM = 128;          // rows per tile = UMMA M = TMEM lanes
 constexpr int BK = 64;           // bf16 elements per K block: 128 bytes = one swizzle span
 constexpr int BN = 256;          // weight rows per ring stage = UMMA N
 constexpr int STAGES = 3;
 constexpr int KBLOCK_BYTES = BM * BK * 2;            // 16 KiB: one K block of the A operand
-constexpr int A_BYTES = BM * 512 * 2;                // 128 KiB: x (2 K blocks), then H1 / H2 (8), then H3 (4)
+constexpr int A_BYTES = BM * 512 * 2;                // 128 KiB: x (ceil(in_dim / 64) <= 4 K blocks), then H1 / H2 (8), then H3 (4)
 constexpr int STAGE_BYTES = BN * BK * 2;             // 32 KiB
 #ifndef HLYNR_POLICY_EPI_WARPS
 #define HLYNR_POLICY_EPI_WARPS 16   /* measured on B200 at 131072 rows: 8 warps 219 us, 16 warps 203 us (profiles/r02_h_policy_epilogue_warps.log) */
@@ -67,7 +68,8 @@ static_assert(SMEM_BYTES <= 232448, "shared memory budget of one CTA (227 KiB)")
 constexpr uint32_t TMEM_COLS = 512;
 constexpr int N_LAYERS = 4;      // three hidden GEMMs + the head GEMM
 
-__host__ __device__ constexpr int layer_kblocks(int l) { return l == 0 ? IN_PAD / BK : (l == 3 ? H3 / BK : 512 / BK); }
+// kb0 = K blocks of the first GEMM, ceil(in_dim / 64)
+__host__ __device__ constexpr int layer_kblocks(int l, int kb0) { return l == 0 ? kb0 : (l == 3 ? H3 / BK : 512 / BK); }
 __host__ __device__ constexpr int layer_nchunks(int l) { return l < 2 ? 2 : 1; }
 __host__ __device__ constexpr int layer_n(int l) { return l == 3 ? HEAD_N : BN; }
 __host__ __device__ constexpr uint32_t layer_col(int l, int nc) { return l == 3 ? 256u : (uint32_t)(nc * BN); }   // TMEM column of the accumulator
@@ -84,7 +86,8 @@ constexpr int VEC_B1 = 0, VEC_G1 = 512, VEC_BE1 = 1024, VEC_B2 = 1536, VEC_G2 = 
               VEC_BE3 = 3584, VEC_BH = 3840, VEC_LS = 3856, VEC_TOTAL = 3864;
 
 struct Params {
-    const float* obs;
+    const float* obs;       // [n_rows, in_dim]
+    int in_dim, kb0;        // row width, K blocks of the first GEMM (ceil(in_dim / 64))
     int64_t n_rows;
     const int32_t* n_rows_dev;
     const float* vec;   // the per-column vectors, VEC_* offsets
@@ -373,7 +376,8 @@ __device__ __forceinline__ void layer_epilogue(uint32_t lane_addr, uint32_t a_ba
 // every weight tile: CTA r loads rows [r * N / CL, (r + 1) * N / CL) of a stage and multicasts them to all, so the L2 -> SM weight
 // traffic (904 KiB per 128-row tile, the kernel's bottleneck at CL = 1) is divided by CL.  A stage may be refilled only after the
 // MMAs of ALL CTAs have read it: the empty barriers count CL arrivals, delivered by multicast tcgen05.commit.
-template <int CL>
+// XW = IN: rows of exactly 104 floats, 16-byte aligned (the default network); XW = 0: any in_dim in [1, 256], rows 4-byte aligned.
+template <int CL, int XW>
 __global__ void __launch_bounds__(THREADS, 1)   // (ptxas caps the registers per SM sub-partition: 3 of 10 warps x 168, 5 of 18 warps x 96)
 policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1,
                       const __grid_constant__ CUtensorMap tm2, const __grid_constant__ CUtensorMap tm3, const Params P) {
@@ -384,6 +388,7 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
     volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + OFF_TMEM);
     const uint32_t bar_full = bars, bar_empty = bars + STAGES * 8, bar_a = bars + 2 * STAGES * 8, bar_acc = bar_a + 8;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int kb0 = XW == IN ? IN_PAD / BK : P.kb0;
 
     int64_t n_rows = P.n_rows;
     if (P.n_rows_dev) { const int64_t lim = (int64_t)*P.n_rows_dev; n_rows = lim < n_rows ? (lim < 0 ? 0 : lim) : n_rows; }
@@ -424,7 +429,7 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
                     const uint32_t bytes = (uint32_t)(layer_n(l) * BK * 2);        // of the whole stage, all slices
                     const int slice_rows = layer_n(l) / CL;
                     for (int nc = 0; nc < layer_nchunks(l); ++nc)
-                        for (int kb = 0; kb < layer_kblocks(l); ++kb) {
+                        for (int kb = 0; kb < layer_kblocks(l, kb0); ++kb) {
                             mbar_wait(bar_empty + stage * 8, phase ^ 1u, P.error_flag, 1);   // released by the MMAs of all CL CTAs
                             mbar_expect_tx(bar_full + stage * 8, bytes);
                             const uint32_t dst = ring + stage * STAGE_BYTES + cta_rank * (uint32_t)(slice_rows * BK * 2);
@@ -449,7 +454,7 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
                     const uint32_t idesc = instr_desc(layer_n(l));
                     for (int nc = 0; nc < layer_nchunks(l); ++nc) {
                         const uint32_t d = tmem_base + layer_col(l, nc);
-                        for (int kb = 0; kb < layer_kblocks(l); ++kb) {
+                        for (int kb = 0; kb < layer_kblocks(l, kb0); ++kb) {
                             mbar_wait(bar_full + stage * 8, phase, P.error_flag, 3);
                             tc_fence_after();
                             const uint64_t adesc = smem_desc(a_base + kb * KBLOCK_BYTES), bdesc = smem_desc(ring + stage * STAGE_BYTES);
@@ -477,19 +482,42 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
             const int64_t tile = (int64_t)blockIdx.x + it * gridDim.x;
             tstamp = (P.timing && blockIdx.x == 0 && threadIdx.x == 0 && it < P.timing_tiles) ? P.timing + it * 16 : nullptr;
             if (tstamp) tstamp[0] = clock64();
-            // x tile: fp32 [128, 104] -> bf16, K padded to 128 with zeros, swizzled K-major
+            if constexpr (XW == IN) {
+                // x tile: fp32 [128, 104] -> bf16, K padded to 128 with zeros, swizzled K-major
 #pragma unroll
-            for (int i = 0; i < (BM * IN_PAD / 8) / EPI_THREADS; ++i) {
-                const int task = (int)threadIdx.x + i * EPI_THREADS;
-                const int r = task >> 4, c = task & 15;
-                uint4 packed = make_uint4(0u, 0u, 0u, 0u);
-                const int64_t grow = tile * BM + r;
-                if (c < IN / 8 && grow < n_rows) {
-                    const float4* src = reinterpret_cast<const float4*>(P.obs + grow * IN + c * 8);
-                    const float4 a = __ldg(src), b = __ldg(src + 1);
-                    packed = make_uint4(pack_bf16(a.x, a.y), pack_bf16(a.z, a.w), pack_bf16(b.x, b.y), pack_bf16(b.z, b.w));
+                for (int i = 0; i < (BM * IN_PAD / 8) / EPI_THREADS; ++i) {
+                    const int task = (int)threadIdx.x + i * EPI_THREADS;
+                    const int r = task >> 4, c = task & 15;
+                    uint4 packed = make_uint4(0u, 0u, 0u, 0u);
+                    const int64_t grow = tile * BM + r;
+                    if (c < IN / 8 && grow < n_rows) {
+                        const float4* src = reinterpret_cast<const float4*>(P.obs + grow * IN + c * 8);
+                        const float4 a = __ldg(src), b = __ldg(src + 1);
+                        packed = make_uint4(pack_bf16(a.x, a.y), pack_bf16(a.z, a.w), pack_bf16(b.x, b.y), pack_bf16(b.z, b.w));
+                    }
+                    st_shared_v4(a_base + a_chunk_offset(r, c), packed);
                 }
-                st_shared_v4(a_base + a_chunk_offset(r, c), packed);
+            } else {
+                // x tile: fp32 [128, in_dim] -> bf16, K padded to 64 * kb0 with zeros, swizzled K-major.  A row of a rollout buffer
+                // [T + 1, N, in_dim] is only 4-byte aligned when in_dim * N is odd: one float per load, the 8 loads of a chunk
+                // in flight together; the lanes of a warp cover consecutive chunks of a row
+                const int chunks = kb0 * 8, in_dim = P.in_dim;
+#pragma unroll 1
+                for (int task = (int)threadIdx.x; task < BM * chunks; task += EPI_THREADS) {
+                    const int r = task / chunks, c = task - r * chunks, c0 = c * 8;
+                    const int64_t grow = tile * BM + r;
+                    float x[8];
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) x[j] = 0.f;
+                    if (c0 < in_dim && grow < n_rows) {
+                        const float* src = P.obs + grow * in_dim + c0;
+#pragma unroll
+                        for (int j = 0; j < 8; ++j)
+                            if (c0 + j < in_dim) x[j] = __ldg(src + j);
+                    }
+                    st_shared_v4(a_base + a_chunk_offset(r, c),
+                                 make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7])));
+                }
             }
             fence_async_smem();    // generic-proxy writes -> visible to the tensor core's async-proxy reads
             tc_fence_before();
@@ -602,7 +630,8 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 
 struct hlynr_policy {
     int device = 0, sm_count = 148;
-    __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wh = nullptr;   // [512,128], [512,512], [256,512], [16,256]
+    int in_dim = IN, kb0 = IN_PAD / BK;   // input width, K blocks of the first GEMM
+    __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wh = nullptr;   // [512,64*kb0], [512,512], [256,512], [16,256]
     float* vec = nullptr;   // b1 g1 be1 (512 x3) | b2 g2 be2 (512 x3) | b3 g3 be3 (256 x3) | bh (16) | log_std (8)
     int* error_flag = nullptr;
     long long* timing = nullptr;   // debug timestamps (option "timing")
@@ -636,8 +665,11 @@ void hlynr_policy_destroy(hlynr_policy_t* p) {
     delete p;
 }
 
-int hlynr_policy_create(int device, hlynr_policy_t** out) {
+int hlynr_policy_create(int device, hlynr_policy_t** out) { return hlynr_policy_create_dim(device, IN, out); }
+
+int hlynr_policy_create_dim(int device, int in_dim, hlynr_policy_t** out) {
     if (!out) return fail("hlynr_policy_create: null argument");
+    if (in_dim < 1 || in_dim > HLYNR_POLICY_MAX_IN) return fail("hlynr_policy_create: in_dim must be in [1, %d], got %d", HLYNR_POLICY_MAX_IN, in_dim);
     int ndev = 0;
     CK(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail("hlynr_policy_create: device %d not available (%d devices)", device, ndev);
@@ -648,8 +680,10 @@ int hlynr_policy_create(int device, hlynr_policy_t** out) {
     hlynr_policy* p = new (std::nothrow) hlynr_policy();
     if (!p) return fail("hlynr_policy_create: out of host memory");
     p->device = device; p->sm_count = prop.multiProcessorCount;
+    p->in_dim = in_dim; p->kb0 = (in_dim + BK - 1) / BK;
     cudaError_t e = cudaSuccess;
-    if (e == cudaSuccess) e = cudaMalloc(&p->w1, sizeof(__nv_bfloat16) * H1 * IN_PAD);
+    // the TMA map needs 16-byte row strides: w1 lives in a [512, 64 * kb0] buffer whose columns past in_dim are zero
+    if (e == cudaSuccess) e = cudaMalloc(&p->w1, sizeof(__nv_bfloat16) * H1 * BK * p->kb0);
     if (e == cudaSuccess) e = cudaMalloc(&p->w2, sizeof(__nv_bfloat16) * H2 * H1);
     if (e == cudaSuccess) e = cudaMalloc(&p->w3, sizeof(__nv_bfloat16) * H3 * H2);
     if (e == cudaSuccess) e = cudaMalloc(&p->wh, sizeof(__nv_bfloat16) * HEAD_N * H3);
@@ -668,7 +702,7 @@ int hlynr_policy_create(int device, hlynr_policy_t** out) {
     EncodeTiledFn enc = reinterpret_cast<EncodeTiledFn>(fn);
     for (int c = 0; c < 3; ++c) {
         const int cl = 1 << c;
-        if (make_map(enc, &p->tm[c][0], p->w1, H1, IN_PAD, BN / cl) || make_map(enc, &p->tm[c][1], p->w2, H2, H1, BN / cl) ||
+        if (make_map(enc, &p->tm[c][0], p->w1, H1, BK * p->kb0, BN / cl) || make_map(enc, &p->tm[c][1], p->w2, H2, H1, BN / cl) ||
             make_map(enc, &p->tm[c][2], p->w3, H3, H2, BN / cl) || make_map(enc, &p->tm[c][3], p->wh, HEAD_N, H3, HEAD_N / cl)) {
             hlynr_policy_destroy(p);
             return 1;
@@ -690,7 +724,7 @@ int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, voi
         pack_bf16_kernel<<<(n + 255) / 256, 256, 0, st>>>(src, rows, k, dst, rows_dst, k_dst);
     };
     auto vec = [&](const float* src, int n, int off, int n_dst) { copy_f32_kernel<<<(n_dst + 255) / 256, 256, 0, st>>>(src, p->vec + off, n, n_dst); };
-    pack(w->w1, H1, IN, p->w1, H1, IN_PAD);
+    pack(w->w1, H1, p->in_dim, p->w1, H1, BK * p->kb0);
     pack(w->w2, H2, H1, p->w2, H2, H1);
     pack(w->w3, H3, H2, p->w3, H3, H2);
     CK(cudaMemsetAsync(p->wh, 0, sizeof(__nv_bfloat16) * HEAD_N * H3, st));
@@ -716,17 +750,25 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
     if (!p || !obs_dev) return fail("hlynr_policy_forward: null argument");
     if (!p->ready) return fail("hlynr_policy_forward: hlynr_policy_set_weights has not been called");
     if (n_rows <= 0) return fail("hlynr_policy_forward: n_rows must be positive");
-    if (((uintptr_t)obs_dev & 15u) != 0) return fail("hlynr_policy_forward: obs_dev must be 16-byte aligned");
+    const bool fixed = p->in_dim == IN;   // the 104-wide instantiation: float4 loads of 16-byte aligned rows
+    if (fixed && ((uintptr_t)obs_dev & 15u) != 0) return fail("hlynr_policy_forward: obs_dev must be 16-byte aligned");
+    if (((uintptr_t)obs_dev & 3u) != 0) return fail("hlynr_policy_forward: obs_dev must be 4-byte aligned");
     DeviceGuard g(p->device);
     if (!p->smem_configured) {
-        CK(cudaFuncSetAttribute(policy_forward_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        CK(cudaFuncSetAttribute(policy_forward_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        CK(cudaFuncSetAttribute(policy_forward_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        if (fixed) {
+            CK(cudaFuncSetAttribute(policy_forward_kernel<1, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+            CK(cudaFuncSetAttribute(policy_forward_kernel<2, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+            CK(cudaFuncSetAttribute(policy_forward_kernel<4, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        } else {
+            CK(cudaFuncSetAttribute(policy_forward_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+            CK(cudaFuncSetAttribute(policy_forward_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+            CK(cudaFuncSetAttribute(policy_forward_kernel<4, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        }
         p->smem_configured = true;
     }
     Params P;
     memset(&P, 0, sizeof(P));
-    P.obs = obs_dev; P.n_rows = n_rows; P.n_rows_dev = n_rows_dev;
+    P.obs = obs_dev; P.in_dim = p->in_dim; P.kb0 = p->kb0; P.n_rows = n_rows; P.n_rows_dev = n_rows_dev;
     P.vec = p->vec;
     P.actions = actions_dev; P.values = values_dev; P.logp = logp_dev; P.mean = mean_dev; P.actions_clipped = actions_clipped_dev;
     P.ln_eps = p->ln_eps;
@@ -747,8 +789,11 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
         if (cl > 1) {
             cfg.gridDim = dim3((unsigned)(clusters * cl));
             int fit = 0;
-            const cudaError_t oe = cl == 2 ? cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<2>, &cfg)
-                                           : cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<4>, &cfg);
+            cudaError_t oe;
+            if (fixed) oe = cl == 2 ? cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<2, IN>, &cfg)
+                                    : cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<4, IN>, &cfg);
+            else oe = cl == 2 ? cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<2, 0>, &cfg)
+                              : cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<4, 0>, &cfg);
             if (oe == cudaSuccess && fit > 0 && fit < clusters) clusters = fit;
             else if (oe != cudaSuccess) cudaGetLastError();
         }
@@ -759,9 +804,15 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
     cfg.gridDim = dim3((unsigned)grid);
     const CUtensorMap* tm = p->tm[ci];
     cudaError_t le;
-    if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1>, tm[0], tm[1], tm[2], tm[3], P);
-    else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2>, tm[0], tm[1], tm[2], tm[3], P);
-    else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4>, tm[0], tm[1], tm[2], tm[3], P);
+    if (fixed) {
+        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, IN>, tm[0], tm[1], tm[2], tm[3], P);
+        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, IN>, tm[0], tm[1], tm[2], tm[3], P);
+        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, IN>, tm[0], tm[1], tm[2], tm[3], P);
+    } else {
+        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, 0>, tm[0], tm[1], tm[2], tm[3], P);
+        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, 0>, tm[0], tm[1], tm[2], tm[3], P);
+        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, 0>, tm[0], tm[1], tm[2], tm[3], P);
+    }
     if (le != cudaSuccess) return fail("hlynr_policy_forward: launch failed: %s", cudaGetErrorString(le));
     CK(cudaGetLastError());
     p->launches += 1;

@@ -2,13 +2,16 @@
 //
 // Semantics restated from stable-baselines3 2.x (oracle/sb3_post.py cites the source files):
 //   stacked[e] = concat(frame[t-k+1], ..., frame[t]); a finished env's stack is zeroed before its reset observation
-//   is inserted; info['terminal_observation'] = concat(previous_stack[26:], terminal_obs);
+//   is inserted; info['terminal_observation'] = concat(previous_stack[F:], terminal_obs[0:F]);
 //   obs_rms.update(stacked batch) (batch mean/var merged into the running float64 moments), then
 //   out = clip((stacked - mean) / sqrt(var + eps), -clip, clip) as float32; terminal observations likewise.
 //
 // HBM traffic per env-step (n_stack = 4): 104 B column-sum read of the new frame + 416 B ring read + 416 B output
 // write (+ 9 B age/done flags, 16 B returns) -- the explicit roll/copy of SB3 (another 832 B) never happens, and the
 // step kernel writes its observation straight into the ring slot.
+//
+// The frame width F is 26 (the full observation) or 17 (the leading radar channels obs[0:17], HlynrSim(obs_dim=17)); every
+// kernel that touches the ring is a template on F, so the 26-wide code is what it was before F became a parameter.
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -29,17 +32,17 @@ extern "C" int hlynr_internal_fail(const char* fmt, ...);  // hlynr_capi.cu: set
 
 namespace {
 
-constexpr int OD = HLYNR_OBS_DIM;  // 26
+constexpr int OD = HLYNR_OBS_DIM;  // 26: the widest frame, and the row capacity of the per-lag arrays of PostStats
 constexpr int KMAX = HLYNR_POST_MAX_STACK;
 constexpr int DMAX = OD * KMAX;
 
-// device statistics block (doubles)
+// device statistics block (doubles); a 17-wide frame uses the first 17 entries of every [KMAX][OD] row
 struct PostStats {
     double S[KMAX][OD], Q[KMAX][OD];        // per-lag column sums / sums of squares of the current stacked batch (lag 0 = newest)
     double col[OD], colq[OD];               // scratch: sums over the new frame
     double corr[KMAX][OD], corrq[KMAX][OD]; // scratch: frames of the envs that finished in this step (subtracted)
     double ret_sum, ret_sq;                 // scratch: sums over the discounted returns
-    double mean[DMAX], var[DMAX], count;    // obs_rms (feature f = j*26 + c, j = 0 oldest)
+    double mean[DMAX], var[DMAX], count;    // obs_rms (feature f = j*F + c, j = 0 oldest)
     double ret_mean, ret_var, ret_count;    // ret_rms
     double chk_S[KMAX][OD], chk_Q[KMAX][OD];  // check_sums scratch
     double inv_std[DMAX];                   // 1 / sqrt(var + eps): the normalise kernels compute in float64 like SB3 (obs f32 - mean f64)
@@ -53,37 +56,40 @@ struct DeviceGuard {
 
 __device__ __forceinline__ int ring_slot(int newest, int lag, int k) { int s = newest - lag; return s < 0 ? s + k : s; }
 
-// ---- sums over the new frame: thread-constant channel, 16 envs per 416-thread block iteration, coalesced ----
+// ---- sums over the new frame: thread-constant channel, 16 envs per 16*F-thread block iteration, coalesced ----
 // Every reduction of this file is two-stage and atomic-free: blocks write partial sums to partials[block][word], one
 // block per word then folds them in a fixed order, so the statistics (and with them the normalised observations) are
 // bit-reproducible from run to run.
-constexpr int PW_COL = 0, PW_COLQ = OD, PW_RET = 2 * OD, PW_RETQ = 2 * OD + 1, PW_CORR = 2 * OD + 2;
-constexpr int PART_WORDS = PW_CORR + 2 * (KMAX - 1) * OD;   // + corr[(k-1)][26], corrq[(k-1)][26]
+template <int F>   // word offsets of a partial row for frame width F: [col F | colq F | ret | retq | corr (k-1)*F | corrq (k-1)*F]
+struct PW { static constexpr int COL = 0, COLQ = F, RET = 2 * F, RETQ = 2 * F + 1, CORR = 2 * F + 2; };
+constexpr int PART_WORDS = PW<OD>::CORR + 2 * (KMAX - 1) * OD;   // sized for the widest frame
 
-__global__ void __launch_bounds__(16 * OD) colsum_kernel(const float* __restrict__ frame, int64_t n, double* __restrict__ partials) {
-    __shared__ double sh[16 * OD];
-    const int t = threadIdx.x, c = t % OD, r = t / OD;
+template <int F>
+__global__ void __launch_bounds__(16 * F) colsum_kernel(const float* __restrict__ frame, int64_t n, double* __restrict__ partials) {
+    __shared__ double sh[16 * F];
+    const int t = threadIdx.x, c = t % F, r = t / F;
     double s = 0.0, q = 0.0;
     for (int64_t e = (int64_t)blockIdx.x * 16 + r; e < n; e += (int64_t)gridDim.x * 16) {
-        const double v = (double)frame[e * OD + c];
+        const double v = (double)frame[e * F + c];
         s += v; q += v * v;
     }
     sh[t] = s;
     __syncthreads();
     double* mine = partials + (size_t)blockIdx.x * PART_WORDS;
-    if (r == 0) { double a = 0.0; for (int i = 0; i < 16; ++i) a += sh[i * OD + c]; mine[PW_COL + c] = a; }
+    if (r == 0) { double a = 0.0; for (int i = 0; i < 16; ++i) a += sh[i * F + c]; mine[PW<F>::COL + c] = a; }
     __syncthreads();
     sh[t] = q;
     __syncthreads();
-    if (r == 0) { double a = 0.0; for (int i = 0; i < 16; ++i) a += sh[i * OD + c]; mine[PW_COLQ + c] = a; }
+    if (r == 0) { double a = 0.0; for (int i = 0; i < 16; ++i) a += sh[i * F + c]; mine[PW<F>::COLQ + c] = a; }
 }
 
 // second stage: block w folds word w of the partial rows (fixed order) into its PostStats field
+template <int F>
 __global__ void __launch_bounds__(256) fold_kernel(const double* __restrict__ partials, int nb_col, int nb_ret, int nb_corr, int per,
                                                    PostStats* st) {
     __shared__ double sh[256];
-    const int w = blockIdx.x < 2 * OD + 2 ? blockIdx.x : PW_CORR + (blockIdx.x - (2 * OD + 2));
-    const int nblocks = w < 2 * OD ? nb_col : (w < PW_CORR ? nb_ret : nb_corr);
+    const int w = blockIdx.x;
+    const int nblocks = w < 2 * F ? nb_col : (w < PW<F>::CORR ? nb_ret : nb_corr);
     double a = 0.0;
     for (int b = threadIdx.x; b < nblocks; b += 256) a += partials[(size_t)b * PART_WORDS + w];
     sh[threadIdx.x] = a;
@@ -93,15 +99,17 @@ __global__ void __launch_bounds__(256) fold_kernel(const double* __restrict__ pa
         __syncthreads();
     }
     if (threadIdx.x != 0) return;
-    if (w < 2 * OD) (&st->col[0])[w] = sh[0];                       // col[26], colq[26] are adjacent
-    else if (w < PW_CORR) (&st->ret_sum)[w - 2 * OD] = sh[0];        // ret_sum, ret_sq
-    else if (w - PW_CORR < per) (&st->corr[1][0])[w - PW_CORR] = sh[0];
-    else (&st->corrq[1][0])[w - PW_CORR - per] = sh[0];
+    if (w < F) st->col[w] = sh[0];
+    else if (w < 2 * F) st->colq[w - F] = sh[0];
+    else if (w < PW<F>::CORR) (&st->ret_sum)[w - 2 * F] = sh[0];     // ret_sum, ret_sq
+    else if (w - PW<F>::CORR < per) { const int f = w - PW<F>::CORR; st->corr[1 + f / F][f % F] = sh[0]; }
+    else { const int f = w - PW<F>::CORR - per; st->corrq[1 + f / F][f % F] = sh[0]; }
 }
 
 // ---- VecNormalize._update_reward: returns = returns * gamma + reward; ret_rms sums; returns[done] = 0 ----
 // Also the per-env part of VecFrameStack: age_new = done ? 0 : min(age_old + 1, k - 1) (how many older frames of the
 // ring belong to the env's current episode).
+template <int F>
 __global__ void __launch_bounds__(256) returns_kernel(double* __restrict__ ret, const float* __restrict__ rew,
                                                       const uint8_t* __restrict__ term, const uint8_t* __restrict__ trunc, int64_t n,
                                                       double gamma, double* __restrict__ partials, int training,
@@ -125,34 +133,35 @@ __global__ void __launch_bounds__(256) returns_kernel(double* __restrict__ ret, 
     if (threadIdx.x == 0) {
         double a = 0.0, b = 0.0;
         for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { a += shs[i]; b += shq[i]; }
-        partials[(size_t)blockIdx.x * PART_WORDS + PW_RET] = a; partials[(size_t)blockIdx.x * PART_WORDS + PW_RETQ] = b;
+        partials[(size_t)blockIdx.x * PART_WORDS + PW<F>::RET] = a; partials[(size_t)blockIdx.x * PART_WORDS + PW<F>::RETQ] = b;
     }
 }
 
 // ---- frames of finished envs leave the stack: accumulate what has to be subtracted from the shifted sums ----
 // thread = (record lane r, old lag d in [0, k-2], channel c); old lag d becomes lag d+1 for the envs that go on.
+template <int F>
 __global__ void __launch_bounds__(512) done_corr_kernel(const HlynrDoneRecord* __restrict__ recs, const int32_t* __restrict__ counter,
                                                         int32_t cap, const float* __restrict__ frames, int64_t plane,
                                                         const uint8_t* __restrict__ age_old, int k, int newest_old,
                                                         double* __restrict__ partials) {
-    const int per = (k - 1) * OD;                 // threads per record
+    const int per = (k - 1) * F;                  // threads per record
     const int lanes = blockDim.x / per;           // records per block iteration
     const int t = threadIdx.x;
     if (t >= lanes * per) return;
-    const int r = t / per, f = t % per, d = f / OD, c = f % OD;
+    const int r = t / per, f = t % per, d = f / F, c = f % F;
     int32_t count = *counter;
     if (count > cap) count = cap;
     double s = 0.0, q = 0.0;
     const float* src = frames + (int64_t)ring_slot(newest_old, d, k) * plane;
     for (int32_t i = blockIdx.x * lanes + r; i < count; i += gridDim.x * lanes) {
         const int32_t e = recs[i].env;
-        if (d <= (int)age_old[e]) { const double v = (double)src[(int64_t)e * OD + c]; s += v; q += v * v; }
+        if (d <= (int)age_old[e]) { const double v = (double)src[(int64_t)e * F + c]; s += v; q += v * v; }
     }
-    // fold the record lanes of this block, then one partial row per block: [corr (k-1)*26 | corrq (k-1)*26]
+    // fold the record lanes of this block, then one partial row per block: [corr (k-1)*F | corrq (k-1)*F]
     __shared__ double sh[512];
     sh[t] = s;
     __syncthreads();
-    double* mine = partials + (size_t)blockIdx.x * PART_WORDS + PW_CORR;
+    double* mine = partials + (size_t)blockIdx.x * PART_WORDS + PW<F>::CORR;
     if (r == 0) { double a = 0.0; for (int i = 0; i < lanes; ++i) a += sh[i * per + f]; mine[f] = a; }
     __syncthreads();
     sh[t] = q;
@@ -161,9 +170,10 @@ __global__ void __launch_bounds__(512) done_corr_kernel(const HlynrDoneRecord* _
 }
 
 // ---- shift the per-lag sums, merge the batch moments into obs_rms / ret_rms (RunningMeanStd.update_from_moments) ----
+template <int F>
 __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int training, int reset_all, int with_returns, double eps) {
-    const int f = threadIdx.x, D = k * OD;
-    if (shift && f < OD) {  // the per-lag sums follow the ring on every reset / step
+    const int f = threadIdx.x, D = k * F;
+    if (shift && f < F) {  // the per-lag sums follow the ring on every reset / step
         const int c = f;
         for (int d = k - 1; d >= 1; --d) {
             st->S[d][c] = reset_all ? 0.0 : st->S[d - 1][c] - st->corr[d][c];
@@ -177,7 +187,7 @@ __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int trai
     __syncthreads();
     if (f < D) {
         if (training) {
-            const int j = f / OD, c = f % OD, d = k - 1 - j;
+            const int j = f / F, c = f % F, d = k - 1 - j;
             const double bm = st->S[d][c] / n;
             double bv = st->Q[d][c] / n - bm * bm;
             if (bv < 0.0) bv = 0.0;
@@ -205,8 +215,8 @@ __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int trai
     }
 }
 
-// ---- stacked (+ normalised) observation: thread-constant feature PAIR (26 is even, so a float2 never straddles two
-// ring slots and every load/store is 8-byte aligned), 4 envs in flight per thread, coalesced [N, 26k] output ----
+// ---- stacked (+ normalised) observation of 26-wide frames: thread-constant feature PAIR (26 is even, so a float2 never
+// straddles two ring slots and every load/store is 8-byte aligned), 8 envs in flight per thread, coalesced [N, 26k] output ----
 #define NORM_UNROLL 8
 __global__ void __launch_bounds__(512) normalize_kernel(const float* __restrict__ frames, int64_t plane, const uint8_t* __restrict__ age,
                                                         const PostStats* __restrict__ st, float* __restrict__ out, int64_t n, int k,
@@ -246,14 +256,51 @@ __global__ void __launch_bounds__(512) normalize_kernel(const float* __restrict_
     }
 }
 
-// ---- info['terminal_observation'] of finished envs: concat(previous_stack[26:], terminal_obs), normalised ----
+// ---- the same for 17-wide frames: thread-constant single feature.  A feature pair would straddle two ring slots at every
+// odd frame boundary, and an output row of odd width 17k starts only 4-byte aligned, so every access is one float; the
+// block's `lanes` consecutive envs still read lanes * 17 contiguous floats per ring slot and write lanes * 17k contiguous
+// floats, and NORM_UNROLL envs are in flight per thread.  Per element the same float operations as normalize_kernel. ----
+template <int F>
+__global__ void __launch_bounds__(512) normalize1_kernel(const float* __restrict__ frames, int64_t plane, const uint8_t* __restrict__ age,
+                                                         const PostStats* __restrict__ st, float* __restrict__ out, int64_t n, int k,
+                                                         int newest, float clip, int raw) {
+    const int D = k * F, lanes = blockDim.x / D, t = threadIdx.x;
+    if (t >= lanes * D) return;
+    const int r = t / D, f = t % D, j = f / F, c = f % F, lag = k - 1 - j;
+    const float mh = (float)st->mean[f], ml = (float)(st->mean[f] - (double)mh), inv = (float)st->inv_std[f];
+    const float* src = frames + (int64_t)ring_slot(newest, lag, k) * plane + c;
+    const int64_t stride = (int64_t)gridDim.x * lanes;
+    for (int64_t e0 = (int64_t)blockIdx.x * lanes + r; e0 < n; e0 += stride * NORM_UNROLL) {
+        float v[NORM_UNROLL];
+        int ag[NORM_UNROLL];
+        bool ok[NORM_UNROLL];
+#pragma unroll
+        for (int u = 0; u < NORM_UNROLL; ++u) {
+            const int64_t e = e0 + u * stride;
+            ok[u] = e < n;
+            v[u] = 0.f;
+            ag[u] = 0;
+            if (ok[u]) { v[u] = __ldcs(src + e * F); ag[u] = (int)__ldg(age + e); }
+        }
+#pragma unroll
+        for (int u = 0; u < NORM_UNROLL; ++u) {
+            if (!ok[u]) continue;
+            float w = lag <= ag[u] ? v[u] : 0.f;
+            if (!raw) w = fminf(fmaxf(((w - mh) - ml) * inv, -clip), clip);
+            __stcs(out + (e0 + u * stride) * D + f, w);
+        }
+    }
+}
+
+// ---- info['terminal_observation'] of finished envs: concat(previous_stack[F:], terminal_obs[0:F]), normalised ----
+template <int F>
 __global__ void __launch_bounds__(512) terminal_kernel(const HlynrDoneRecord* __restrict__ recs, const int32_t* __restrict__ counter, int32_t cap,
                                                        const float* __restrict__ frames, int64_t plane, const uint8_t* __restrict__ age_old,
                                                        const PostStats* __restrict__ st, float* __restrict__ out, int k, int newest_old,
                                                        float clip) {
-    const int D = k * OD, lanes = blockDim.x / D, t = threadIdx.x;
+    const int D = k * F, lanes = blockDim.x / D, t = threadIdx.x;
     if (t >= lanes * D) return;
-    const int r = t / D, f = t % D, j = f / OD, c = f % OD;
+    const int r = t / D, f = t % D, j = f / F, c = f % F;
     const double mean = st->mean[f], inv = st->inv_std[f];
     int32_t count = *counter;
     if (count > cap) count = cap;
@@ -263,7 +310,7 @@ __global__ void __launch_bounds__(512) terminal_kernel(const HlynrDoneRecord* __
         else {
             const int32_t e = recs[i].env;
             const int lag_old = k - 2 - j;
-            v = lag_old <= (int)age_old[e] ? frames[(int64_t)ring_slot(newest_old, lag_old, k) * plane + (int64_t)e * OD + c] : 0.f;
+            v = lag_old <= (int)age_old[e] ? frames[(int64_t)ring_slot(newest_old, lag_old, k) * plane + (int64_t)e * F + c] : 0.f;
         }
         out[(int64_t)i * D + f] = (float)fmin(fmax(((double)v - mean) * inv, -(double)clip), (double)clip);
     }
@@ -281,23 +328,24 @@ __global__ void __launch_bounds__(512) normalize_rows_kernel(const float* __rest
 }
 
 // ---- test hook: per-lag sums recomputed from the ring ----
+template <int F>
 __global__ void __launch_bounds__(512) recompute_sums_kernel(const float* __restrict__ frames, int64_t plane, const uint8_t* __restrict__ age,
                                                              int64_t n, int k, int newest, PostStats* st) {
-    const int D = k * OD, lanes = blockDim.x / D, t = threadIdx.x;
+    const int D = k * F, lanes = blockDim.x / D, t = threadIdx.x;
     if (t >= lanes * D) return;
-    const int r = t / D, f = t % D, d = f / OD, c = f % OD;  // here f enumerates (lag d, channel c)
+    const int r = t / D, f = t % D, d = f / F, c = f % F;  // here f enumerates (lag d, channel c)
     const float* src = frames + (int64_t)ring_slot(newest, d, k) * plane + c;
     double s = 0.0, q = 0.0;
     for (int64_t e = (int64_t)blockIdx.x * lanes + r; e < n; e += (int64_t)gridDim.x * lanes)
-        if (d <= (int)age[e]) { const double v = (double)src[e * OD]; s += v; q += v * v; }
+        if (d <= (int)age[e]) { const double v = (double)src[e * F]; s += v; q += v * v; }
     atomicAdd(&st->chk_S[d][c], s); atomicAdd(&st->chk_Q[d][c], q);
 }
 
 }  // namespace
 
 struct hlynr_post {
-    int64_t n = 0, plane = 0;   // plane = floats per ring slot (n * 26 rounded up to 16-byte multiples)
-    int device = 0, k = 1, D = OD;
+    int64_t n = 0, plane = 0;   // plane = floats per ring slot (n * fw rounded up to 128-byte multiples)
+    int device = 0, fw = OD, k = 1, D = OD;   // frame width (26 or 17), n_stack, fw * n_stack
     double clip = 10.0, eps = 1e-8, gamma = 0.99;
     float* frames = nullptr;
     uint8_t* age[2] = {nullptr, nullptr};
@@ -318,11 +366,96 @@ static int blocks_for(const hlynr_post* p, int64_t items, int per_block) {
     return b < 1 ? 1 : (int)b;
 }
 
+template <int F>
+static int launch_normalize_t(hlynr_post* p, float* out, int raw, cudaStream_t st) {
+    const int newest = (int)((p->t - 1) % (uint32_t)p->k);
+    if constexpr (F % 2 == 0) {
+        const int P = p->D / 2;
+        const int lanes = 512 / P > 0 ? 512 / P : 1;
+        normalize_kernel<<<blocks_for(p, (p->n + NORM_UNROLL - 1) / NORM_UNROLL, lanes), lanes * P, 0, st>>>(
+            p->frames, p->plane, p->age[p->age_cur], p->st, out, p->n, p->k, newest, (float)p->clip, raw);
+    } else {
+        const int lanes = 512 / p->D;
+        normalize1_kernel<F><<<blocks_for(p, (p->n + NORM_UNROLL - 1) / NORM_UNROLL, lanes), lanes * p->D, 0, st>>>(
+            p->frames, p->plane, p->age[p->age_cur], p->st, out, p->n, p->k, newest, (float)p->clip, raw);
+    }
+    CK(cudaGetLastError());
+    p->launches += 1;
+    return 0;
+}
+
+static int launch_normalize(hlynr_post* p, float* out, int raw, cudaStream_t st) {
+    return p->fw == OD ? launch_normalize_t<OD>(p, out, raw, st) : launch_normalize_t<17>(p, out, raw, st);
+}
+
+template <int F>
+static int reset_t(hlynr_post* p, float* out_dev, int training, cudaStream_t st) {
+    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
+    p->t += 1;
+    CK(cudaMemsetAsync(p->returns, 0, sizeof(double) * p->n, st));  // VecNormalize.reset: returns = zeros
+    const int nb_col = blocks_for(p, p->n, 16);
+    colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials);
+    fold_kernel<F><<<2 * F, 256, 0, st>>>(p->partials, nb_col, 0, 0, 0, p->st);
+    merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 1, 0, p->eps);
+    CK(cudaGetLastError());
+    p->launches += 3;
+    p->sums_valid = true;
+    CK(cudaMemsetAsync(p->age[p->age_cur], 0, p->n, st));  // VecFrameStack.reset: only the newest frame is valid
+    return launch_normalize_t<F>(p, out_dev, 0, st);
+}
+
+template <int F>
+static int step_t(hlynr_post* p, const float* reward_dev, const uint8_t* terminated_dev, const uint8_t* truncated_dev,
+                  const HlynrDoneRecord* records_dev, const int32_t* counter_dev, int32_t capacity, float* out_dev,
+                  float* terminal_out_dev, int training, bool can_maintain, cudaStream_t st) {
+    const int newest_old = (int)((p->t - 1) % (uint32_t)p->k);
+    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
+    const uint8_t* age_old = p->age[p->age_cur];
+    p->t += 1;
+    const int nb_ret = blocks_for(p, p->n, 256);
+    returns_kernel<F><<<nb_ret, 256, 0, st>>>(p->returns, reward_dev, terminated_dev, truncated_dev, p->n, p->gamma, p->partials, training,
+                                              age_old, p->age[p->age_cur ^ 1], p->k);
+    p->launches += 1;
+    if (can_maintain && p->sums_valid) {  // the sums follow the ring on every step; obs_rms / ret_rms only move when training
+        const int nb_col = blocks_for(p, p->n, 16);
+        colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials);
+        p->launches += 1;
+        const int per = (p->k - 1) * F;
+        if (p->k > 1) {
+            const int lanes = 512 / per;
+            done_corr_kernel<F><<<64, lanes * per, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->k, newest_old,
+                                                            p->partials);
+            p->launches += 1;
+        }
+        fold_kernel<F><<<2 * F + 2 + 2 * per, 256, 0, st>>>(p->partials, nb_col, training ? nb_ret : 0, 64, per, p->st);
+        p->launches += 1;
+        merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 0, training, p->eps);
+        p->launches += 1;
+    } else {
+        p->sums_valid = false;
+    }
+    if (terminal_out_dev) {
+        const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
+        terminal_kernel<F><<<64, lanes * p->D, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->st, terminal_out_dev,
+                                                        p->k, newest_old, (float)p->clip);
+        p->launches += 1;
+    }
+    CK(cudaGetLastError());
+    p->age_cur ^= 1;  // returns_kernel wrote the new ages; done_corr / terminal above used the old ones
+    return launch_normalize_t<F>(p, out_dev, 0, st);
+}
+
 extern "C" {
 
 int hlynr_post_create(int64_t n_envs, int device, int n_stack, double clip_obs, double epsilon, double gamma, hlynr_post_t** out) {
+    return hlynr_post_create_frames(n_envs, device, OD, n_stack, clip_obs, epsilon, gamma, out);
+}
+
+int hlynr_post_create_frames(int64_t n_envs, int device, int frame_dim, int n_stack, double clip_obs, double epsilon, double gamma,
+                             hlynr_post_t** out) {
     if (!out) return fail("hlynr_post_create: null argument");
     if (n_envs <= 0) return fail("hlynr_post_create: n_envs must be positive");
+    if (frame_dim != OD && frame_dim != 17) return fail("hlynr_post_create: frame_dim must be 26 or 17, got %d", frame_dim);
     if (n_stack < 1 || n_stack > KMAX) return fail("hlynr_post_create: n_stack must be in [1, %d]", KMAX);
     int ndev = 0;
     CK(cudaGetDeviceCount(&ndev));
@@ -330,9 +463,9 @@ int hlynr_post_create(int64_t n_envs, int device, int n_stack, double clip_obs, 
     DeviceGuard g(device);
     hlynr_post* p = new (std::nothrow) hlynr_post();
     if (!p) return fail("hlynr_post_create: out of host memory");
-    p->n = n_envs; p->device = device; p->k = n_stack; p->D = OD * n_stack;
+    p->n = n_envs; p->device = device; p->fw = frame_dim; p->k = n_stack; p->D = frame_dim * n_stack;
     p->clip = clip_obs; p->eps = epsilon; p->gamma = gamma;
-    p->plane = ((n_envs * OD + 31) / 32) * 32;  // every slot starts 128-byte aligned
+    p->plane = ((n_envs * frame_dim + 31) / 32) * 32;  // every slot starts 128-byte aligned
     cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device);
     cudaError_t e = cudaMalloc(&p->frames, sizeof(float) * p->plane * n_stack);
     if (e == cudaSuccess) e = cudaMalloc(&p->age[0], n_envs);
@@ -379,33 +512,11 @@ int hlynr_post_obs_target(hlynr_post_t* p, float** obs_dev) {
     return 0;
 }
 
-static int launch_normalize(hlynr_post* p, float* out, int raw, cudaStream_t st) {
-    const int P = p->D / 2;
-    const int lanes = 512 / P > 0 ? 512 / P : 1;
-    const int newest = (int)((p->t - 1) % (uint32_t)p->k);
-    normalize_kernel<<<blocks_for(p, (p->n + NORM_UNROLL - 1) / NORM_UNROLL, lanes), lanes * P, 0, st>>>(
-        p->frames, p->plane, p->age[p->age_cur], p->st, out, p->n, p->k, newest, (float)p->clip, raw);
-    CK(cudaGetLastError());
-    p->launches += 1;
-    return 0;
-}
-
 int hlynr_post_reset(hlynr_post_t* p, float* out_dev, int training, void* stream) {
     if (!p || !out_dev) return fail("hlynr_post_reset: null argument");
     DeviceGuard g(p->device);
     cudaStream_t st = (cudaStream_t)stream;
-    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
-    p->t += 1;
-    CK(cudaMemsetAsync(p->returns, 0, sizeof(double) * p->n, st));  // VecNormalize.reset: returns = zeros
-    const int nb_col = blocks_for(p, p->n, 16);
-    colsum_kernel<<<nb_col, 16 * OD, 0, st>>>(frame, p->n, p->partials);
-    fold_kernel<<<2 * OD, 256, 0, st>>>(p->partials, nb_col, 0, 0, 0, p->st);
-    merge_kernel<<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 1, 0, p->eps);
-    CK(cudaGetLastError());
-    p->launches += 3;
-    p->sums_valid = true;
-    CK(cudaMemsetAsync(p->age[p->age_cur], 0, p->n, st));  // VecFrameStack.reset: only the newest frame is valid
-    return launch_normalize(p, out_dev, 0, st);
+    return p->fw == OD ? reset_t<OD>(p, out_dev, training, st) : reset_t<17>(p, out_dev, training, st);
 }
 
 int hlynr_post_step(hlynr_post_t* p, const float* reward_dev, const uint8_t* terminated_dev, const uint8_t* truncated_dev,
@@ -420,41 +531,10 @@ int hlynr_post_step(hlynr_post_t* p, const float* reward_dev, const uint8_t* ter
     if (terminal_out_dev && (!records_dev || !counter_dev)) return fail("hlynr_post_step: terminal_out_dev needs the done list of the step");
     DeviceGuard g(p->device);
     cudaStream_t st = (cudaStream_t)stream;
-    const int newest_old = (int)((p->t - 1) % (uint32_t)p->k);
-    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
-    const uint8_t* age_old = p->age[p->age_cur];
-    p->t += 1;
-    const int nb_ret = blocks_for(p, p->n, 256);
-    returns_kernel<<<nb_ret, 256, 0, st>>>(p->returns, reward_dev, terminated_dev, truncated_dev, p->n, p->gamma, p->partials, training,
-                                           age_old, p->age[p->age_cur ^ 1], p->k);
-    p->launches += 1;
-    if (can_maintain && p->sums_valid) {  // the sums follow the ring on every step; obs_rms / ret_rms only move when training
-        const int nb_col = blocks_for(p, p->n, 16);
-        colsum_kernel<<<nb_col, 16 * OD, 0, st>>>(frame, p->n, p->partials);
-        p->launches += 1;
-        const int per = (p->k - 1) * OD;
-        if (p->k > 1) {
-            const int lanes = 512 / per;
-            done_corr_kernel<<<64, lanes * per, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->k, newest_old,
-                                                         p->partials);
-            p->launches += 1;
-        }
-        fold_kernel<<<2 * OD + 2 + 2 * per, 256, 0, st>>>(p->partials, nb_col, training ? nb_ret : 0, 64, per, p->st);
-        p->launches += 1;
-        merge_kernel<<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 0, training, p->eps);
-        p->launches += 1;
-    } else {
-        p->sums_valid = false;
-    }
-    if (terminal_out_dev) {
-        const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
-        terminal_kernel<<<64, lanes * p->D, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->st, terminal_out_dev,
-                                                     p->k, newest_old, (float)p->clip);
-        p->launches += 1;
-    }
-    CK(cudaGetLastError());
-    p->age_cur ^= 1;  // returns_kernel wrote the new ages; done_corr / terminal above used the old ones
-    return launch_normalize(p, out_dev, 0, st);
+    return p->fw == OD ? step_t<OD>(p, reward_dev, terminated_dev, truncated_dev, records_dev, counter_dev, capacity, out_dev,
+                                    terminal_out_dev, training, can_maintain, st)
+                       : step_t<17>(p, reward_dev, terminated_dev, truncated_dev, records_dev, counter_dev, capacity, out_dev,
+                                    terminal_out_dev, training, can_maintain, st);
 }
 
 int hlynr_post_original(hlynr_post_t* p, float* out_dev, void* stream) {
@@ -504,7 +584,8 @@ int hlynr_post_set_stats(hlynr_post_t* p, const double* mean, const double* var,
     const double tail[4] = {count, ret_mean, ret_var, ret_count};
     CK(cudaMemcpyAsync(&p->st->count, &tail[0], sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(&p->st->ret_mean, &tail[1], sizeof(double) * 3, cudaMemcpyHostToDevice, st));
-    merge_kernel<<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps);  // refresh inv_std
+    if (p->fw == OD) merge_kernel<OD><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps);  // refresh inv_std
+    else merge_kernel<17><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));  // `tail` is a stack array
     p->launches += 1;
@@ -518,8 +599,13 @@ int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, voi
     cudaStream_t st = (cudaStream_t)stream;
     CK(cudaMemsetAsync(p->st->chk_S, 0, sizeof(double) * KMAX * OD * 2, st));
     const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
-    recompute_sums_kernel<<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
-                                                                              (int)((p->t - 1) % (uint32_t)p->k), p->st);
+    const int newest = (int)((p->t - 1) % (uint32_t)p->k);
+    if (p->fw == OD)
+        recompute_sums_kernel<OD><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
+                                                                                      newest, p->st);
+    else
+        recompute_sums_kernel<17><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
+                                                                                      newest, p->st);
     CK(cudaGetLastError());
     p->launches += 1;
     PostStats* h = new (std::nothrow) PostStats();
@@ -529,7 +615,7 @@ int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, voi
     if (e != cudaSuccess) { delete h; return fail("hlynr_post_check_sums: %s", cudaGetErrorString(e)); }
     double m = 0.0;
     for (int d = 0; d < p->k; ++d)
-        for (int c = 0; c < OD; ++c) {
+        for (int c = 0; c < p->fw; ++c) {
             m = fmax(m, fabs(h->S[d][c] - h->chk_S[d][c]));
             m = fmax(m, fabs(h->Q[d][c] - h->chk_Q[d][c]));
         }

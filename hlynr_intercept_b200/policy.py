@@ -5,7 +5,8 @@ train_flat_ppo.py:37-85 CustomMLP as SB3 features extractor, :419-429 net_arch=[
 features, state-independent log_std): it is the fp32 definition the fused kernel is checked against and the container of the
 weights.  `FusedActorCritic` runs the same forward as ONE hand-written kernel (tcgen05 GEMMs with bf16 operands and fp32
 accumulation in TMEM, TMA-fed weight tiles, bias + LayerNorm + ReLU as the epilogue between layers, both heads, Gaussian
-sampling and log-probability) on device tensors, for `DeviceRolloutCollector`.
+sampling and log-probability) on device tensors, for `DeviceRolloutCollector`.  Its input width is that of the first Linear,
+1-256: 104 for frame_stack 4 of the 26-D observation, 68 for frame_stack 4 of the 17-D one, and so on.
 """
 import ctypes as C
 import math
@@ -83,9 +84,11 @@ def bf16_emulated_forward(net, obs):
 class FusedActorCritic:
     """hlynr_policy_* behind the policy interface DeviceRolloutCollector uses: __call__(obs) -> (actions, values, log_probs),
     value(obs), value_rows(obs, n_rows_dev).  `net` holds the weights (a ReferenceActorCritic, or any object with the same
-    attribute names, e.g. an SB3 policy: .features_extractor.network / .action_net / .value_net / .log_std)."""
+    attribute names, e.g. an SB3 policy: .features_extractor.network / .action_net / .value_net / .log_std).  The input width
+    `in_dim` is read from the first Linear."""
 
     fused = True
+    MAX_IN = 256   # HLYNR_POLICY_MAX_IN: four 64-wide K blocks of the first GEMM
 
     def __init__(self, net, device=0, seed=0):
         torch = _torch()
@@ -93,8 +96,9 @@ class FusedActorCritic:
         self.net = net
         self.device_index = int(device)
         self.device = torch.device("cuda", self.device_index)
+        self.in_dim = int(self._modules()[0][0].weight.shape[1])
         h = C.c_void_p()
-        _lib.check(self.L.hlynr_policy_create(self.device_index, C.byref(h)))
+        _lib.check(self.L.hlynr_policy_create_dim(self.device_index, self.in_dim, C.byref(h)))
         self.h = h
         self.seed = int(seed)
         self.calls = 0
@@ -110,9 +114,13 @@ class FusedActorCritic:
         mods = list(seq)
         lins = [m for m in mods if m.__class__.__name__ == "Linear"]
         lns = [m for m in mods if m.__class__.__name__ == "LayerNorm"]
-        if [tuple(m.weight.shape) for m in lins] != [(512, 104), (512, 512), (256, 512)] or len(lns) != 3:
-            raise NotImplementedError("the fused forward is built for the reference's default architecture: 104 -> [512, 512, 256] "
-                                      "with LayerNorm + ReLU (train_flat_ppo.py:410); other shapes run through torch")
+        shapes = [tuple(m.weight.shape) for m in lins]
+        in_dim = shapes[0][1] if shapes else 0
+        if (shapes != [(512, in_dim), (512, 512), (256, 512)] or not 1 <= in_dim <= FusedActorCritic.MAX_IN or len(lns) != 3
+                or getattr(self, "in_dim", in_dim) != in_dim):
+            raise NotImplementedError("the fused forward is built for the reference's default architecture: in_dim -> [512, 512, 256] "
+                                      "with LayerNorm + ReLU (train_flat_ppo.py:410), in_dim 1-256 and fixed for the handle; "
+                                      "other shapes run through torch")
         if tuple(net.action_net.weight.shape) != (6, 256) or tuple(net.value_net.weight.shape) != (1, 256):
             raise NotImplementedError("action_net must be Linear(256, 6) and value_net Linear(256, 1)")
         if any(m.weight is None or m.bias is None for m in lns):
@@ -150,13 +158,15 @@ class FusedActorCritic:
         return t
 
     def forward(self, obs, deterministic=False, n_rows_dev=None, want=("actions", "values", "logp"), out=None):
-        """obs: float32 cuda tensor [n, 104] (contiguous).  Returns (actions [n,6], values [n], log_probs [n]); the tensors are
+        """obs: float32 cuda tensor [n, in_dim] (contiguous).  Returns (actions [n,6], values [n], log_probs [n]); the tensors are
         reused by the next call.  n_rows_dev: optional int32 cuda tensor [1] limiting the rows that are computed.
         out: optional dict of caller tensors the kernel writes into directly ('actions', 'values', 'logp', 'mean', and
         'clipped' = the action clipped to [-1, 1]^6 as SB3 passes it to env.step), e.g. rows of a rollout buffer."""
         torch = _torch()
-        if not (obs.is_cuda and obs.dtype == torch.float32 and obs.dim() == 2 and obs.shape[1] == 104 and obs.is_contiguous()):
-            obs = obs.to(device=self.device, dtype=torch.float32).reshape(-1, 104).contiguous()
+        if obs.dim() == 0 or obs.shape[-1] != self.in_dim:
+            raise ValueError(f"obs rows must be {self.in_dim} wide (the policy's input width), got shape {tuple(obs.shape)}")
+        if not (obs.is_cuda and obs.dtype == torch.float32 and obs.dim() == 2 and obs.is_contiguous()):
+            obs = obs.to(device=self.device, dtype=torch.float32).reshape(-1, self.in_dim).contiguous()
         n = obs.shape[0]
         out = out or {}
 

@@ -6,8 +6,9 @@ The reference wraps its VecEnv as
 and loads the statistics for inference with VecNormalize.load(...); env.training = False (inference.py:455-471).
 This class keeps the same names (n_stack, training, norm_obs, clip_obs, epsilon, gamma, obs_rms, ret_rms,
 normalize_obs, get_original_obs) over include/hlynr_post.h: the simulator writes its observation straight into the
-frame ring, and one pass produces the stacked, normalised [N, 26*n_stack] tensor the policy consumes -- no host round
-trip, no np.roll of the stack.
+frame ring, and one pass produces the stacked, normalised [N, F*n_stack] tensor the policy consumes -- no host round
+trip, no np.roll of the stack.  F, the frame width, is the sim's obs_dim: 26, or 17 for the leading radar channels obs[0:17]
+of the pre-ground-radar models (HlynrSim(obs_dim=17)).
 """
 import ctypes as C
 
@@ -30,14 +31,17 @@ class HlynrObsPipeline:
             raise NotImplementedError("norm_reward=True is not on the reference's path (train_flat_ppo.py:395)")
         import torch
 
-        if getattr(sim, "obs_dim", abi.OBS_DIM) != abi.OBS_DIM:
-            raise ValueError("HlynrObsPipeline stacks the full 26-D frames: create the HlynrSim with obs_dim=26")
+        frame_dim = int(getattr(sim, "obs_dim", abi.OBS_DIM))
+        if frame_dim not in (abi.OBS_DIM, 17):
+            raise ValueError(f"HlynrObsPipeline stacks 26-D or 17-D frames, the sim writes {frame_dim}-D ones")
         self.sim, self.L, self._torch = sim, sim.L, torch
+        self.frame_dim = frame_dim
         self.n_stack, self.training, self.norm_obs = int(n_stack), bool(training), bool(norm_obs)
         self.clip_obs, self.clip_reward, self.gamma, self.epsilon = float(clip_obs), float(clip_reward), float(gamma), float(epsilon)
-        self.obs_dim = abi.OBS_DIM * self.n_stack
+        self.obs_dim = frame_dim * self.n_stack
         h = C.c_void_p()
-        _lib.check(self.L.hlynr_post_create(sim.n, sim.device_index, self.n_stack, self.clip_obs, self.epsilon, self.gamma, C.byref(h)))
+        _lib.check(self.L.hlynr_post_create_frames(sim.n, sim.device_index, frame_dim, self.n_stack, self.clip_obs, self.epsilon,
+                                                   self.gamma, C.byref(h)))
         self.h = h
         n, d = sim.n, sim.device
         self._out = torch.empty((n, self.obs_dim), dtype=torch.float32, device=d)
@@ -72,7 +76,7 @@ class HlynrObsPipeline:
         return out
 
     def reset(self, out=None):
-        """VecFrameStack.reset + VecNormalize.reset: returns the stacked, normalised observation [N, 26*n_stack]
+        """VecFrameStack.reset + VecNormalize.reset: returns the stacked, normalised observation [N, F*n_stack]
         (written into `out` if given, e.g. a row of a rollout buffer)."""
         dst = self._out if out is None else self._check_out(out, (self.sim.n, self.obs_dim))
         _lib.check(self.L.hlynr_reset(self.sim.h, None, self._target(), self._stream()))
@@ -80,9 +84,9 @@ class HlynrObsPipeline:
         return dst
 
     def step(self, actions, auto_reset=True, out=None, reward_out=None):
-        """One tick + post-processing.  Returns (obs[N, 26k], reward[N], terminated[N], truncated[N], done) where
+        """One tick + post-processing.  Returns (obs[N, Fk], reward[N], terminated[N], truncated[N], done) where
         `done` = (records uint8 tensor viewable with abi.done_record_numpy_dtype, counter int32[1],
-        terminal_obs[capacity, 26k] or None): row r of terminal_obs is the stacked + normalised
+        terminal_obs[capacity, Fk] or None): row r of terminal_obs is the stacked + normalised
         info['terminal_observation'] of record r.  All tensors are overwritten by the next call."""
         t, sim = self._torch, self.sim
         if not (actions.is_cuda and actions.dtype == t.float32 and actions.shape == (sim.n, 6) and actions.is_contiguous()):
@@ -119,7 +123,7 @@ class HlynrObsPipeline:
         return self._orig
 
     def normalize_obs(self, stacked):
-        """VecNormalize.normalize_obs on a cuda float32 tensor [rows, 26*n_stack]."""
+        """VecNormalize.normalize_obs on a cuda float32 tensor [rows, F*n_stack]."""
         t = self._torch
         x = stacked.to(device=self.sim.device, dtype=t.float32).reshape(-1, self.obs_dim).contiguous()
         out = t.empty_like(x)
@@ -151,13 +155,17 @@ class HlynrObsPipeline:
         return _Rms(s["ret_mean"], s["ret_var"], s["ret_count"])
 
     def save(self, path):
-        """Statistics + hyper-parameters as .npz (the fields VecNormalize.__getstate__ pickles)."""
+        """Statistics + hyper-parameters as .npz (the fields VecNormalize.__getstate__ pickles, and the frame width)."""
         s = self.get_stats()
-        np.savez(path, n_stack=self.n_stack, clip_obs=self.clip_obs, clip_reward=self.clip_reward, gamma=self.gamma,
-                 epsilon=self.epsilon, norm_obs=self.norm_obs, **s)
+        np.savez(path, n_stack=self.n_stack, frame_dim=self.frame_dim, clip_obs=self.clip_obs, clip_reward=self.clip_reward,
+                 gamma=self.gamma, epsilon=self.epsilon, norm_obs=self.norm_obs, **s)
 
     def load(self, path):
+        """Statistics saved by save(); a file without a frame width is from a 26-D pipeline."""
         z = np.load(path)
+        frame_dim = int(z["frame_dim"]) if "frame_dim" in z.files else abi.OBS_DIM
+        if frame_dim != self.frame_dim:
+            raise ValueError(f"the statistics are of {frame_dim}-D frames, this pipeline stacks {self.frame_dim}-D ones")
         assert int(z["n_stack"]) == self.n_stack, "frame_stack of the statistics differs"
         self.set_stats(z["mean"], z["var"], float(z["count"]), float(z["ret_mean"]), float(z["ret_var"]), float(z["ret_count"]))
 

@@ -5,7 +5,7 @@
  *   reference interface                                                                    replaced by
  *   ------------------------------------------------------------------------------------  ----------------------
  *   CustomMLP.forward            rl_system/scripts/train_flat_ppo.py:37-85                 hlynr_policy_forward
- *     (104 -> Linear 512 -> LayerNorm -> ReLU -> Linear 512 -> LayerNorm -> ReLU -> Linear 256 -> LayerNorm -> ReLU)
+ *     (in_dim -> Linear 512 -> LayerNorm -> ReLU -> Linear 512 -> LayerNorm -> ReLU -> Linear 256 -> LayerNorm -> ReLU)
  *   SB3 ActorCriticPolicy heads with net_arch=[] (train_flat_ppo.py:419-429): action_net
  *     Linear(256, 6), value_net Linear(256, 1), state-independent log_std; forward() samples
  *     a = mean + exp(log_std) * eps and returns (a, V, log pi(a))                          hlynr_policy_forward
@@ -16,8 +16,9 @@
  * the tcgen05 tensor cores (bf16 operands, fp32 accumulators in TMEM), weight tiles arrive by TMA into a shared-memory
  * ring, and bias + LayerNorm + ReLU is the epilogue that turns the TMEM accumulators of one layer into the bf16 A operand
  * of the next without leaving the SM.  Conventions as in hlynr.h (plain pointers, 0 = success, hlynr_last_error()).
- * The architecture is the reference's default (train_flat_ppo.py:410 net_arch [512, 512, 256], frame_stack 4 x 26-D);
- * other shapes are rejected.
+ * The hidden layers and heads are the reference's default (train_flat_ppo.py:410 net_arch [512, 512, 256], 6 actions); the
+ * input width in_dim is that of the stacked observation, 1-256: 104 = frame_stack 4 x 26-D (the default), 68 = 4 x 17-D, and
+ * every other frame_stack of either frame width.  Other shapes are rejected.
  */
 #ifndef HLYNR_POLICY_H
 #define HLYNR_POLICY_H
@@ -29,7 +30,8 @@
 extern "C" {
 #endif
 
-#define HLYNR_POLICY_IN 104   /* 4 stacked 26-D frames */
+#define HLYNR_POLICY_IN 104   /* 4 stacked 26-D frames: the default input width */
+#define HLYNR_POLICY_MAX_IN 256   /* widest input: four 64-wide K blocks of the first GEMM */
 #define HLYNR_POLICY_H1 512
 #define HLYNR_POLICY_H2 512
 #define HLYNR_POLICY_H3 256
@@ -40,7 +42,7 @@ typedef struct hlynr_policy hlynr_policy_t;
 /* fp32 parameters in PyTorch layout (nn.Linear.weight is [out, in]); device pointers, copied (as bf16 for the GEMM operands)
  * by hlynr_policy_set_weights, so the caller's tensors may change afterwards. */
 typedef struct HlynrPolicyWeights {
-    const float *w1, *b1, *ln1_g, *ln1_b;   /* [512,104], [512] x3 */
+    const float *w1, *b1, *ln1_g, *ln1_b;   /* [512,in_dim], [512] x3 */
     const float *w2, *b2, *ln2_g, *ln2_b;   /* [512,512], [512] x3 */
     const float *w3, *b3, *ln3_g, *ln3_b;   /* [256,512], [256] x3 */
     const float *wa, *ba;                   /* action_net [6,256], [6] */
@@ -49,11 +51,15 @@ typedef struct HlynrPolicyWeights {
     float ln_eps;                           /* nn.LayerNorm eps (1e-5) */
 } HlynrPolicyWeights;
 
+/* A network with input width in_dim in [1, HLYNR_POLICY_MAX_IN]. */
+int hlynr_policy_create_dim(int device, int in_dim, hlynr_policy_t** out);
+/* hlynr_policy_create_dim with in_dim = HLYNR_POLICY_IN (104). */
 int hlynr_policy_create(int device, hlynr_policy_t** out);
 void hlynr_policy_destroy(hlynr_policy_t* p);
 int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, void* stream);
 
-/* Forward of rows [0, n_rows) of obs_dev float[n_rows, 104].
+/* Forward of rows [0, n_rows) of obs_dev float[n_rows, in_dim]: rows of pitch in_dim floats.  obs_dev must be 16-byte aligned
+ * for in_dim = 104 and 4-byte aligned for every other width (a row of a [T + 1, N, in_dim] rollout buffer).
  *   n_rows_dev   NULL, or a device int32: only min(n_rows, *n_rows_dev) rows are computed (tiles beyond it exit at once);
  *                lets the value net run on "the finished episodes of this step" without a host round trip
  *   actions_dev  float[n_rows, 6] or NULL: mean + exp(log_std) * eps (deterministic != 0: the mean)

@@ -9,12 +9,13 @@
  *   VecNormalize.load(...); env.training = False       rl_system/inference.py:455-471      hlynr_post_set_stats, training = 0
  *   VecNormalize.normalize_obs / get_original_obs                                           hlynr_post_normalize / _original
  *
- * Layout: the last n_stack raw frames live in a ring of [n_stack][N][26] planes; hlynr_step / hlynr_reset write their
- * observation STRAIGHT into the ring slot hlynr_post_obs_target returns (no copy), a per-env age byte says how many
- * older frames are valid since the env's last reset (SB3 zeroes the stack of a finished env), and the stacked,
- * normalised [N, 26*n_stack] observation is produced in one pass.  The running mean/variance (float64, SB3's
+ * Layout: the last n_stack raw frames live in a ring of [n_stack][N][F] planes, F = the frame width: 26 (the full
+ * observation) or 17 (the leading radar channels obs[0:17] a sim with option "obs_dim" = 17 writes); hlynr_step /
+ * hlynr_reset write their observation STRAIGHT into the ring slot hlynr_post_obs_target returns (no copy), a per-env age
+ * byte says how many older frames are valid since the env's last reset (SB3 zeroes the stack of a finished env), and the
+ * stacked, normalised [N, F*n_stack] observation is produced in one pass.  The running mean/variance (float64, SB3's
  * RunningMeanStd) is updated from per-lag column sums that are maintained incrementally: only the new frame is summed
- * (104 B per env) and the frames of the few finished envs are subtracted.
+ * (4F B per env) and the frames of the few finished envs are subtracted.
  *
  * Conventions as in hlynr.h: 0 = ok, message from hlynr_last_error(); device pointers are caller-owned; all work is
  * ordered on `stream`.
@@ -32,25 +33,29 @@ extern "C" {
 
 typedef struct hlynr_post hlynr_post_t;
 
-/* n_stack = VecFrameStack n_stack (1 = no stacking); clip_obs / epsilon / gamma = VecNormalize's (10.0, 1e-8, 0.99). */
+/* frame_dim = F, the width of one frame: 26, or 17 for a sim created with option "obs_dim" = 17;
+ * n_stack = VecFrameStack n_stack (1 = no stacking); clip_obs / epsilon / gamma = VecNormalize's (10.0, 1e-8, 0.99). */
+int hlynr_post_create_frames(int64_t n_envs, int device, int frame_dim, int n_stack, double clip_obs, double epsilon,
+                             double gamma, hlynr_post_t** out);
+/* hlynr_post_create_frames with frame_dim = 26. */
 int hlynr_post_create(int64_t n_envs, int device, int n_stack, double clip_obs, double epsilon, double gamma,
                       hlynr_post_t** out);
 void hlynr_post_destroy(hlynr_post_t* post);
-int hlynr_post_obs_dim(const hlynr_post_t* post, int* out); /* 26 * n_stack */
+int hlynr_post_obs_dim(const hlynr_post_t* post, int* out); /* F * n_stack */
 
-/* Device pointer (float[N,26]) the NEXT hlynr_reset / hlynr_step call must pass as obs_dev. */
+/* Device pointer (float[N,F]) the NEXT hlynr_reset / hlynr_step call must pass as obs_dev. */
 int hlynr_post_obs_target(hlynr_post_t* post, float** obs_dev);
 
 /* VecFrameStack.reset + VecNormalize.reset, after hlynr_reset(all envs) wrote into the target.
- * out_dev float[N, 26*n_stack]; training != 0 updates the running statistics with this batch. */
+ * out_dev float[N, F*n_stack]; training != 0 updates the running statistics with this batch. */
 int hlynr_post_reset(hlynr_post_t* post, float* out_dev, int training, void* stream);
 
 /* VecFrameStack.step_wait + VecNormalize.step_wait, after hlynr_step wrote into the target.
  *   reward_dev, terminated_dev, truncated_dev : outputs of that hlynr_step call
  *   records_dev, counter_dev, capacity        : its compact done list (hlynr_set_done_list), or NULL
- *   out_dev            float[N, 26*n_stack]   : stacked + normalised observation
- *   terminal_out_dev   float[capacity, 26*n_stack] or NULL: row r = stacked + normalised info['terminal_observation']
- *                      of records_dev[r]
+ *   out_dev            float[N, F*n_stack]   : stacked + normalised observation
+ *   terminal_out_dev   float[capacity, F*n_stack] or NULL: row r = stacked + normalised info['terminal_observation']
+ *                      of records_dev[r]; its newest frame is terminal_obs[0:F] of the record
  *   training           != 0: update obs_rms (and returns / ret_rms) with this batch before normalising */
 int hlynr_post_step(hlynr_post_t* post, const float* reward_dev, const uint8_t* terminated_dev,
                     const uint8_t* truncated_dev, const HlynrDoneRecord* records_dev, const int32_t* counter_dev,
@@ -58,10 +63,10 @@ int hlynr_post_step(hlynr_post_t* post, const float* reward_dev, const uint8_t* 
 
 /* VecNormalize.get_original_obs(): the stacked, un-normalised observation of the last reset/step. */
 int hlynr_post_original(hlynr_post_t* post, float* out_dev, void* stream);
-/* VecNormalize.normalize_obs on `rows` caller-provided stacked rows (float[rows, 26*n_stack], in place allowed). */
+/* VecNormalize.normalize_obs on `rows` caller-provided stacked rows (float[rows, F*n_stack], in place allowed). */
 int hlynr_post_normalize(hlynr_post_t* post, const float* stacked_dev, int64_t rows, float* out_dev, void* stream);
 
-/* obs_rms (mean/var: double[26*n_stack], count) and ret_rms (scalars); host pointers, any may be NULL.
+/* obs_rms (mean/var: double[F*n_stack], count) and ret_rms (scalars); host pointers, any may be NULL.
  * These are the fields of SB3's vec_normalize.pkl. */
 int hlynr_post_get_stats(hlynr_post_t* post, double* mean, double* var, double* count, double* ret_mean,
                          double* ret_var, double* ret_count, void* stream);
