@@ -23,7 +23,7 @@ EXPORTS = [
     "hlynr_post_step", "hlynr_post_original", "hlynr_post_normalize", "hlynr_post_get_stats", "hlynr_post_set_stats",
     "hlynr_post_check_sums", "hlynr_post_launch_count", "hlynr_post_note_replayed_steps",
     # include/hlynr_rollout.h
-    "hlynr_bootstrap_timeouts", "hlynr_gae",
+    "hlynr_bootstrap_timeouts", "hlynr_gae", "hlynr_eval_record",
     # include/hlynr_policy.h
     "hlynr_policy_create", "hlynr_policy_create_dim", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
 ]
@@ -102,6 +102,7 @@ def load(build_if_missing=True):
     L.hlynr_tick_count.argtypes = [vp, C.POINTER(i64)]
     L.hlynr_bootstrap_timeouts.argtypes = [vp, vp, vp, C.c_int32, vp, C.c_double, vp, i32, vp]
     L.hlynr_gae.argtypes = [vp, vp, vp, vp, vp, i64, i64, C.c_double, C.c_double, vp, vp, i32, vp]
+    L.hlynr_eval_record.argtypes = [vp, vp, i64, i64, vp, vp, vp, vp, vp, i32, vp]
     L.hlynr_policy_create.argtypes = [i32, C.POINTER(vp)]
     L.hlynr_policy_create_dim.argtypes = [i32, i32, C.POINTER(vp)]
     L.hlynr_policy_destroy.argtypes = [vp]

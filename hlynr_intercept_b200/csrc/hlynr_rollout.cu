@@ -1,6 +1,7 @@
-// hlynr_rollout.cu -- timeout bootstrapping and GAE(lambda) on the device (C ABI: include/hlynr_rollout.h).
-// Restated from stable-baselines3 2.x: common/on_policy_algorithm.py collect_rollouts, common/buffers.py
-// RolloutBuffer.compute_returns_and_advantage (float32 arrays, Python-float gamma / gae_lambda).
+// hlynr_rollout.cu -- timeout bootstrapping, GAE(lambda) and evaluation episode quotas on the device (C ABI:
+// include/hlynr_rollout.h).  Restated from stable-baselines3 2.x: common/on_policy_algorithm.py collect_rollouts,
+// common/buffers.py RolloutBuffer.compute_returns_and_advantage (float32 arrays, Python-float gamma / gae_lambda),
+// common/evaluation.py evaluate_policy.
 #include <cuda_runtime.h>
 
 #include "../../include/hlynr_rollout.h"
@@ -37,6 +38,33 @@ __global__ void bootstrap_kernel(float* __restrict__ rewards, const HlynrDoneRec
         }
         if (missed) atomicAdd(overflow, missed);
     }
+}
+
+// evaluate_policy's quota accounting: an env has at most one record per step, so its counts / ticks words are touched by one
+// thread only; results are addressed by (env, episode index) instead of appended, which makes the table independent of the
+// unspecified order of the records within a step
+__global__ void eval_record_kernel(const HlynrDoneRecord* __restrict__ recs, const int32_t* __restrict__ counter, int64_t n_envs,
+                                   int64_t q, int64_t rem, int32_t* __restrict__ counts, int64_t* __restrict__ ticks,
+                                   HlynrDoneRecord* __restrict__ results, int64_t* __restrict__ end_tick,
+                                   unsigned long long* remaining) {
+    const int64_t count = *counter;
+    const int64_t m = count < n_envs ? count : n_envs;
+    const int64_t full = n_envs - rem;   // targets: q for envs [0, full), q + 1 for envs [full, n_envs)
+    int taken = 0;
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < m; r += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t e = recs[r].env;
+        const int32_t c = counts[e];
+        if (c >= (e < full ? q : q + 1)) continue;   // past the env's quota: SB3 ignores the episode
+        const int64_t t = ticks[e] + recs[r].steps;   // auto-reset starts the next episode on the following step
+        const int64_t k = e * q + (e > full ? e - full : 0) + c;
+        results[k] = recs[r];
+        end_tick[k] = t;
+        ticks[e] = t;
+        counts[e] = c + 1;
+        ++taken;
+    }
+    taken = __reduce_add_sync(0xffffffffu, taken);   // every lane of every warp leaves the loop: blockDim is a multiple of 32
+    if (taken && (threadIdx.x & 31) == 0) atomicAdd(remaining, (unsigned long long)(-(long long)taken));
 }
 
 // one thread per env, reverse scan over T; every access is coalesced over N
@@ -89,6 +117,23 @@ int hlynr_gae(const float* rewards_dev, const float* values_dev, const float* ep
                                                                             advantages_dev, returns_dev);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail("hlynr_gae: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+int hlynr_eval_record(const HlynrDoneRecord* records_dev, const int32_t* counter_dev, int64_t n_envs, int64_t n_episodes,
+                      int32_t* counts_dev, int64_t* ticks_dev, HlynrDoneRecord* results_dev, int64_t* end_tick_dev,
+                      int64_t* remaining_dev, int device, void* stream) {
+    if (!records_dev || !counter_dev || !counts_dev || !ticks_dev || !results_dev || !end_tick_dev || !remaining_dev)
+        return fail("hlynr_eval_record: null argument");
+    if (n_envs <= 0 || n_envs > INT32_MAX) return fail("hlynr_eval_record: n_envs must be in [1, INT32_MAX]");
+    if (n_episodes <= 0 || n_episodes > INT32_MAX) return fail("hlynr_eval_record: n_episodes must be in [1, INT32_MAX]");
+    DeviceGuard g(device);
+    const int blocks = n_envs < 256 * 64 ? (int)((n_envs + 255) / 256) : 64;
+    eval_record_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(records_dev, counter_dev, n_envs, n_episodes / n_envs, n_episodes % n_envs,
+                                                                 counts_dev, ticks_dev, results_dev, end_tick_dev,
+                                                                 reinterpret_cast<unsigned long long*>(remaining_dev));
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail("hlynr_eval_record: %s", cudaGetErrorString(e));
     return 0;
 }
 

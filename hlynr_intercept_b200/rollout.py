@@ -150,34 +150,15 @@ class DeviceRolloutCollector:
 
     # ---- CUDA graph: the whole collect() (T x ~20 launches) as one graph launch --------------------------------------
     def graph_period(self):
-        """collect() can be captured once and replayed iff n_steps is a multiple of this (ring rows of the delay buffers,
-        frame-ring slot and the age ping-pong are kernel arguments derived from host-side tick counters)."""
-        per = C.c_int()
-        _lib.check(self.L.hlynr_ring_period(self.sim.h, C.byref(per)))
-        return math.lcm(per.value, self.pipe.n_stack, 2)
+        """collect() can be captured once and replayed iff n_steps is a multiple of this (see graph_period())."""
+        return graph_period(self.pipe)
 
     def capture(self):
         """Warm-up + stream capture of collect() into a CUDA graph (launch-bound at small n_envs: ~20 launches per step).
         The curriculum scalars and the seed are baked into the captured kernel arguments: re-capture after changing them."""
-        torch = _torch()
         if self.T % self.graph_period():
             raise ValueError(f"n_steps={self.T} must be a multiple of {self.graph_period()} to be graph-captured")
-        cur = torch.cuda.current_stream(self.sim.device)
-        side = torch.cuda.Stream(device=self.sim.device)
-        side.wait_stream(cur)
-        with torch.cuda.stream(side):
-            self.collect()   # allocations, cuBLAS workspaces, lazy module init
-        cur.wait_stream(side)
-        torch.cuda.synchronize(self.sim.device)
-        l0, p0 = self.sim.launch_count(), self.pipe.launch_count()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            self.collect()   # recorded, not executed: the host-side tick counters advance by T, the device state does not,
-        self._graph = g      # which is consistent because T is a multiple of every ring period
-        self._graph_launches = (self.sim.launch_count() - l0, self.pipe.launch_count() - p0)
-        # the recording advanced the host-side counters although nothing ran: undo (ring phases are unchanged, T % period == 0)
-        _lib.check(self.L.hlynr_note_replayed_ticks(self.sim.h, -self.T, -self._graph_launches[0]))
-        _lib.check(self.L.hlynr_post_note_replayed_steps(self.pipe.h, -self.T, -self._graph_launches[1]))
+        self._graph = TickGraph(self.pipe, self.T, self.collect)
         return self
 
     def replay(self):
@@ -185,6 +166,50 @@ class DeviceRolloutCollector:
         if self._graph is None:
             raise RuntimeError("capture() first")
         self._graph.replay()
-        _lib.check(self.L.hlynr_note_replayed_ticks(self.sim.h, self.T, self._graph_launches[0]))
-        _lib.check(self.L.hlynr_post_note_replayed_steps(self.pipe.h, self.T, self._graph_launches[1]))
         return self
+
+
+def graph_period(pipe):
+    """A captured sequence of ticks of `pipe` (HlynrObsPipeline) and its sim replays correctly iff its length is a multiple of
+    this: ring rows of the delay buffers, the frame-ring slot and the age ping-pong are kernel arguments derived from host-side
+    tick counters."""
+    per = C.c_int()
+    _lib.check(pipe.L.hlynr_ring_period(pipe.sim.h, C.byref(per)))
+    return math.lcm(per.value, pipe.n_stack, 2)
+
+
+class TickGraph:
+    """fn(), which runs `ticks` steps of `pipe` and its sim (and whatever else it launches on the current stream), as one CUDA
+    graph.  Construction runs fn() once for real on a side stream (allocations, cuBLAS workspaces, lazy module init), then
+    records it.  The recording advances the host-side tick counters although nothing runs; that is undone, and replay()
+    advances them by what the graph ran.  Both are consistent only because `ticks` is a multiple of graph_period(pipe): the
+    counters come back to the phases the captured kernel arguments were derived from."""
+
+    def __init__(self, pipe, ticks, fn):
+        torch = _torch()
+        self.pipe, self.sim, self.ticks = pipe, pipe.sim, int(ticks)
+        if self.ticks <= 0 or self.ticks % graph_period(pipe):
+            raise ValueError(f"{ticks} ticks must be a positive multiple of {graph_period(pipe)} to be graph-captured")
+        dev = self.sim.device
+        cur = torch.cuda.current_stream(dev)
+        side = torch.cuda.Stream(device=dev)
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            fn()
+        cur.wait_stream(side)
+        torch.cuda.synchronize(dev)
+        l0, p0 = self.sim.launch_count(), pipe.launch_count()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            fn()   # recorded, not executed
+        self.launches = (self.sim.launch_count() - l0, pipe.launch_count() - p0)
+        self._note(-1)
+
+    def _note(self, sign):
+        L = self.pipe.L
+        _lib.check(L.hlynr_note_replayed_ticks(self.sim.h, sign * self.ticks, sign * self.launches[0]))
+        _lib.check(L.hlynr_post_note_replayed_steps(self.pipe.h, sign * self.ticks, sign * self.launches[1]))
+
+    def replay(self):
+        self.graph.replay()
+        self._note(1)

@@ -9,6 +9,8 @@
  *       rewards[idx] += gamma * policy.predict_values(terminal_observation)"
  *   RolloutBuffer.compute_returns_and_advantage (GAE(lambda), called at rl_system/scripts/       hlynr_gae
  *       train_flat_ppo.py:431-448 through model.learn)
+ *   evaluate_policy's per-env episode quotas (EvalCallback, train_flat_ppo.py:497-504):          hlynr_eval_record
+ *       "if episode_counts[i] < episode_count_targets[i] and dones[i]: append info['episode']"
  *
  * Conventions as in hlynr.h.
  */
@@ -37,6 +39,21 @@ int hlynr_bootstrap_timeouts(float* rewards_dev, const HlynrDoneRecord* records_
 int hlynr_gae(const float* rewards_dev, const float* values_dev, const float* episode_starts_dev,
               const float* last_values_dev, const uint8_t* last_dones_dev, int64_t T, int64_t N, double gamma,
               double gae_lambda, float* advantages_dev, float* returns_dev, int device, void* stream);
+
+/* SB3 evaluate_policy's episode accounting: env e counts its first target_e = (n_episodes + e) / n_envs finished episodes.
+ * For each record r < min(*counter_dev, n_envs) of the step's done list (records_dev has n_envs entries) whose env e has
+ * counts_dev[e] < target_e:
+ *   ticks_dev[e] += steps;  k = offset_e + counts_dev[e];  results_dev[k] = record;  end_tick_dev[k] = ticks_dev[e];
+ *   counts_dev[e] += 1;     *remaining_dev -= 1
+ * offset_e = e*q + max(0, e - (n_envs - rem)), q = n_episodes / n_envs, rem = n_episodes % n_envs  (= sum of targets before e).
+ * Every env starts at the same reset and auto-reset starts its next episode on the following step, so end_tick_dev[k] is the
+ * step on which episode k ended, counted from that reset; SB3's list order is the sort by (end_tick, env).  The table does not
+ * depend on the order of the records within a step.  The caller zeroes counts_dev (int32[n_envs]) and ticks_dev (int64[n_envs])
+ * and sets *remaining_dev (int64) to n_episodes; results_dev / end_tick_dev have n_episodes entries.
+ * n_episodes must be in [1, INT32_MAX]. */
+int hlynr_eval_record(const HlynrDoneRecord* records_dev, const int32_t* counter_dev, int64_t n_envs, int64_t n_episodes,
+                      int32_t* counts_dev, int64_t* ticks_dev, HlynrDoneRecord* results_dev, int64_t* end_tick_dev,
+                      int64_t* remaining_dev, int device, void* stream);
 
 #ifdef __cplusplus
 }
