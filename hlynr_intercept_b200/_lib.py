@@ -25,7 +25,8 @@ EXPORTS = [
     # include/hlynr_rollout.h
     "hlynr_bootstrap_timeouts", "hlynr_gae", "hlynr_eval_record",
     # include/hlynr_policy.h
-    "hlynr_policy_create", "hlynr_policy_create_dim", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
+    "hlynr_policy_create", "hlynr_policy_create_dim", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_forward_dev",
+    "hlynr_policy_set_counter", "hlynr_policy_get_counter", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
 ]
 
 
@@ -109,6 +110,9 @@ def load(build_if_missing=True):
     L.hlynr_policy_destroy.restype = None
     L.hlynr_policy_set_weights.argtypes = [vp, C.POINTER(abi.HlynrPolicyWeights), vp]
     L.hlynr_policy_forward.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, u64, u64, i32, vp]
+    L.hlynr_policy_forward_dev.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, u64, i32, vp]
+    L.hlynr_policy_set_counter.argtypes = [vp, u64, vp]
+    L.hlynr_policy_get_counter.argtypes = [vp, C.POINTER(u64), vp]
     L.hlynr_policy_launch_count.argtypes = [vp, C.POINTER(i64)]
     L.hlynr_policy_set_option.argtypes = [vp, C.c_char_p, i64]
     L.hlynr_policy_get_timing.argtypes = [vp, vp]

@@ -63,6 +63,7 @@ constexpr int OFF_RING = A_BYTES;
 constexpr int OFF_STATS = OFF_RING + STAGES * STAGE_BYTES;      // float2[2][128]
 constexpr int OFF_BARS = OFF_STATS + 2 * BM * 8;                 // full[S], empty[S], a_ready, acc_ready
 constexpr int OFF_TMEM = OFF_BARS + (2 * STAGES + 2) * 8;
+constexpr int OFF_CTR = OFF_TMEM + 8;                            // this launch's call counter, read from the device (u64)
 constexpr int SMEM_BYTES = OFF_TMEM + 16;
 static_assert(SMEM_BYTES <= 232448, "shared memory budget of one CTA (227 KiB)");
 constexpr uint32_t TMEM_COLS = 512;
@@ -372,15 +373,30 @@ __device__ __forceinline__ void layer_epilogue(uint32_t lane_addr, uint32_t a_ba
     }
 }
 
+// Device-resident call counter: every launch advances it by exactly one, a launch that computes no row included.  Each CTA
+// reads it into shared memory (OFF_CTR, for its head epilogue), then arrives on the ticket; only the last arrival, after every
+// CTA has read the old value, stores the new one and re-arms the ticket.  A CTA with tiles does it in the shadow of its second
+// GEMM (4.7 us), where it costs nothing measurable: 206.1 against 206.3 us per forward at 131 072 rows (B200, 1000 W).  Placements
+// measured and dropped: at the start of the kernel, before the CTA-wide barrier, 1.8 us; in the shadow of the first GEMM, 0.7 us.
+__device__ __forceinline__ void counter_arrive(unsigned long long* ctr_dev, unsigned char* smem) {
+    unsigned int* ticket = reinterpret_cast<unsigned int*>(ctr_dev + 1);
+    const unsigned long long c = *reinterpret_cast<volatile unsigned long long*>(ctr_dev) + 1ull;
+    *reinterpret_cast<unsigned long long*>(smem + OFF_CTR) = c;
+    __threadfence();   // this CTA's read is ordered before its arrival
+    if (atomicAdd(ticket, 1u) == gridDim.x - 1u) { *ctr_dev = c; *ticket = 0u; }
+}
+
 // CL = CTAs per thread-block cluster (1, 2 or 4).  The CTAs of a cluster work on different row tiles in lock step and share
 // every weight tile: CTA r loads rows [r * N / CL, (r + 1) * N / CL) of a stage and multicasts them to all, so the L2 -> SM weight
 // traffic (904 KiB per 128-row tile, the kernel's bottleneck at CL = 1) is divided by CL.  A stage may be refilled only after the
 // MMAs of ALL CTAs have read it: the empty barriers count CL arrivals, delivered by multicast tcgen05.commit.
 // XW = IN: rows of exactly 104 floats, 16-byte aligned (the default network); XW = 0: any in_dim in [1, 256], rows 4-byte aligned.
+// ctr_dev: NULL (the counter is P.ctr_lo / P.ctr_hi), or the handle's {u64 counter, u32 ticket} block.  It is a kernel argument
+// of its own because two more fields in Params, even unused ones, made ptxas spill 80-96 B in the XW = 104 instantiations.
 template <int CL, int XW>
 __global__ void __launch_bounds__(THREADS, 1)   // (ptxas caps the registers per SM sub-partition: 3 of 10 warps x 168, 5 of 18 warps x 96)
 policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1,
-                      const __grid_constant__ CUtensorMap tm2, const __grid_constant__ CUtensorMap tm3, const Params P) {
+                      const __grid_constant__ CUtensorMap tm2, const __grid_constant__ CUtensorMap tm3, const Params P, unsigned long long* ctr_dev) {
     extern __shared__ __align__(1024) unsigned char smem[];
     const uint32_t sbase = smem_u32(smem);
     const uint32_t a_base = sbase, ring = sbase + OFF_RING, bars = sbase + OFF_BARS;
@@ -393,7 +409,10 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
     int64_t n_rows = P.n_rows;
     if (P.n_rows_dev) { const int64_t lim = (int64_t)*P.n_rows_dev; n_rows = lim < n_rows ? (lim < 0 ? 0 : lim) : n_rows; }
     const int64_t n_tiles = (n_rows + BM - 1) / BM;
-    if ((int64_t)(blockIdx.x / CL) * CL >= n_tiles) return;   // uniform for the whole cluster: nothing was allocated yet
+    if ((int64_t)(blockIdx.x / CL) * CL >= n_tiles) {   // uniform for the whole cluster: nothing was allocated yet
+        if (ctr_dev && threadIdx.x == 0) counter_arrive(ctr_dev, smem);   // a launch without rows advances the counter too
+        return;
+    }
     // every CTA that stays runs the same number of iterations (the ring protocol is cluster-wide); a tile index beyond n_tiles is
     // an all-padding tile: zero rows in, no rows out
     const int64_t n_iter = (n_tiles + gridDim.x - 1) / gridDim.x;
@@ -536,6 +555,8 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
                 fence_async_smem();
                 tc_fence_before();
                 mbar_arrive(bar_a);
+                // while the second GEMM runs; the head epilogue reads the counter after the next layers' bar.sync 1
+                if (it == 0 && l == 0 && ctr_dev && threadIdx.x == 0) counter_arrive(ctr_dev, smem);
                 if (tstamp) tstamp[3 + 2 * l] = clock64();
             }
             // heads
@@ -555,8 +576,13 @@ policy_forward_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_cons
                     for (int k = 0; k < ACT; ++k) { mean[k] = __uint_as_float(v[k]) + vf[VEC_BH + k]; eps[k] = 0.f; }
                     const float value = __uint_as_float(v[ACT]) + vf[VEC_BH + ACT];
                     if (!P.deterministic && (P.actions || P.logp || P.actions_clipped)) {
-                        const uint4 r0 = philox((uint32_t)grow, (uint32_t)((uint64_t)grow >> 32), P.ctr_lo, P.ctr_hi, P.k0, P.k1);
-                        const uint4 r1 = philox((uint32_t)grow, (uint32_t)((uint64_t)grow >> 32) | 0x80000000u, P.ctr_lo, P.ctr_hi, P.k0, P.k1);
+                        uint32_t clo = P.ctr_lo, chi = P.ctr_hi;
+                        if (ctr_dev) {
+                            const unsigned long long c = *reinterpret_cast<const unsigned long long*>(smem + OFF_CTR);
+                            clo = (uint32_t)c; chi = (uint32_t)(c >> 32);
+                        }
+                        const uint4 r0 = philox((uint32_t)grow, (uint32_t)((uint64_t)grow >> 32), clo, chi, P.k0, P.k1);
+                        const uint4 r1 = philox((uint32_t)grow, (uint32_t)((uint64_t)grow >> 32) | 0x80000000u, clo, chi, P.k0, P.k1);
                         box_muller(r0.x, r0.y, &eps[0], &eps[1]);
                         box_muller(r0.z, r0.w, &eps[2], &eps[3]);
                         box_muller(r1.x, r1.y, &eps[4], &eps[5]);
@@ -611,6 +637,11 @@ __global__ void copy_centred_f32_kernel(const float* __restrict__ src, float* __
     const float m = (float)(part[0] / n);
     for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = src[i] - m;
 }
+// the handle's {counter, ticket} block: a new counter value, and a ticket re-armed for the next forward
+__global__ void set_counter_kernel(unsigned long long* ctr, unsigned long long value) {
+    ctr[0] = value;
+    *reinterpret_cast<unsigned int*>(ctr + 1) = 0u;
+}
 __global__ void copy_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int n, int n_dst) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n_dst) dst[i] = i < n ? src[i] : 0.f;
@@ -634,6 +665,7 @@ struct hlynr_policy {
     __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wh = nullptr;   // [512,64*kb0], [512,512], [256,512], [16,256]
     float* vec = nullptr;   // b1 g1 be1 (512 x3) | b2 g2 be2 (512 x3) | b3 g3 be3 (256 x3) | bh (16) | log_std (8)
     int* error_flag = nullptr;
+    unsigned long long* ctr = nullptr;   // 16 bytes: the device-resident call counter (u64), then the forward's ticket (u32)
     long long* timing = nullptr;   // debug timestamps (option "timing")
     int timing_on = 0;
     CUtensorMap tm[3][4];   // [log2(cluster size)][layer]: box rows = N / cluster size
@@ -661,7 +693,7 @@ extern "C" {
 void hlynr_policy_destroy(hlynr_policy_t* p) {
     if (!p) return;
     DeviceGuard g(p->device);
-    cudaFree(p->w1); cudaFree(p->w2); cudaFree(p->w3); cudaFree(p->wh); cudaFree(p->vec); cudaFree(p->error_flag); cudaFree(p->timing);
+    cudaFree(p->w1); cudaFree(p->w2); cudaFree(p->w3); cudaFree(p->wh); cudaFree(p->vec); cudaFree(p->error_flag); cudaFree(p->ctr); cudaFree(p->timing);
     delete p;
 }
 
@@ -690,6 +722,8 @@ int hlynr_policy_create_dim(int device, int in_dim, hlynr_policy_t** out) {
     if (e == cudaSuccess) e = cudaMalloc(&p->vec, sizeof(float) * VEC_TOTAL);
     if (e == cudaSuccess) e = cudaMalloc(&p->error_flag, sizeof(int));
     if (e == cudaSuccess) e = cudaMemset(p->error_flag, 0, sizeof(int));
+    if (e == cudaSuccess) e = cudaMalloc(&p->ctr, 16);
+    if (e == cudaSuccess) e = cudaMemset(p->ctr, 0, 16);
     if (e != cudaSuccess) { const int r = fail("hlynr_policy_create: %s", cudaGetErrorString(e)); hlynr_policy_destroy(p); return r; }
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
@@ -744,15 +778,19 @@ int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, voi
     return 0;
 }
 
-int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev, float* actions_dev,
-                         float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev, uint64_t seed,
-                         uint64_t counter, int deterministic, void* stream) {
-    if (!p || !obs_dev) return fail("hlynr_policy_forward: null argument");
-    if (!p->ready) return fail("hlynr_policy_forward: hlynr_policy_set_weights has not been called");
-    if (n_rows <= 0) return fail("hlynr_policy_forward: n_rows must be positive");
+}  // extern "C"
+
+namespace {
+// hlynr_policy_forward (counter by value) and hlynr_policy_forward_dev (dev_counter: the handle's device-resident counter)
+int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev,
+                   float* actions_dev, float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev,
+                   uint64_t seed, uint64_t counter, bool dev_counter, int deterministic, void* stream) {
+    if (!p || !obs_dev) return fail("%s: null argument", fn);
+    if (!p->ready) return fail("%s: hlynr_policy_set_weights has not been called", fn);
+    if (n_rows <= 0) return fail("%s: n_rows must be positive", fn);
     const bool fixed = p->in_dim == IN;   // the 104-wide instantiation: float4 loads of 16-byte aligned rows
-    if (fixed && ((uintptr_t)obs_dev & 15u) != 0) return fail("hlynr_policy_forward: obs_dev must be 16-byte aligned");
-    if (((uintptr_t)obs_dev & 3u) != 0) return fail("hlynr_policy_forward: obs_dev must be 4-byte aligned");
+    if (fixed && ((uintptr_t)obs_dev & 15u) != 0) return fail("%s: obs_dev must be 16-byte aligned", fn);
+    if (((uintptr_t)obs_dev & 3u) != 0) return fail("%s: obs_dev must be 4-byte aligned", fn);
     DeviceGuard g(p->device);
     if (!p->smem_configured) {
         if (fixed) {
@@ -773,6 +811,7 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
     P.actions = actions_dev; P.values = values_dev; P.logp = logp_dev; P.mean = mean_dev; P.actions_clipped = actions_clipped_dev;
     P.ln_eps = p->ln_eps;
     P.k0 = (uint32_t)seed; P.k1 = (uint32_t)(seed >> 32); P.ctr_lo = (uint32_t)counter; P.ctr_hi = (uint32_t)(counter >> 32);
+    unsigned long long* ctr_dev = dev_counter ? p->ctr : nullptr;
     P.deterministic = deterministic; P.error_flag = p->error_flag;
     P.timing = p->timing_on ? p->timing : nullptr; P.timing_tiles = 8;
     const int64_t n_tiles = (n_rows + BM - 1) / BM;
@@ -805,17 +844,55 @@ int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows
     const CUtensorMap* tm = p->tm[ci];
     cudaError_t le;
     if (fixed) {
-        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, IN>, tm[0], tm[1], tm[2], tm[3], P);
-        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, IN>, tm[0], tm[1], tm[2], tm[3], P);
-        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, IN>, tm[0], tm[1], tm[2], tm[3], P);
+        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
+        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
+        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
     } else {
-        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, 0>, tm[0], tm[1], tm[2], tm[3], P);
-        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, 0>, tm[0], tm[1], tm[2], tm[3], P);
-        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, 0>, tm[0], tm[1], tm[2], tm[3], P);
+        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
+        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
+        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
     }
-    if (le != cudaSuccess) return fail("hlynr_policy_forward: launch failed: %s", cudaGetErrorString(le));
+    if (le != cudaSuccess) return fail("%s: launch failed: %s", fn, cudaGetErrorString(le));
     CK(cudaGetLastError());
     p->launches += 1;
+    return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev, float* actions_dev,
+                         float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev, uint64_t seed,
+                         uint64_t counter, int deterministic, void* stream) {
+    return launch_forward("hlynr_policy_forward", p, obs_dev, n_rows, n_rows_dev, actions_dev, values_dev, logp_dev, mean_dev,
+                          actions_clipped_dev, seed, counter, false, deterministic, stream);
+}
+
+int hlynr_policy_forward_dev(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev, float* actions_dev,
+                             float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev, uint64_t seed,
+                             int deterministic, void* stream) {
+    return launch_forward("hlynr_policy_forward_dev", p, obs_dev, n_rows, n_rows_dev, actions_dev, values_dev, logp_dev, mean_dev,
+                          actions_clipped_dev, seed, 0, true, deterministic, stream);
+}
+
+int hlynr_policy_set_counter(hlynr_policy_t* p, uint64_t value, void* stream) {
+    if (!p) return fail("hlynr_policy_set_counter: null argument");
+    DeviceGuard g(p->device);
+    set_counter_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(p->ctr, (unsigned long long)value);
+    CK(cudaGetLastError());
+    p->launches += 1;
+    return 0;
+}
+
+int hlynr_policy_get_counter(hlynr_policy_t* p, uint64_t* out, void* stream) {
+    if (!p || !out) return fail("hlynr_policy_get_counter: null argument");
+    DeviceGuard g(p->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    CK(cudaStreamSynchronize(st));
+    unsigned long long v = 0;
+    CK(cudaMemcpyAsync(&v, p->ctr, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    *out = (uint64_t)v;
     return 0;
 }
 

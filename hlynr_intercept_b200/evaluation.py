@@ -1,4 +1,4 @@
-"""Deterministic evaluation of a policy on the device: stable-baselines3's `evaluate_policy` over HlynrObsPipeline.
+"""Evaluation of a policy on the device: stable-baselines3's `evaluate_policy` over HlynrObsPipeline.
 
 The reference evaluates with `evaluate_policy(model, eval_env, n_eval_episodes, deterministic=True)` (EvalCallback,
 rl_system/scripts/train_flat_ppo.py:497-504; `inference.py --mode offline`) on a Monitor-wrapped, VecNormalize-wrapped eval env
@@ -8,9 +8,9 @@ stepping until every quota is met.  Counting "the first E episodes that finish" 
 intercept that fails early finishes first.  With fewer episodes than envs only the LAST n_eval_episodes envs are evaluated,
 as in SB3.
 
-One tick here is the deterministic forward (clip(mean, -1, 1)), `pipe.step` and `hlynr_eval_record`
-(include/hlynr_rollout.h), which files each counted episode's done record in a table addressed by (env, episode index), with
-the step it ended on.  The host reads one counter per chunk of ticks; with graph=True a chunk is one CUDA graph launch.
+One tick here is the policy's action clipped to [-1, 1] (the mean with deterministic=True, a sample otherwise), `pipe.step` and
+`hlynr_eval_record` (include/hlynr_rollout.h), which files each counted episode's done record in a table addressed by
+(env, episode index), with the step it ended on.  The host reads one counter per chunk of ticks; with graph=True a chunk is one CUDA graph launch.
 """
 import ctypes as C
 import dataclasses
@@ -55,11 +55,13 @@ class EvalResult:
 
 
 class DeviceEvaluator:
-    """evaluate_policy(policy, pipe, n_eval_episodes, deterministic=True) on device tensors.
+    """evaluate_policy(policy, pipe, n_eval_episodes, deterministic) on device tensors.
 
     pipe: an HlynrObsPipeline with training=False (load or sync its statistics first).
-    policy: a FusedActorCritic (one kernel writes clip(mean, -1, 1)) or a torch module with mean(obs), such as
-      ReferenceActorCritic; its input width must be pipe.obs_dim.
+    policy: a FusedActorCritic (one kernel writes the clipped action), or a torch module with mean(obs) for deterministic
+      evaluation and the collector's forward(obs) -> (actions, values, log_probs) for stochastic evaluation, such as
+      ReferenceActorCritic (both) or GaussianMlpPolicy (stochastic only); its input width must be pipe.obs_dim.  For a torch
+      module, value(obs) only marks the collector's interface: the forward's signature is not checked before the first tick.
     chunk: ticks between two reads of the remaining-episodes counter and the length of the CUDA graph; a multiple of
       graph_period(pipe).  Default: the smallest such multiple that is at least 16."""
 
@@ -71,10 +73,11 @@ class DeviceEvaluator:
         self.fused = bool(getattr(policy, "fused", False))
         if self.fused:
             in_dim = policy.in_dim
-        elif hasattr(policy, "mean"):
+        elif hasattr(policy, "mean") or hasattr(policy, "value"):
             in_dim = next(p for p in policy.parameters() if p.dim() == 2).shape[1]
         else:
-            raise ValueError("policy must be a FusedActorCritic or a torch module with mean(obs)")
+            raise ValueError("policy must be a FusedActorCritic, or a torch module with mean(obs) or the rollout collector's "
+                             "forward(obs) -> (actions, values, log_probs) and value(obs)")
         if in_dim != pipe.obs_dim:
             raise ValueError(f"the policy takes {in_dim}-wide observations, the pipeline produces {pipe.obs_dim}-wide ones")
         period = graph_period(pipe)
@@ -89,14 +92,17 @@ class DeviceEvaluator:
         self.remaining = torch.zeros(1, dtype=torch.int64, device=dev)
         self._rec_dtype = abi.done_record_numpy_dtype()
         self._n_episodes, self._results, self._end_tick = 0, None, None
+        self._deterministic = True
 
     def _tick(self):
         torch, sim = _torch(), self.sim
         if self.fused:
-            self.policy.forward(self.obs, deterministic=True, want=(), out=dict(clipped=self.actions))
+            self.policy.forward(self.obs, deterministic=self._deterministic, want=(), out=dict(clipped=self.actions))
             act = self.actions
-        else:
+        elif self._deterministic:
             act = self.policy.mean(self.obs).float().clamp(-1.0, 1.0)
+        else:   # SB3's predict(deterministic=False): a sample, clipped to the Box bounds
+            act = self.policy(self.obs)[0].float().clamp(-1.0, 1.0)
         _, _, _, _, (records, counter, _) = self.pipe.step(act, out=self.obs)
         p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
         _lib.check(sim.L.hlynr_eval_record(p(records), p(counter), sim.n, self._n_episodes, p(self.counts), p(self.ticks),
@@ -107,14 +113,22 @@ class DeviceEvaluator:
         for _ in range(self.chunk):
             self._tick()
 
-    def evaluate(self, n_eval_episodes, graph=True):
+    def evaluate(self, n_eval_episodes, graph=True, deterministic=True):
         """Resets the pipeline and runs until every env has finished its quota.  graph=True: chunks of `chunk` ticks, the
         first one eager, the others as replays of one CUDA graph, so `ticks` is a multiple of `chunk`; graph=False: the
-        counter is read after every tick and `ticks` is the step on which the last counted episode ended."""
+        counter is read after every tick and `ticks` is the step on which the last counted episode ended.
+        deterministic=False samples the action, as SB3's evaluate_policy(..., deterministic=False): the fused policy draws at
+        its device-side noise counter, one step per tick, so every graph replay draws fresh noise; a torch module draws from
+        torch's generator."""
         torch = _torch()
         E = int(n_eval_episodes)
         if not 1 <= E <= INT32_MAX:
             raise ValueError(f"n_eval_episodes must be in [1, {INT32_MAX}], got {n_eval_episodes}")
+        if not self.fused and not hasattr(self.policy, "mean" if deterministic else "value"):
+            raise ValueError("deterministic evaluation of a torch module needs its mean(obs)" if deterministic else
+                             "stochastic evaluation of a torch module needs the collector's forward(obs) -> (actions, values, "
+                             "log_probs) and value(obs)")
+        self._deterministic = bool(deterministic)
         n = self.sim.n
         # every episode ends within max_steps ticks, and an env needs at most ceil(E / n) of them
         limit = -(-E // n) * int(self.sim.params.max_steps) + self.chunk

@@ -101,12 +101,24 @@ class FusedActorCritic:
         _lib.check(self.L.hlynr_policy_create_dim(self.device_index, self.in_dim, C.byref(h)))
         self.h = h
         self.seed = int(seed)
-        self.calls = 0
         self._buf = {}
         self.sync_weights()
 
     def _stream(self):
         return C.c_void_p(_torch().cuda.current_stream(self.device).cuda_stream)
+
+    @property
+    def calls(self):
+        """The noise counter of the last forward: the next one draws at calls + 1.  It lives on the device and every forward
+        advances it there, so a forward captured in a CUDA graph draws fresh noise on every replay.  Reading it synchronises the
+        current stream; setting it is ordered on that stream."""
+        v = C.c_uint64()
+        _lib.check(self.L.hlynr_policy_get_counter(self.h, C.byref(v), self._stream()))
+        return v.value
+
+    @calls.setter
+    def calls(self, value):
+        _lib.check(self.L.hlynr_policy_set_counter(self.h, int(value), self._stream()))
 
     def _modules(self):
         net = self.net
@@ -160,6 +172,7 @@ class FusedActorCritic:
     def forward(self, obs, deterministic=False, n_rows_dev=None, want=("actions", "values", "logp"), out=None):
         """obs: float32 cuda tensor [n, in_dim] (contiguous).  Returns (actions [n,6], values [n], log_probs [n]); the tensors are
         reused by the next call.  n_rows_dev: optional int32 cuda tensor [1] limiting the rows that are computed.
+        Every call, of any kind, advances `calls` by one on the device and samples at the new value.
         out: optional dict of caller tensors the kernel writes into directly ('actions', 'values', 'logp', 'mean', and
         'clipped' = the action clipped to [-1, 1]^6 as SB3 passes it to env.step), e.g. rows of a rollout buffer."""
         torch = _torch()
@@ -181,9 +194,8 @@ class FusedActorCritic:
         a, v, lp, m = buf("actions", (n, 6)), buf("values", (n,)), buf("logp", (n,)), buf("mean", (n, 6))
         cl = buf("clipped", (n, 6))
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None  # noqa: E731
-        self.calls += 1
-        _lib.check(self.L.hlynr_policy_forward(self.h, ptr(obs), n, ptr(n_rows_dev), ptr(a), ptr(v), ptr(lp), ptr(m), ptr(cl), self.seed,
-                                               self.calls, int(bool(deterministic)), self._stream()))
+        _lib.check(self.L.hlynr_policy_forward_dev(self.h, ptr(obs), n, ptr(n_rows_dev), ptr(a), ptr(v), ptr(lp), ptr(m), ptr(cl),
+                                                   self.seed, int(bool(deterministic)), self._stream()))
         return (a, v, lp) if m is None else (a, v, lp, m)
 
     __call__ = forward

@@ -155,7 +155,9 @@ class DeviceRolloutCollector:
 
     def capture(self):
         """Warm-up + stream capture of collect() into a CUDA graph (launch-bound at small n_envs: ~20 launches per step).
-        The curriculum scalars and the seed are baked into the captured kernel arguments: re-capture after changing them."""
+        The curriculum scalars and the seed are baked into the captured kernel arguments: re-capture after changing them.
+        The fused policy's noise counter lives on the device and each forward advances it there, so every replay draws fresh
+        exploration noise, exactly as the same number of eager collects would."""
         if self.T % self.graph_period():
             raise ValueError(f"n_steps={self.T} must be a multiple of {self.graph_period()} to be graph-captured")
         self._graph = TickGraph(self.pipe, self.T, self.collect)

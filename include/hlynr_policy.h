@@ -68,10 +68,23 @@ int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, voi
  *   mean_dev     float[n_rows, 6] or NULL
  *   actions_clipped_dev float[n_rows, 6] or NULL: the sampled action clipped to the action space [-1, 1]^6 -- what SB3's
  *                collect_rollouts passes to env.step while the rollout buffer keeps the unclipped one
- *   seed, counter: eps comes from Philox4x32-10 keyed by seed with counter (row, counter): pass a new counter per call */
+ *   seed, counter: eps comes from Philox4x32-10 keyed by seed with counter (row, counter): pass a new counter per call.
+ * This entry never reads or changes the handle's device-resident counter (hlynr_policy_forward_dev). */
 int hlynr_policy_forward(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev,
                          float* actions_dev, float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev,
                          uint64_t seed, uint64_t counter, int deterministic, void* stream);
+
+/* hlynr_policy_forward with the call counter kept on the device: every launch draws at counter = *dev_counter + 1 and stores
+ * that value, for every kind of call (deterministic, value only, any *n_rows_dev, zero included), so a forward captured in a CUDA
+ * graph draws fresh noise on every replay.  The handle owns the counter (0 after hlynr_policy_create*).  Forwards through the
+ * device counter of one handle must be ordered on one stream: each launch reads the value the previous one stored. */
+int hlynr_policy_forward_dev(hlynr_policy_t* p, const float* obs_dev, int64_t n_rows, const int32_t* n_rows_dev,
+                             float* actions_dev, float* values_dev, float* logp_dev, float* mean_dev, float* actions_clipped_dev,
+                             uint64_t seed, int deterministic, void* stream);
+/* Sets the device-resident counter, ordered on `stream` (a one-thread kernel: value is a kernel argument, no host buffer). */
+int hlynr_policy_set_counter(hlynr_policy_t* p, uint64_t value, void* stream);
+/* Synchronises `stream` and returns the device-resident counter: the counter of the last forward_dev that ran on it. */
+int hlynr_policy_get_counter(hlynr_policy_t* p, uint64_t* out, void* stream);
 
 /* Options.  "cluster": CTAs per thread-block cluster, 1 (default), 2 or 4: the CTAs of a cluster share every weight tile through
  * TMA multicast, which divides the L2 -> SM weight traffic (the kernel's bottleneck without it) by the cluster size. */
