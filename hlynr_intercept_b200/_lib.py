@@ -18,6 +18,8 @@ EXPORTS = [
     "hlynr_stats_device_ptr", "hlynr_stats_reduce", "hlynr_get_stats", "hlynr_export_state", "hlynr_import_state",
     "hlynr_debug_draws", "hlynr_launch_count", "hlynr_set_option", "hlynr_set_done_list", "hlynr_done_records_host",
     "hlynr_ring_period", "hlynr_note_replayed_ticks", "hlynr_tick_count", "hlynr_pinned_done", "hlynr_host_done_buffer",
+    "hlynr_curriculum_schedule_size", "hlynr_attach_curriculum", "hlynr_detach_curriculum", "hlynr_set_timesteps", "hlynr_get_timesteps",
+    "hlynr_debug_curriculum_at",
     # include/hlynr_post.h
     "hlynr_post_create", "hlynr_post_create_frames", "hlynr_post_destroy", "hlynr_post_obs_dim", "hlynr_post_obs_target", "hlynr_post_reset",
     "hlynr_post_step", "hlynr_post_original", "hlynr_post_normalize", "hlynr_post_get_stats", "hlynr_post_set_stats",
@@ -56,12 +58,18 @@ def load(build_if_missing=True):
     L.hlynr_last_error.restype = C.c_char_p
     L.hlynr_params_size.restype = C.c_size_t
     L.hlynr_env_state_size.restype = C.c_size_t
+    L.hlynr_curriculum_schedule_size.restype = C.c_size_t
     L.hlynr_create.argtypes = [C.POINTER(abi.HlynrParams), i64, i32, u64, i64, i32, C.POINTER(vp)]
     L.hlynr_destroy.argtypes = [vp]
     L.hlynr_destroy.restype = None
     L.hlynr_num_envs.argtypes = [vp, C.POINTER(i64)]
     L.hlynr_set_curriculum.argtypes = [vp, C.POINTER(abi.HlynrCurriculum)]
     L.hlynr_get_curriculum.argtypes = [vp, C.POINTER(abi.HlynrCurriculum)]
+    L.hlynr_attach_curriculum.argtypes = [vp, C.POINTER(abi.HlynrCurriculumSchedule), u64, i64]
+    L.hlynr_detach_curriculum.argtypes = [vp]
+    L.hlynr_set_timesteps.argtypes = [vp, u64, vp]
+    L.hlynr_get_timesteps.argtypes = [vp, C.POINTER(u64), vp]
+    L.hlynr_debug_curriculum_at.argtypes = [vp, u64, C.POINTER(C.c_double)]
     L.hlynr_seed.argtypes = [vp, u64]
     L.hlynr_reset.argtypes = [vp, vp, vp, vp]
     L.hlynr_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(abi.HlynrInfoSoA), i32, vp]
@@ -122,6 +130,9 @@ def load(build_if_missing=True):
         raise HlynrError(f"HlynrParams layout mismatch: C {L.hlynr_params_size()} vs ctypes {C.sizeof(abi.HlynrParams)}")
     if L.hlynr_env_state_size() != C.sizeof(abi.HlynrEnvState):
         raise HlynrError("HlynrEnvState layout mismatch")
+    if L.hlynr_curriculum_schedule_size() != C.sizeof(abi.HlynrCurriculumSchedule):
+        raise HlynrError(f"HlynrCurriculumSchedule layout mismatch: C {L.hlynr_curriculum_schedule_size()} vs ctypes "
+                         f"{C.sizeof(abi.HlynrCurriculumSchedule)}")
     _LIB = L
     return L
 

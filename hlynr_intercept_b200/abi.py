@@ -57,6 +57,12 @@ class HlynrCurriculum(C.Structure):
                 ("onboard_reliability", C.c_double), ("ground_reliability", C.c_double)]
 
 
+class HlynrCurriculumSchedule(C.Structure):
+    _fields_ = [("enabled", C.c_int32), ("radar_enabled", C.c_int32),
+                ("initial_radius", C.c_double), ("final_radius", C.c_double), ("curriculum_steps", C.c_double)] + [
+        (f"{ramp}_{k}", C.c_double) for ramp in ("beam", "onboard", "ground") for k in ("initial", "final", "start", "end")]
+
+
 class HlynrInfoSoA(C.Structure):
     _fields_ = [("distance", C.c_void_p), ("min_distance", C.c_void_p), ("fuel_remaining", C.c_void_p),
                 ("fuel_used", C.c_void_p), ("steps", C.c_void_p), ("flags", C.c_void_p),

@@ -230,6 +230,33 @@ class Curriculum:
                                       rc.get("noise_transition_end", 7000000),
                                       rc.get("initial_noise_level", 0.0), rc.get("final_noise_level", 0.05))
 
+    def schedule(self):
+        """The whole schedule as an abi.HlynrCurriculumSchedule, for HlynrSim.track_training_steps: the device then computes
+        intercept_radius() and set_training_step_count() from its own counter, with the same double operations."""
+        s = abi.HlynrCurriculumSchedule()
+        s.enabled = int(self.use_curriculum)
+        s.initial_radius, s.final_radius = self.initial_radius, self.final_radius
+        s.curriculum_steps = float(self.curriculum_steps)
+        rc = self.rc
+        s.radar_enabled = int(self.use_radar_curriculum and bool(rc))
+        if s.radar_enabled:
+            ramps = dict(beam=("beam_width_transition_start", 3000000, "beam_width_transition_end", 5000000,
+                               "initial_beam_width", 120.0, "final_beam_width", 60.0),
+                         onboard=("reliability_transition_start", 4500000, "reliability_transition_end", 6000000,
+                                  "initial_detection_reliability", 1.0, "final_detection_reliability", 0.75),
+                         ground=("ground_reliability_transition_start", 4500000, "ground_reliability_transition_end", 6000000,
+                                 "initial_ground_reliability", 1.0, "final_ground_reliability", 0.85))
+            for name, (ks, ds, ke, de, ki, di, kf, df) in ramps.items():   # the keys and defaults of set_training_step_count
+                setattr(s, name + "_start", float(rc.get(ks, ds)))
+                setattr(s, name + "_end", float(rc.get(ke, de)))
+                setattr(s, name + "_initial", float(rc.get(ki, di)))
+                setattr(s, name + "_final", float(rc.get(kf, df)))
+        else:   # the values __init__ chose, constant
+            s.beam_initial = s.beam_final = self.beam_width
+            s.onboard_initial = s.onboard_final = float(self.onboard_reliability)
+            s.ground_initial = s.ground_final = float(self.ground_reliability)
+        return s
+
     def to_struct(self):
         c = abi.HlynrCurriculum()
         c.intercept_radius = float(self.intercept_radius())

@@ -220,6 +220,11 @@ struct hlynr_sim {
     int32_t done_cap = 0;
     uint8_t* io_done = nullptr;   // set by hlynr_step_host for the duration of the call
     uint8_t* host_done = nullptr; // caller's page-locked `dones` buffer (hlynr_host_done_buffer), NULL = the handle's own
+    // attached curriculum schedule (hlynr_attach_curriculum): a CurBlock<R> allocated on first attach and kept until hlynr_destroy
+    void* cur_block = nullptr;
+    bool cur_attached = false;
+    HlynrCurriculumSchedule sched;
+    int64_t cur_increment = 0;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -286,6 +291,60 @@ template <typename R> static KCurriculum<R> make_kcur(const HlynrCurriculum& c) 
     k.onboard_rel = (float)c.onboard_reliability; k.ground_rel = (float)c.ground_reliability;
     return k;
 }
+// ---- the curriculum schedule on the device --------------------------------------------------------------------------------
+// config.Curriculum in double, operation by operation: the explicit _rn intrinsics keep nvcc from contracting a*(1-t) + b*t into
+// an FMA, which would round once where Python rounds twice.  Counts are exact in double below 2^53, as in Python.
+__device__ double ramp_dev(double c, double start, double end, double a, double b) {   // Curriculum._ramp
+    if (c < start) return a;
+    if (c >= end) return b;
+    const double t = __ddiv_rn(__dsub_rn(c, start), __dsub_rn(end, start));
+    return __dadd_rn(__dmul_rn(a, __dsub_rn(1.0, t)), __dmul_rn(b, t));
+}
+template <typename R> __device__ KCurriculum<R> kcur_at(const HlynrCurriculumSchedule& s, unsigned long long count) {
+    const double c = (double)count;
+    double radius = s.final_radius, beam = s.beam_initial, onb = s.onboard_initial, gnd = s.ground_initial;
+    if (s.enabled) {   // Curriculum.intercept_radius
+        double progress = __ddiv_rn(c, s.curriculum_steps);
+        if (!(progress < 1.0)) progress = 1.0;   // Python min(1.0, x)
+        radius = __dadd_rn(__dmul_rn(s.initial_radius, __dsub_rn(1.0, progress)), __dmul_rn(s.final_radius, progress));
+    }
+    if (s.radar_enabled) {   // Curriculum.set_training_step_count
+        beam = ramp_dev(c, s.beam_start, s.beam_end, s.beam_initial, s.beam_final);
+        onb = ramp_dev(c, s.onboard_start, s.onboard_end, s.onboard_initial, s.onboard_final);
+        gnd = ramp_dev(c, s.ground_start, s.ground_end, s.ground_initial, s.ground_final);
+    }
+    KCurriculum<R> k;   // make_kcur
+    k.intercept_radius = (R)radius;
+    const double hb = __dmul_rn(__ddiv_rn(beam, 2.0), M_PI / 180.0);
+    k.cos_half_beam = hb >= M_PI ? -2.0f : (float)cos(hb);
+    k.onboard_rel = (float)onb; k.ground_rel = (float)gnd;
+    return k;
+}
+template <typename R> struct CurBlock {
+    unsigned long long num_timesteps;
+    KCurriculum<R> slot;
+};
+// Launched by hlynr_step before the step kernel (increment = the run's env count) and by hlynr_reset before the reset kernel
+// (increment 0), always WITHOUT programmatic serialization: it starts only once the previous kernel of the stream, which may be a
+// step kernel still reading the slot, has completed.  It lets the next launch be scheduled at once; that launch reads the slot
+// only after its griddepcontrol.wait, i.e. after this kernel has completed and its stores are visible (DESIGN section 15).
+template <typename R> __global__ void curriculum_tick_kernel(CurBlock<R>* b, const HlynrCurriculumSchedule s, unsigned long long increment) {
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    const unsigned long long c = b->num_timesteps;
+#ifdef HLYNR_CURRICULUM_TICK_DELAY_NS
+    // test hook, off in every ordinary build (tools/build_variant.py <tag> -DHLYNR_CURRICULUM_TICK_DELAY_NS=20000): holds the stores back
+    // so that a step kernel reading the slot before its griddepcontrol.wait would see the previous tick's values (DESIGN section 15)
+    for (int k = 0; k < HLYNR_CURRICULUM_TICK_DELAY_NS / 1000; ++k) __nanosleep(1000);
+#endif
+    b->slot = kcur_at<R>(s, c);
+    b->num_timesteps = c + increment;
+}
+template <typename R> __global__ void curriculum_probe_kernel(const HlynrCurriculumSchedule s, unsigned long long count, double* out) {
+    const KCurriculum<R> k = kcur_at<R>(s, count);
+    out[0] = (double)k.intercept_radius; out[1] = (double)k.cos_half_beam; out[2] = (double)k.onboard_rel; out[3] = (double)k.ground_rel;
+}
+__global__ void set_timesteps_kernel(unsigned long long* count, unsigned long long value) { *count = value; }
+
 static RoundKeys make_round_keys(uint64_t seed) {
     RoundKeys rk;
     uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
@@ -442,7 +501,17 @@ template <typename R> static KernelArgs<R> base_args(hlynr_sim* s, const StatePl
     A.prefetch_ahead = s->sm_count * s->prefetch_waves * HLYNR_BLOCK;
     A.obs_dim = s->obs_dim;
     A.compact = s->compact;
+    A.cur_dev = s->cur_attached ? &((CurBlock<R>*)s->cur_block)->slot : nullptr;
     return A;
+}
+// Before a step (increment = the attached increment) or a reset (0): the slot the next launch reads, and the count advanced.
+static int curriculum_tick(hlynr_sim* s, int64_t increment, cudaStream_t st) {
+    if (!s->cur_attached) return 0;
+    if (s->precision == HLYNR_FP32) curriculum_tick_kernel<float><<<1, 1, 0, st>>>((CurBlock<float>*)s->cur_block, s->sched, (unsigned long long)increment);
+    else curriculum_tick_kernel<double><<<1, 1, 0, st>>>((CurBlock<double>*)s->cur_block, s->sched, (unsigned long long)increment);
+    CK(cudaGetLastError());
+    s->launches += 1;
+    return 0;
 }
 static inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
 
@@ -465,7 +534,7 @@ static int feature_set(const HlynrParams& p) {
 // One launch of an instantiation.  pdl: programmatic dependent launch -- the grid may be scheduled while the previous kernel
 // of the stream is still draining; the kernel itself waits (griddepcontrol.wait, its first instruction that matters) until
 // that kernel has completed and its writes are visible, so only launch latency and the tail of the previous grid overlap.
-template <typename R, bool kRollout, int F> static void launch_inst(const KernelArgs<R>& A, int grid, cudaStream_t st, bool pdl) {
+template <typename R, bool kRollout, int F, bool kCur> static void launch_inst(const KernelArgs<R>& A, int grid, cudaStream_t st, bool pdl) {
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(HLYNR_STEP_BLOCK); cfg.dynamicSmemBytes = 0; cfg.stream = st;
@@ -473,7 +542,7 @@ template <typename R, bool kRollout, int F> static void launch_inst(const Kernel
         // resident CTAs per SM, which gives the sensitivity of the launch time to the number of resident warps
         static const int pad = getenv("HLYNR_OCC_PAD_BYTES") ? atoi(getenv("HLYNR_OCC_PAD_BYTES")) : 0;
         if (pad > 0) {
-            cudaFuncSetAttribute(step_kernel<R, kRollout, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, pad);
+            cudaFuncSetAttribute(step_kernel<R, kRollout, F, kCur>, cudaFuncAttributeMaxDynamicSharedMemorySize, pad);
             cfg.dynamicSmemBytes = (size_t)pad;
         }
     }
@@ -481,19 +550,26 @@ template <typename R, bool kRollout, int F> static void launch_inst(const Kernel
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = pdl ? 1u : 0u;
-    cudaLaunchKernelEx(&cfg, step_kernel<R, kRollout, F>, A);
+    cudaLaunchKernelEx(&cfg, step_kernel<R, kRollout, F, kCur>, A);
 }
-// Both builds dispatch to the feature-specialised instantiation of the three BASELINE configurations when it matches.
+template <typename R, bool kRollout, bool kCur> static void launch_feature(const KernelArgs<R>& A, int f, int grid, cudaStream_t st, bool pdl) {
+    if (f == FT_V2ON) launch_inst<R, kRollout, FT_V2ON, kCur>(A, grid, st, pdl);
+    else if (f == FT_V2OFF) launch_inst<R, kRollout, FT_V2OFF, kCur>(A, grid, st, pdl);
+    else if (f == FT_V2ON_DR) launch_inst<R, kRollout, FT_V2ON_DR, kCur>(A, grid, st, pdl);
+    else if (f == FT_GENERIC_MODES) launch_inst<R, kRollout, FT_GENERIC_MODES, kCur>(A, grid, st, pdl);
+    else launch_inst<R, kRollout, FT_GENERIC, kCur>(A, grid, st, pdl);
+}
+// Both builds dispatch to the feature-specialised instantiation of the three BASELINE configurations when it matches, and API-mode
+// ticks to the instantiation that reads the curriculum slot while a schedule is attached (hlynr_rollout refuses one).
 template <typename R, bool kRollout> static void launch_step(const hlynr_sim* s, const KernelArgs<R>& A, cudaStream_t st, bool specialise) {
     const int grid = grid_for(A.lim - A.first, HLYNR_STEP_BLOCK);
     const bool pdl = s->pdl != 0;
     int f = feature_set(s->params);
     if (!specialise && f >= 0) f = FT_GENERIC;
-    if (f == FT_V2ON) launch_inst<R, kRollout, FT_V2ON>(A, grid, st, pdl);
-    else if (f == FT_V2OFF) launch_inst<R, kRollout, FT_V2OFF>(A, grid, st, pdl);
-    else if (f == FT_V2ON_DR) launch_inst<R, kRollout, FT_V2ON_DR>(A, grid, st, pdl);
-    else if (f == FT_GENERIC_MODES) launch_inst<R, kRollout, FT_GENERIC_MODES>(A, grid, st, pdl);
-    else launch_inst<R, kRollout, FT_GENERIC>(A, grid, st, pdl);
+    if constexpr (!kRollout) {
+        if (A.cur_dev) { launch_feature<R, false, true>(A, f, grid, st, pdl); return; }
+    }
+    launch_feature<R, kRollout, false>(A, f, grid, st, pdl);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -505,11 +581,12 @@ const char* hlynr_last_error(void) { return g_err; }
 int hlynr_abi_version(void) { return HLYNR_ABI_VERSION; }
 size_t hlynr_params_size(void) { return sizeof(HlynrParams); }
 size_t hlynr_env_state_size(void) { return sizeof(HlynrEnvState); }
+size_t hlynr_curriculum_schedule_size(void) { return sizeof(HlynrCurriculumSchedule); }
 
 void hlynr_destroy(hlynr_t* s) {
     if (!s) return;
     DeviceGuard g(s->device);
-    cudaFree(s->state_mem); cudaFree(s->stats); cudaFree(s->xchg);
+    cudaFree(s->state_mem); cudaFree(s->stats); cudaFree(s->xchg); cudaFree(s->cur_block);
     HostIO& h = s->hio;
     delete h.pool;
     cudaFreeHost(h.h_actions); cudaFreeHost(h.h_obs); cudaFreeHost(h.h_reward); cudaFreeHost(h.h_records_ab[0]); cudaFreeHost(h.h_records_ab[1]); cudaFreeHost(h.h_count);
@@ -584,7 +661,14 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
 }
 
 int hlynr_num_envs(const hlynr_t* s, int64_t* out) { if (!s || !out) return fail("null argument"); *out = s->n; return 0; }
-int hlynr_set_curriculum(hlynr_t* s, const HlynrCurriculum* c) { if (!s || !c) return fail("null argument"); s->cur = *c; return 0; }
+int hlynr_set_curriculum(hlynr_t* s, const HlynrCurriculum* c) {
+    if (!s || !c) return fail("null argument");
+    if (s->cur_attached)
+        return fail("hlynr_set_curriculum: a curriculum schedule is attached and the device computes the curriculum from its counter: "
+                    "set the count with hlynr_set_timesteps, or hlynr_detach_curriculum first");
+    s->cur = *c;
+    return 0;
+}
 int hlynr_get_curriculum(const hlynr_t* s, HlynrCurriculum* c) { if (!s || !c) return fail("null argument"); *c = s->cur; return 0; }
 int hlynr_seed(hlynr_t* s, uint64_t seed) { if (!s) return fail("null handle"); s->seed = seed; return 0; }
 static int make_pool(hlynr_sim* s);
@@ -641,14 +725,17 @@ int hlynr_reset(hlynr_t* s, const uint8_t* mask_dev, float* obs_dev, void* strea
     if (!s) return fail("hlynr_reset: null handle");
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
+    if (curriculum_tick(s, 0, st)) return 1;   // the reference's reset uses the last pushed count and does not advance it
     if (s->precision == HLYNR_FP32) {
         KernelArgs<float> A = base_args<float>(s, s->pf);
         A.io.reset_mask = mask_dev; A.io.obs = obs_dev;
-        reset_kernel<float><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
+        if (A.cur_dev) reset_kernel<float, true><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
+        else reset_kernel<float><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
     } else {
         KernelArgs<double> A = base_args<double>(s, s->pd);
         A.io.reset_mask = mask_dev; A.io.obs = obs_dev;
-        reset_kernel<double><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
+        if (A.cur_dev) reset_kernel<double, true><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
+        else reset_kernel<double><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
     }
     CK(cudaGetLastError());
     s->launches += 1;
@@ -686,9 +773,69 @@ int hlynr_step(hlynr_t* s, const float* actions_dev, float* obs_dev, float* rewa
     if (!s) return fail("hlynr_step: null handle");
     if (!actions_dev || !obs_dev || !reward_dev || !terminated_dev || !truncated_dev) return fail("hlynr_step: null output/input pointer");
     DeviceGuard g(s->device);
+    if (curriculum_tick(s, s->cur_increment, (cudaStream_t)stream)) return 1;
     s->tick += 1;
     return step_range(s, 0, s->n, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, terminal_obs_dev, info,
                       auto_reset, (cudaStream_t)stream);
+}
+
+int hlynr_attach_curriculum(hlynr_t* s, const HlynrCurriculumSchedule* c, uint64_t num_timesteps, int64_t increment) {
+    if (!s || !c) return fail("hlynr_attach_curriculum: null argument");
+    const double f[] = {c->initial_radius, c->final_radius, c->curriculum_steps, c->beam_initial, c->beam_final, c->beam_start,
+                        c->beam_end, c->onboard_initial, c->onboard_final, c->onboard_start, c->onboard_end, c->ground_initial,
+                        c->ground_final, c->ground_start, c->ground_end};
+    for (double v : f)
+        if (!std::isfinite(v)) return fail("hlynr_attach_curriculum: every field of the schedule must be finite");
+    if (c->enabled && !(c->curriculum_steps > 0.0)) return fail("hlynr_attach_curriculum: curriculum_steps must be positive while the curriculum is enabled");
+    if (increment < 0) return fail("hlynr_attach_curriculum: increment must not be negative");
+    DeviceGuard g(s->device);
+    if (!s->cur_block) CK(cudaMalloc(&s->cur_block, sizeof(CurBlock<double>)));
+    CK(cudaDeviceSynchronize());   // no launch of an earlier attachment still reads or writes the block
+    const unsigned long long v = num_timesteps;
+    CK(cudaMemcpy(s->cur_block, &v, sizeof(v), cudaMemcpyHostToDevice));
+    s->sched = *c; s->cur_increment = increment; s->cur_attached = true;
+    return 0;
+}
+int hlynr_detach_curriculum(hlynr_t* s) {
+    if (!s) return fail("hlynr_detach_curriculum: null handle");
+    s->cur_attached = false;
+    return 0;
+}
+int hlynr_set_timesteps(hlynr_t* s, uint64_t num_timesteps, void* stream) {
+    if (!s) return fail("hlynr_set_timesteps: null handle");
+    if (!s->cur_attached) return fail("hlynr_set_timesteps: no curriculum schedule is attached (hlynr_attach_curriculum)");
+    DeviceGuard g(s->device);
+    set_timesteps_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((unsigned long long*)s->cur_block, (unsigned long long)num_timesteps);
+    CK(cudaGetLastError());
+    s->launches += 1;
+    return 0;
+}
+int hlynr_get_timesteps(hlynr_t* s, uint64_t* out, void* stream) {
+    if (!s || !out) return fail("hlynr_get_timesteps: null argument");
+    if (!s->cur_attached) return fail("hlynr_get_timesteps: no curriculum schedule is attached (hlynr_attach_curriculum)");
+    DeviceGuard g(s->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    CK(cudaStreamSynchronize(st));
+    unsigned long long v = 0;
+    CK(cudaMemcpyAsync(&v, s->cur_block, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    *out = (uint64_t)v;
+    return 0;
+}
+int hlynr_debug_curriculum_at(hlynr_t* s, uint64_t count, double out[4]) {
+    if (!s || !out) return fail("hlynr_debug_curriculum_at: null argument");
+    if (!s->cur_attached) return fail("hlynr_debug_curriculum_at: no curriculum schedule is attached (hlynr_attach_curriculum)");
+    DeviceGuard g(s->device);
+    double* buf = nullptr;
+    CK(cudaMalloc(&buf, 4 * sizeof(double)));
+    if (s->precision == HLYNR_FP32) curriculum_probe_kernel<float><<<1, 1>>>(s->sched, (unsigned long long)count, buf);
+    else curriculum_probe_kernel<double><<<1, 1>>>(s->sched, (unsigned long long)count, buf);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpy(out, buf, 4 * sizeof(double), cudaMemcpyDeviceToHost);
+    cudaFree(buf);
+    if (e != cudaSuccess) return fail("hlynr_debug_curriculum_at: %s", cudaGetErrorString(e));
+    s->launches += 1;
+    return 0;
 }
 
 int hlynr_set_done_list(hlynr_t* s, HlynrDoneRecord* records_dev, int32_t* counter_dev, int32_t capacity) {
@@ -702,6 +849,9 @@ int hlynr_rollout(hlynr_t* s, int k_steps, const float* actions_dev, float* obs_
                   int32_t* done_count_dev, void* stream) {
     if (!s) return fail("hlynr_rollout: null handle");
     if (k_steps <= 0) return fail("hlynr_rollout: k_steps must be positive");
+    if (s->cur_attached)
+        return fail("hlynr_rollout: not available while a curriculum schedule is attached (the fused ticks would each need their own "
+                    "curriculum slot): step with hlynr_step, or hlynr_detach_curriculum first");
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (s->precision == HLYNR_FP32) {
@@ -922,6 +1072,9 @@ int hlynr_reset_host(hlynr_t* s, const uint8_t* mask_host, float* obs_host) {
 int hlynr_step_host(hlynr_t* s, const float* actions_host, float* obs_host, float* reward_host, uint8_t* terminated_host,
                     uint8_t* truncated_host, float* terminal_obs_host, int auto_reset) {
     if (!s || !actions_host || !obs_host || !reward_host || !terminated_host || !truncated_host) return fail("hlynr_step_host: null argument");
+    if (s->cur_attached)
+        return fail("hlynr_step_host: not available while a curriculum schedule is attached: the host path takes its curriculum from "
+                    "hlynr_set_curriculum, which the host-side training callback drives; hlynr_detach_curriculum first");
     DeviceGuard g(s->device);
     if (ensure_hostio(s)) return 1;
     if (s->host_info && ensure_host_info(s)) return 1;

@@ -323,7 +323,30 @@ template <typename R> struct KernelArgs {
     int32_t prefetch_ahead;  // envs per resident wave of CTAs (0 = no L2 prefetch of the next wave's planes)
     int32_t obs_dim;         // row pitch of io.obs / io.terminal_obs: HLYNR_OBS_DIM, or 17 = the leading "17-D radar" channels only
     int32_t compact;         // compact plane layout (see load_env): the counters ride in r6.w / f1.w, the i0 plane is unused
+    // NULL = the curriculum is C.  Else the device slot curriculum_tick_kernel (hlynr_capi.cu) filled before this launch from the
+    // attached schedule's training-step counter, and the host launches the kCur instantiation, which reads it (cur_*() below).
+    const KCurriculum<R>* cur_dev;
 };
+
+// Curriculum scalars of a launch.  kCur = false: the by-value C, exactly the code of a build without schedules.  kCur = true (a
+// separate instantiation, launched while a schedule is attached): the slot at cur_dev, which the kernel launched right before this
+// one wrote, read at each use site and only after griddepcontrol.wait (nothing calls these earlier).  `ldu` is PTX's load of a
+// warp-uniform read-only address; volatile so that the compiler neither hoists it above the wait nor keeps the value in a register
+// across the tick (the step kernel holds 112 registers with no spills).
+HD float ldu_slot(const float* p) { float v; asm volatile("ldu.global.f32 %0, [%1];" : "=f"(v) : "l"(p)); return v; }
+HD double ldu_slot(const double* p) { double v; asm volatile("ldu.global.f64 %0, [%1];" : "=d"(v) : "l"(p)); return v; }
+template <bool kCur, typename R> HD R cur_radius(const KernelArgs<R>& A) {
+    if constexpr (kCur) return ldu_slot(&A.cur_dev->intercept_radius); else return A.C.intercept_radius;
+}
+template <bool kCur, typename R> HD float cur_cos_half_beam(const KernelArgs<R>& A) {
+    if constexpr (kCur) return ldu_slot(&A.cur_dev->cos_half_beam); else return A.C.cos_half_beam;
+}
+template <bool kCur, typename R> HD float cur_onboard_rel(const KernelArgs<R>& A) {
+    if constexpr (kCur) return ldu_slot(&A.cur_dev->onboard_rel); else return A.C.onboard_rel;
+}
+template <bool kCur, typename R> HD float cur_ground_rel(const KernelArgs<R>& A) {
+    if constexpr (kCur) return ldu_slot(&A.cur_dev->ground_rel); else return A.C.ground_rel;
+}
 
 // ------------------------------------------------------------------------------------------------
 // per-env register state
@@ -669,12 +692,11 @@ HD void euler_over_pi(float w, float x, float y, float z, float* roll, float* pi
     *pitch = fast_asin(clip(sinp, -1.f, 1.f)) * ipi;
     *yaw = fast_atan2(siny, cosy) * ipi;
 }
-template <typename R, int F>
+template <typename R, int F, bool kCur = false>
 HD void observe(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, const uint4 ur, int64_t i, int g_row, int o_row, ObsOut& out) {
     typedef R W;
     typedef Feat<F> FT;
     const KParams<R>& P = A.P;
-    const KCurriculum<R>& C = A.C;
     const int64_t n = A.ring_stride;
     const float ipx = (float)e.ipx, ipy = (float)e.ipy, ipz = (float)e.ipz;
     const float ivx = (float)e.ivx, ivy = (float)e.ivy, ivz = (float)e.ivz;
@@ -689,10 +711,10 @@ HD void observe(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, const uint
     bool onb = !(range > P.radar_range);
     if (onb) {
         float cb = ndot3(fx, fy, fz, rx, ry, rz) * nrcp(range + 1e-6f);
-        if (cb < C.cos_half_beam) onb = false;  // acos(clip(cb)) > radians(beam/2), core.py:547-553
+        if (cb < cur_cos_half_beam<kCur>(A)) onb = false;  // acos(clip(cb)) > radians(beam/2), core.py:547-553
     }
     if (onb) {
-        float q = P.radar_quality * (1.f - range * P.rc_radar_range * 0.5f) * C.onboard_rel;
+        float q = P.radar_quality * (1.f - range * P.rc_radar_range * 0.5f) * cur_onboard_rel<kCur>(A);
         if (u01(ur.y) > q) onb = false;
     }
     float orx, ory, orz;
@@ -723,7 +745,7 @@ HD void observe(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, const uint
         }
         if (ok && mpz < 50.f) ok = false;
         if (ok) {
-            float prob = P.g_base_q * (1.f - gr * P.rc_g_max_range * 0.4f) * C.ground_rel;
+            float prob = P.g_base_q * (1.f - gr * P.rc_g_max_range * 0.4f) * cur_ground_rel<kCur>(A);
             if (u01(ur.z) > prob) ok = false;
             else {
                 float z0, z1, z2, y0, y1, y2;
@@ -1433,12 +1455,12 @@ HD void tick_wind(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, uint32_t
 
 // ---- distance / intercept / termination (environment.py:657-814) and _calculate_reward (:1131-1320).  Reads the interceptor's
 // position, velocity and fuel AFTER its update; `dist` / `vo` come from volley_step() in volley mode ----
-template <typename R, int F>
+template <typename R, int F, bool kCur = false>
 HD void tick_outcome(const KernelArgs<R>& A, Env<R>& e, const float act0, R dist, const VolleyOut vo, TickOut& t) {
     typedef Feat<F> FT;
     const KParams<R>& P = A.P;
     const R dt = P.dt;
-    const R radius = FT::fuze(P) ? P.kill_radius : A.C.intercept_radius;
+    const R radius = FT::fuze(P) ? P.kill_radius : cur_radius<kCur>(A);
     bool intercepted, term = false, hit = false;
     if (FT::volley(P)) {
         intercepted = vo.intercepted; hit = vo.hit;
@@ -1480,7 +1502,7 @@ HD void tick_outcome(const KernelArgs<R>& A, Env<R>& e, const float act0, R dist
         if (term) {
             R md = e.min_d;
             if (e.flags & FLAG_CROSSED) {
-                R cr = A.C.intercept_radius;
+                R cr = cur_radius<kCur>(A);
                 r = R(3000.0);
                 if (md < cr) r = add(r, mul(dvd(sub(cr, md), cr), R(1000.0)));
                 r = add(r, mul(nexp(dvd(-md, R(25.0))), R(500.0)));
@@ -1530,7 +1552,7 @@ HD void tick_outcome(const KernelArgs<R>& A, Env<R>& e, const float act0, R dist
     t.reward = (float)r;
 }
 
-template <typename R, int F>
+template <typename R, int F, bool kCur = false>
 HD void tick_physics(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, const float act[6], int64_t ring_i, TickOut& t) {
     typedef Feat<F> FT;
     const KParams<R>& P = A.P;
@@ -1549,11 +1571,11 @@ HD void tick_physics(const KernelArgs<R>& A, Env<R>& e, const RngKey& key, const
     // missiles, their priority selection and intercept checks are one pass over the missile planes ----
     R dist = R(0);
     VolleyOut vo{false, false, false};
-    const R radius = FT::fuze(P) ? P.kill_radius : A.C.intercept_radius;
+    const R radius = FT::fuze(P) ? P.kill_radius : cur_radius<kCur>(A);
     if (FT::volley(P)) vo = volley_step<R, F>(A, e, key, ep, st, ring_i, radius, &dist);
     else missile_update<R, F>(P, e, key, ep, st, HLYNR_BLK_EVADE, e.mpx, e.mpy, e.mpz, e.mvx, e.mvy, e.mvz, (pre && FT::evasion(P)) ? ze : nullptr);
     tick_wind<R, F>(A, e, key, ep, st, t.ur, (pre && FT::enh_wind(P)) ? zw : nullptr);
-    tick_outcome<R, F>(A, e, act[0], dist, vo, t);
+    tick_outcome<R, F, kCur>(A, e, act[0], dist, vo, t);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1827,7 +1849,8 @@ template <typename R, int F> HD void prefetch_ring_reads(const KernelArgs<R>& A,
 #define HLYNR_F64_MIN_BLOCKS 3
 #endif
 template <typename R> struct StepOcc { static constexpr int ctas = std::is_same<R, double>::value ? HLYNR_F64_MIN_BLOCKS : 4; };
-template <typename R, bool kRollout, int F>
+// kCur: the curriculum comes from the attached schedule's device slot (KernelArgs::cur_dev), API-mode ticks only.
+template <typename R, bool kRollout, int F, bool kCur = false>
 __global__ void __launch_bounds__(HLYNR_STEP_BLOCK, StepOcc<R>::ctas * (HLYNR_BLOCK / HLYNR_STEP_BLOCK))
 step_kernel(const __grid_constant__ KernelArgs<R> A) {
     __shared__ __align__(16) float tiles[HLYNR_STEP_BLOCK / 32][OBS_TILE];
@@ -1886,7 +1909,7 @@ step_kernel(const __grid_constant__ KernelArgs<R> A) {
             act[0] = p0.x; act[1] = p0.y; act[2] = p1.x; act[3] = p1.y; act[4] = p2.x; act[5] = p2.y;
         }
         TickOut t;
-        tick_physics<R, F>(A, e, key, act, i, t);
+        tick_physics<R, F, kCur>(A, e, key, act, i, t);
         ob.emit = !kRollout || (s == steps - 1 && A.io.obs != nullptr);
         uint4 ur = t.ur;
         bool need_reset = false;
@@ -1899,7 +1922,7 @@ step_kernel(const __grid_constant__ KernelArgs<R> A) {
             }
             // ring planes are indexed by the lane's OWN (padded) slot: a shadow lane of another warp may run ticks
             // ahead in a fused rollout and must never touch the rows of the env it shadows
-            observe<R, F>(A, e, key, ur, i, g_row, o_row, ob);
+            observe<R, F, kCur>(A, e, key, ur, i, g_row, o_row, ob);
             if (pass == 0) {
                 const bool done = t.terminated || t.truncated;
                 if (ob.onboard_det) locks += 1;
@@ -1956,7 +1979,7 @@ step_kernel(const __grid_constant__ KernelArgs<R> A) {
 }
 
 // reset(): environment.py:353.  mask == NULL resets every env.
-template <typename R> __global__ void __launch_bounds__(HLYNR_BLOCK) reset_kernel(const __grid_constant__ KernelArgs<R> A) {
+template <typename R, bool kCur = false> __global__ void __launch_bounds__(HLYNR_BLOCK) reset_kernel(const __grid_constant__ KernelArgs<R> A) {
     __shared__ __align__(16) float tiles[HLYNR_BLOCK / 32][OBS_TILE];
     const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const int64_t i = (int64_t)blockIdx.x * HLYNR_BLOCK + threadIdx.x;
@@ -1970,7 +1993,7 @@ template <typename R> __global__ void __launch_bounds__(HLYNR_BLOCK) reset_kerne
     ob.emit = true;
     e.episode += 1;
     const uint4 ur = spawn(A, e, key, i);
-    observe<R, FT_GENERIC_MODES>(A, e, key, ur, i, A.g_row, A.o_row, ob);
+    observe<R, FT_GENERIC_MODES, kCur>(A, e, key, ur, i, A.g_row, A.o_row, ob);
     store_env(A, i, e);
     if (A.io.obs) copy_obs_row_n(ob.row, A.io.obs + i * A.obs_dim, A.obs_dim);
 }

@@ -155,7 +155,9 @@ class DeviceRolloutCollector:
 
     def capture(self):
         """Warm-up + stream capture of collect() into a CUDA graph (launch-bound at small n_envs: ~20 launches per step).
-        The curriculum scalars and the seed are baked into the captured kernel arguments: re-capture after changing them.
+        The seed and host-pushed curriculum scalars are baked into the captured kernel arguments: re-capture after changing them.
+        A sim that tracks training steps (HlynrSim.track_training_steps) keeps its counter on the device and every captured step
+        advances it there, so each replay continues the curriculum schedule; re-capture only after attaching or detaching one.
         The fused policy's noise counter lives on the device and each forward advances it there, so every replay draws fresh
         exploration noise, exactly as the same number of eager collects would."""
         if self.T % self.graph_period():

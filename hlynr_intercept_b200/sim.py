@@ -36,6 +36,7 @@ class HlynrSim:
         if self.obs_dim != 26:   # 17: the leading radar channels obs[0:17] only (include/hlynr.h, option "obs_dim")
             _lib.check(self.L.hlynr_set_option(self.h, b"obs_dim", self.obs_dim))
         self.push_curriculum()
+        self.tracking = False
         self._torch = torch
         self._info_t = None
         self._out = None
@@ -67,12 +68,55 @@ class HlynrSim:
         _lib.check(self.L.hlynr_set_curriculum(self.h, C.byref(c)))
 
     def set_training_step_count(self, n):
-        """environment.py:269 set_training_step_count (global to all envs)."""
+        """environment.py:269 set_training_step_count (global to all envs).  While tracking: sets the device counter, ordered on the
+        current stream."""
         self.curriculum.set_training_step_count(n)
-        self.push_curriculum()
+        if self.tracking:
+            _lib.check(self.L.hlynr_set_timesteps(self.h, int(n), self._stream()))
+        else:
+            self.push_curriculum()
 
     def get_current_intercept_radius(self):
+        """environment.py:223.  While tracking: at the device counter (synchronises the current stream)."""
+        if self.tracking:
+            self.curriculum.set_training_step_count(self.num_timesteps)
         return self.curriculum.intercept_radius()
+
+    def track_training_steps(self, num_timesteps=0, increment=None):
+        """Advance the curriculum on the device, as SB3's per-step set_training_step_count callback would: every step() first
+        computes the curriculum of the device counter, then adds `increment` to it (default: this sim's n; a shard of a multi-GPU
+        run passes the global env count).  reset() uses the counter without advancing it.  Eager steps, StepGraph replays and
+        DeviceRolloutCollector replays all continue the schedule.  step_host-based paths (HlynrVecEnv) and rollout() refuse to run
+        while tracking; untrack_training_steps() ends it."""
+        increment = self.n if increment is None else int(increment)
+        _lib.check(self.L.hlynr_attach_curriculum(self.h, C.byref(self.curriculum.schedule()), int(num_timesteps), increment))
+        self.curriculum.set_training_step_count(int(num_timesteps))
+        self.tracking, self.increment = True, increment
+
+    def untrack_training_steps(self):
+        """Back to the host-pushed curriculum, set to the values of the device counter's current count."""
+        if not self.tracking:
+            return
+        n = self.num_timesteps
+        _lib.check(self.L.hlynr_detach_curriculum(self.h))
+        self.tracking = False
+        self.set_training_step_count(n)
+
+    @property
+    def num_timesteps(self):
+        """The training-step count: the device counter while tracking (synchronises the current stream), else the last pushed."""
+        if not self.tracking:
+            return self.curriculum.training_step_count
+        v = C.c_uint64()
+        _lib.check(self.L.hlynr_get_timesteps(self.h, C.byref(v), self._stream()))
+        return v.value
+
+    def debug_curriculum_at(self, count):
+        """(intercept radius, cos of the half beam width, onboard reliability, ground reliability) the device computes from the
+        tracked schedule at `count`, as float64 (test hook)."""
+        out = (C.c_double * 4)()
+        _lib.check(self.L.hlynr_debug_curriculum_at(self.h, int(count), out))
+        return tuple(out)
 
     def seed(self, seed):
         self.seed_value = int(seed)

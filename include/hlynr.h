@@ -131,6 +131,21 @@ typedef struct HlynrCurriculum {
 } HlynrCurriculum;
 
 /*
+ * The whole curriculum schedule (config.Curriculum): what get_current_intercept_radius and _update_radar_curriculum
+ * (environment.py:223-234, 274-351) compute from training_step_count, for hlynr_attach_curriculum.  Steps are doubles because
+ * YAML may give them as floats.  A ramp is Curriculum._ramp: `initial` below `start`, `final` from `end` on, linear between.
+ * With radar_enabled == 0 the three radar values are the constant `*_initial` ones.
+ */
+typedef struct HlynrCurriculumSchedule {
+    int32_t enabled;          /* curriculum.enabled; 0 = the radius is final_radius at every count */
+    int32_t radar_enabled;    /* curriculum.radar_curriculum present, non-empty and enabled */
+    double initial_radius, final_radius, curriculum_steps;
+    double beam_initial, beam_final, beam_start, beam_end;                 /* degrees */
+    double onboard_initial, onboard_final, onboard_start, onboard_end;     /* detection reliability */
+    double ground_initial, ground_final, ground_start, ground_end;         /* ground reliability */
+} HlynrCurriculumSchedule;
+
+/*
  * Optional per-env info, structure-of-arrays, device pointers (any may be NULL).
  * Field meaning = the reference's info dict, environment.py:829-857.  Values are those of the
  * tick just executed (i.e. of the terminal tick for envs that were auto-reset in this call).
@@ -233,6 +248,7 @@ const char* hlynr_last_error(void);
 int hlynr_abi_version(void);
 size_t hlynr_params_size(void);
 size_t hlynr_env_state_size(void);
+size_t hlynr_curriculum_schedule_size(void);
 
 /* Replaces N x InterceptEnvironment(config) (environment.py:20).  `precision` is HLYNR_FP32 or
  * HLYNR_FP64.  Envs get global ids [env_id_offset, env_id_offset + n_envs): trajectories depend
@@ -244,6 +260,29 @@ void hlynr_destroy(hlynr_t* sim);
 int hlynr_num_envs(const hlynr_t* sim, int64_t* out);
 int hlynr_set_curriculum(hlynr_t* sim, const HlynrCurriculum* cur);
 int hlynr_get_curriculum(const hlynr_t* sim, HlynrCurriculum* out);
+
+/* Device-side training-step counter (SB3's model.num_timesteps, which the reference's callback pushes with
+ * env_method('set_training_step_count') after every env step, train_flat_ppo.py:173-177).  While a schedule is attached, every
+ * hlynr_step first runs a one-thread kernel that computes the curriculum of the current count into a device slot the step kernel
+ * reads, then advances the count by `increment`; hlynr_reset computes the slot without advancing.  So the step at tick t after
+ * attaching sees t0 + t*increment, as in SB3, where the callback runs after the step -- and a CUDA graph of steps continues the
+ * schedule on every replay instead of repeating the curriculum of its capture.
+ *   increment  what one tick adds: the number of envs of the whole run (the shard's n, or the global count of a multi-GPU run).
+ * Refuses non-finite fields, curriculum_steps <= 0 while enabled and increment < 0.  While attached, hlynr_set_curriculum,
+ * hlynr_step_host and hlynr_rollout fail: the host path is driven by the host-side callback, and the fused k-tick rollout would
+ * need one slot per fused tick.  The device block lives until hlynr_destroy, so a captured graph never points at freed memory;
+ * the schedule, the increment and whether one is attached at all are baked into captured launches (re-capture after changing them). */
+int hlynr_attach_curriculum(hlynr_t* sim, const HlynrCurriculumSchedule* schedule, uint64_t num_timesteps, int64_t increment);
+/* Back to the by-value curriculum of hlynr_set_curriculum (unchanged since it was last set). */
+int hlynr_detach_curriculum(hlynr_t* sim);
+/* Sets the count, ordered on `stream` (a one-thread kernel: graph-capturable).  Fails unless a schedule is attached. */
+int hlynr_set_timesteps(hlynr_t* sim, uint64_t num_timesteps, void* stream);
+/* Synchronises `stream` and returns the count.  Fails unless a schedule is attached. */
+int hlynr_get_timesteps(hlynr_t* sim, uint64_t* out, void* stream);
+/* Test hook: the curriculum values the device computes from the attached schedule at `count`, widened to double without rounding:
+ * out[0] intercept radius (in the handle's precision), out[1] cosine of the half beam width (float; -2 for a beam of 360 degrees
+ * or more), out[2] onboard reliability (float), out[3] ground reliability (float).  Synchronous. */
+int hlynr_debug_curriculum_at(hlynr_t* sim, uint64_t count, double out[4]);
 /* Re-keys the counter-based RNG (reference: reset(seed=...), environment.py:357-359). */
 int hlynr_seed(hlynr_t* sim, uint64_t seed);
 
@@ -345,7 +384,8 @@ int hlynr_set_option(hlynr_t* sim, const char* name, int64_t value);
  * tick are kernel arguments computed from the handle's tick counter, so a captured sequence of T ticks replays correctly
  * iff T is a multiple of hlynr_ring_period(); after each replay the host-side counters are advanced with
  * hlynr_note_replayed_ticks(sim, T) (negative values undo the bookkeeping of calls that were only recorded, not executed).
- * Curriculum scalars and the seed are baked into the captured arguments. */
+ * By-value curriculum scalars and the seed are baked into the captured arguments; an attached schedule's count lives on the
+ * device and advances on every replay (hlynr_attach_curriculum). */
 int hlynr_ring_period(const hlynr_t* sim, int* out);   /* lcm(onboard ring length, ground ring length), >= 1 */
 int hlynr_note_replayed_ticks(hlynr_t* sim, int64_t ticks, int64_t launches);
 /* Ticks executed (or accounted for by hlynr_note_replayed_ticks) since hlynr_create: a captured sequence may only be replayed
