@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libhlynr_b200.so")
 SOURCES = [os.path.join(HERE, "csrc", "hlynr_capi.cu"), os.path.join(HERE, "csrc", "hlynr_post.cu"),
            os.path.join(HERE, "csrc", "hlynr_rollout.cu"), os.path.join(HERE, "csrc", "hlynr_policy.cu")]
-DEPS = SOURCES + [os.path.join(HERE, "csrc", "hlynr_device.cuh"),
+DEPS = SOURCES + [os.path.join(HERE, "csrc", "hlynr_device.cuh"), os.path.join(HERE, "csrc", "hlynr_host.cuh"),
                   os.path.join(os.path.dirname(HERE), "include", "hlynr.h"),
                   os.path.join(os.path.dirname(HERE), "include", "hlynr_post.h"),
                   os.path.join(os.path.dirname(HERE), "include", "hlynr_rollout.h"),

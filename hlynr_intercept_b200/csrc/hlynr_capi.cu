@@ -11,6 +11,7 @@
 #include <mutex>
 #include <new>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #if defined(__x86_64__)
@@ -18,20 +19,13 @@
 #endif
 
 #include "hlynr_device.cuh"
+#include "hlynr_host.cuh"
 
 using namespace hlynr;
 
 static_assert(sizeof(HlynrDoneRecord) == 200, "HlynrDoneRecord is 50 words (mirrored by abi.done_record_numpy_dtype)");
 
 static thread_local char g_err[512] = "";
-static int fail(const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return 1;
-}
-// error reporting for the other translation units of the library (hlynr_post.cu)
 extern "C" int hlynr_internal_fail(const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
@@ -39,21 +33,6 @@ extern "C" int hlynr_internal_fail(const char* fmt, ...) {
     va_end(ap);
     return 1;
 }
-#define CK(call)                                                                                      \
-    do {                                                                                              \
-        cudaError_t _e = (call);                                                                      \
-        if (_e != cudaSuccess) return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
-    } while (0)
-
-struct DeviceGuard {
-    int prev = -1;
-    bool ok = true;
-    explicit DeviceGuard(int dev) {
-        if (cudaGetDevice(&prev) != cudaSuccess) { ok = false; return; }
-        if (prev != dev && cudaSetDevice(dev) != cudaSuccess) ok = false;
-    }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 // Staging memcpys between unpinned caller buffers and the pinned buffers.  A single thread copies ~5-10 GB/s, less than the
 // PCIe link moves, so a few persistent helper threads pull 256 KiB blocks off an atomic counter, in address order.  start() is
@@ -226,6 +205,16 @@ struct hlynr_sim {
     HlynrCurriculumSchedule sched;
     int64_t cur_increment = 0;
 };
+
+// Calls f with the state planes of the handle's precision, s->pf or s->pd: the one place the precision picks the instantiations.
+// f is a generic lambda; real_of<decltype(planes)> names its R.
+template <class F> static auto with_planes(hlynr_sim* s, F&& f) {
+    if (s->precision == HLYNR_FP32) return f(s->pf);
+    return f(s->pd);
+}
+template <class P> struct PlanesReal;
+template <class R> struct PlanesReal<StatePlanes<R>> { using type = R; };
+template <class P> using real_of = typename PlanesReal<std::decay_t<P>>::type;
 
 // ------------------------------------------------------------------------------------------------
 // parameter conversion
@@ -507,8 +496,10 @@ template <typename R> static KernelArgs<R> base_args(hlynr_sim* s, const StatePl
 // Before a step (increment = the attached increment) or a reset (0): the slot the next launch reads, and the count advanced.
 static int curriculum_tick(hlynr_sim* s, int64_t increment, cudaStream_t st) {
     if (!s->cur_attached) return 0;
-    if (s->precision == HLYNR_FP32) curriculum_tick_kernel<float><<<1, 1, 0, st>>>((CurBlock<float>*)s->cur_block, s->sched, (unsigned long long)increment);
-    else curriculum_tick_kernel<double><<<1, 1, 0, st>>>((CurBlock<double>*)s->cur_block, s->sched, (unsigned long long)increment);
+    with_planes(s, [&](auto& planes) {
+        using R = real_of<decltype(planes)>;
+        curriculum_tick_kernel<R><<<1, 1, 0, st>>>((CurBlock<R>*)s->cur_block, s->sched, (unsigned long long)increment);
+    });
     CK(cudaGetLastError());
     s->launches += 1;
     return 0;
@@ -631,10 +622,8 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
     s->device = device; s->precision = precision; s->seed = seed; s->env_offset = env_id_offset;
     KParams<float> kp = make_kparams<float>(*p);
     const int gl = kp.gnd_ring_len, ol = kp.onb_ring_len;
-    cudaError_t e;
-    if (precision == HLYNR_FP32) s->state_bytes = carve<float>(s->pf, nullptr, s->n_pad, gl, ol, p->volley_size);
-    else s->state_bytes = carve<double>(s->pd, nullptr, s->n_pad, gl, ol, p->volley_size);
-    e = cudaMalloc(&s->state_mem, s->state_bytes);
+    s->state_bytes = with_planes(s, [&](auto& planes) { return carve(planes, nullptr, s->n_pad, gl, ol, p->volley_size); });
+    cudaError_t e = cudaMalloc(&s->state_mem, s->state_bytes);
     if (e != cudaSuccess) { int r = fail("hlynr_create: cudaMalloc(%zu bytes) failed: %s", s->state_bytes, cudaGetErrorString(e)); delete s; return r; }
     e = cudaMalloc(&s->stats, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS);
     if (e != cudaSuccess) { int r = fail("hlynr_create: cudaMalloc(stats) failed: %s", cudaGetErrorString(e)); cudaFree(s->state_mem); delete s; return r; }
@@ -643,16 +632,16 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
     cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking);
     cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device);
     const int blk = 256;
-    if (precision == HLYNR_FP32) {
-        carve<float>(s->pf, (char*)s->state_mem, s->n_pad, gl, ol, p->volley_size);
-        // compact plane layout (hlynr_device.cuh load_env): fixed for the life of the handle, whichever kernel instantiation runs
+    with_planes(s, [&](auto& planes) {
+        using R = real_of<decltype(planes)>;
+        carve(planes, (char*)s->state_mem, s->n_pad, gl, ol, p->volley_size);
+        // compact plane layout (fp32 build only; hlynr_device.cuh load_env): fixed for the life of the handle, whichever kernel
+        // instantiation runs
         s->compact = 0;
-        if (p->max_steps < 65536 && !getenv("HLYNR_NO_COMPACT")) s->compact = feature_set(*p) == FT_V2ON ? 1 : (feature_set(*p) == FT_V2ON_DR ? 2 : 0);
-        init_kernel<float><<<grid_for(s->n_pad, blk), blk>>>(s->pf, s->n_pad, (float)p->peak_mult, s->compact);
-    } else {
-        carve<double>(s->pd, (char*)s->state_mem, s->n_pad, gl, ol, p->volley_size);
-        init_kernel<double><<<grid_for(s->n_pad, blk), blk>>>(s->pd, s->n_pad, (float)p->peak_mult, 0);
-    }
+        if (std::is_same<R, float>::value && p->max_steps < 65536 && !getenv("HLYNR_NO_COMPACT"))
+            s->compact = feature_set(*p) == FT_V2ON ? 1 : (feature_set(*p) == FT_V2ON_DR ? 2 : 0);
+        init_kernel<R><<<grid_for(s->n_pad, blk), blk>>>(planes, s->n_pad, (float)p->peak_mult, s->compact);
+    });
     e = cudaDeviceSynchronize();
     if (e != cudaSuccess) { int r = fail("hlynr_create: init kernel failed: %s", cudaGetErrorString(e)); hlynr_destroy(s); return r; }
     s->launches += 1;
@@ -726,17 +715,14 @@ int hlynr_reset(hlynr_t* s, const uint8_t* mask_dev, float* obs_dev, void* strea
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (curriculum_tick(s, 0, st)) return 1;   // the reference's reset uses the last pushed count and does not advance it
-    if (s->precision == HLYNR_FP32) {
-        KernelArgs<float> A = base_args<float>(s, s->pf);
+    with_planes(s, [&](auto& planes) {
+        using R = real_of<decltype(planes)>;
+        KernelArgs<R> A = base_args(s, planes);
         A.io.reset_mask = mask_dev; A.io.obs = obs_dev;
-        if (A.cur_dev) reset_kernel<float, true><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
-        else reset_kernel<float><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
-    } else {
-        KernelArgs<double> A = base_args<double>(s, s->pd);
-        A.io.reset_mask = mask_dev; A.io.obs = obs_dev;
-        if (A.cur_dev) reset_kernel<double, true><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
-        else reset_kernel<double><<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
-    }
+        // the instantiation that reads the curriculum slot while a schedule is attached
+        const auto kernel = A.cur_dev ? reset_kernel<R, true> : reset_kernel<R, false>;
+        kernel<<<grid_for(s->n, HLYNR_BLOCK), HLYNR_BLOCK, 0, st>>>(A);
+    });
     CK(cudaGetLastError());
     s->launches += 1;
     return 0;
@@ -747,21 +733,15 @@ int hlynr_reset(hlynr_t* s, const uint8_t* mask_dev, float* obs_dev, void* strea
 static int step_range(hlynr_sim* s, int64_t first, int64_t lim, const float* actions_dev, float* obs_dev, float* reward_dev,
                       uint8_t* terminated_dev, uint8_t* truncated_dev, float* terminal_obs_dev, const HlynrInfoSoA* info,
                       int auto_reset, cudaStream_t st) {
-    if (s->precision == HLYNR_FP32) {
-        KernelArgs<float> A = base_args<float>(s, s->pf);
+    with_planes(s, [&](auto& planes) {
+        using R = real_of<decltype(planes)>;
+        KernelArgs<R> A = base_args(s, planes);
         A.first = first; A.lim = lim;
         A.io.actions = actions_dev; A.io.obs = obs_dev; A.io.reward = reward_dev; A.io.terminated = terminated_dev;
         A.io.truncated = truncated_dev; A.io.terminal_obs = terminal_obs_dev; A.auto_reset = auto_reset;
         if (info) { A.io.info = *info; A.has_info = 1; }
-        launch_step<float, false>(s, A, st, s->specialise != 0);
-    } else {
-        KernelArgs<double> A = base_args<double>(s, s->pd);
-        A.first = first; A.lim = lim;
-        A.io.actions = actions_dev; A.io.obs = obs_dev; A.io.reward = reward_dev; A.io.terminated = terminated_dev;
-        A.io.truncated = truncated_dev; A.io.terminal_obs = terminal_obs_dev; A.auto_reset = auto_reset;
-        if (info) { A.io.info = *info; A.has_info = 1; }
-        launch_step<double, false>(s, A, st, s->specialise != 0);
-    }
+        launch_step<R, false>(s, A, st, s->specialise != 0);
+    });
     CK(cudaGetLastError());
     s->launches += 1;
     s->env_steps += (double)(lim - first);
@@ -828,8 +808,7 @@ int hlynr_debug_curriculum_at(hlynr_t* s, uint64_t count, double out[4]) {
     DeviceGuard g(s->device);
     double* buf = nullptr;
     CK(cudaMalloc(&buf, 4 * sizeof(double)));
-    if (s->precision == HLYNR_FP32) curriculum_probe_kernel<float><<<1, 1>>>(s->sched, (unsigned long long)count, buf);
-    else curriculum_probe_kernel<double><<<1, 1>>>(s->sched, (unsigned long long)count, buf);
+    with_planes(s, [&](auto& planes) { curriculum_probe_kernel<real_of<decltype(planes)>><<<1, 1>>>(s->sched, (unsigned long long)count, buf); });
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpy(out, buf, 4 * sizeof(double), cudaMemcpyDeviceToHost);
     cudaFree(buf);
@@ -854,17 +833,13 @@ int hlynr_rollout(hlynr_t* s, int k_steps, const float* actions_dev, float* obs_
                     "curriculum slot): step with hlynr_step, or hlynr_detach_curriculum first");
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
-    if (s->precision == HLYNR_FP32) {
-        KernelArgs<float> A = base_args<float>(s, s->pf);
+    with_planes(s, [&](auto& planes) {
+        using R = real_of<decltype(planes)>;
+        KernelArgs<R> A = base_args(s, planes);
         set_tick(A, s->tick + 1); A.k_steps = k_steps; A.auto_reset = 1;
         A.io.actions = actions_dev; A.io.obs = obs_dev; A.io.reward_sum = reward_sum_dev; A.io.done_count = done_count_dev;
-        launch_step<float, true>(s, A, st, s->specialise != 0);
-    } else {
-        KernelArgs<double> A = base_args<double>(s, s->pd);
-        set_tick(A, s->tick + 1); A.k_steps = k_steps; A.auto_reset = 1;
-        A.io.actions = actions_dev; A.io.obs = obs_dev; A.io.reward_sum = reward_sum_dev; A.io.done_count = done_count_dev;
-        launch_step<double, true>(s, A, st, s->specialise != 0);
-    }
+        launch_step<R, true>(s, A, st, s->specialise != 0);
+    });
     CK(cudaGetLastError());
     s->tick += (uint64_t)k_steps;
     s->launches += 1;
@@ -919,8 +894,9 @@ int hlynr_export_state(hlynr_t* s, int64_t first, int64_t count, HlynrEnvState* 
     DeviceGuard g(s->device);
     CK(cudaDeviceSynchronize());
     if (ensure_xchg(s, count)) return 1;
-    if (s->precision == HLYNR_FP32) export_kernel<float><<<grid_for(count, 128), 128>>>(base_args<float>(s, s->pf), first, count, s->xchg);
-    else export_kernel<double><<<grid_for(count, 128), 128>>>(base_args<double>(s, s->pd), first, count, s->xchg);
+    with_planes(s, [&](auto& planes) {
+        export_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg);
+    });
     CK(cudaGetLastError());
     CK(cudaMemcpy(host_out, s->xchg, sizeof(HlynrEnvState) * count, cudaMemcpyDeviceToHost));
     s->launches += 1;
@@ -935,8 +911,9 @@ int hlynr_import_state(hlynr_t* s, int64_t first, int64_t count, const HlynrEnvS
     CK(cudaDeviceSynchronize());
     if (ensure_xchg(s, count)) return 1;
     CK(cudaMemcpy(s->xchg, host_in, sizeof(HlynrEnvState) * count, cudaMemcpyHostToDevice));
-    if (s->precision == HLYNR_FP32) import_kernel<float><<<grid_for(count, 128), 128>>>(base_args<float>(s, s->pf), first, count, s->xchg);
-    else import_kernel<double><<<grid_for(count, 128), 128>>>(base_args<double>(s, s->pd), first, count, s->xchg);
+    with_planes(s, [&](auto& planes) {
+        import_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg);
+    });
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     s->launches += 1;

@@ -20,8 +20,6 @@
 //
 // Layers are serialised inside a tile by two mbarriers (a_ready: operand written + TMEM drained; acc_ready: GEMM complete);
 // the weight ring runs ahead across layers and tiles, because weights do not depend on the activations.
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <new>
 
@@ -31,14 +29,7 @@
 
 #include "../../include/hlynr_policy.h"
 #include "../../include/hlynr_rng.h"
-
-extern "C" int hlynr_internal_fail(const char* fmt, ...);  // hlynr_capi.cu: sets the thread's hlynr_last_error()
-#define fail hlynr_internal_fail
-#define CK(call)                                                                                      \
-    do {                                                                                              \
-        cudaError_t _e = (call);                                                                      \
-        if (_e != cudaSuccess) return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
-    } while (0)
+#include "hlynr_host.cuh"
 
 namespace {
 
@@ -647,12 +638,6 @@ __global__ void copy_f32_kernel(const float* __restrict__ src, float* __restrict
     if (i < n_dst) dst[i] = i < n ? src[i] : 0.f;
 }
 
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && prev != dev) cudaSetDevice(dev); }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -685,6 +670,14 @@ int make_map(EncodeTiledFn enc, CUtensorMap* m, void* base, int rows, int k, int
     const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : fail("cuTensorMapEncodeTiled failed with CUresult %d (rows %d, k %d)", (int)r, rows, k);
+}
+
+// The instantiation for log2 of the cluster size (ci: 0, 1, 2) and the input rows (fixed: the 104-wide loader, else the generic one).
+using ForwardKernel = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, Params, unsigned long long*);
+ForwardKernel forward_kernel(int ci, bool fixed) {
+    static const ForwardKernel k[2][3] = {{policy_forward_kernel<1, IN>, policy_forward_kernel<2, IN>, policy_forward_kernel<4, IN>},
+                                          {policy_forward_kernel<1, 0>, policy_forward_kernel<2, 0>, policy_forward_kernel<4, 0>}};
+    return k[fixed ? 0 : 1][ci];
 }
 }  // namespace
 
@@ -793,15 +786,7 @@ int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int6
     if (((uintptr_t)obs_dev & 3u) != 0) return fail("%s: obs_dev must be 4-byte aligned", fn);
     DeviceGuard g(p->device);
     if (!p->smem_configured) {
-        if (fixed) {
-            CK(cudaFuncSetAttribute(policy_forward_kernel<1, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-            CK(cudaFuncSetAttribute(policy_forward_kernel<2, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-            CK(cudaFuncSetAttribute(policy_forward_kernel<4, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        } else {
-            CK(cudaFuncSetAttribute(policy_forward_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-            CK(cudaFuncSetAttribute(policy_forward_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-            CK(cudaFuncSetAttribute(policy_forward_kernel<4, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        }
+        for (int c = 0; c < 3; ++c) CK(cudaFuncSetAttribute(forward_kernel(c, fixed), cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         p->smem_configured = true;
     }
     Params P;
@@ -816,6 +801,7 @@ int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int6
     P.timing = p->timing_on ? p->timing : nullptr; P.timing_tiles = 8;
     const int64_t n_tiles = (n_rows + BM - 1) / BM;
     const int cl = p->cluster, ci = cl == 4 ? 2 : (cl == 2 ? 1 : 0);
+    const ForwardKernel kernel = forward_kernel(ci, fixed);
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = (cudaStream_t)stream;
@@ -828,11 +814,7 @@ int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int6
         if (cl > 1) {
             cfg.gridDim = dim3((unsigned)(clusters * cl));
             int fit = 0;
-            cudaError_t oe;
-            if (fixed) oe = cl == 2 ? cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<2, IN>, &cfg)
-                                    : cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<4, IN>, &cfg);
-            else oe = cl == 2 ? cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<2, 0>, &cfg)
-                              : cudaOccupancyMaxActiveClusters(&fit, policy_forward_kernel<4, 0>, &cfg);
+            const cudaError_t oe = cudaOccupancyMaxActiveClusters(&fit, kernel, &cfg);
             if (oe == cudaSuccess && fit > 0 && fit < clusters) clusters = fit;
             else if (oe != cudaSuccess) cudaGetLastError();
         }
@@ -842,16 +824,7 @@ int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int6
     if (grid > p->grid_for_cluster[ci]) grid = p->grid_for_cluster[ci];
     cfg.gridDim = dim3((unsigned)grid);
     const CUtensorMap* tm = p->tm[ci];
-    cudaError_t le;
-    if (fixed) {
-        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, IN>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-    } else {
-        if (cl == 1) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<1, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-        else if (cl == 2) le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<2, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-        else le = cudaLaunchKernelEx(&cfg, policy_forward_kernel<4, 0>, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
-    }
+    const cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, tm[0], tm[1], tm[2], tm[3], P, ctr_dev);
     if (le != cudaSuccess) return fail("%s: launch failed: %s", fn, cudaGetErrorString(le));
     CK(cudaGetLastError());
     p->launches += 1;

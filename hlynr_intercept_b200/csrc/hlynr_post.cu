@@ -13,22 +13,14 @@
 // The frame width F is 26 (the full observation) or 17 (the leading radar channels obs[0:17], HlynrSim(obs_dim=17)); every
 // kernel that touches the ring is a template on F, so the 26-wide code is what it was before F became a parameter.
 #include <cmath>
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <new>
+#include <type_traits>
 
 #include <cuda_runtime.h>
 
 #include "../../include/hlynr_post.h"
-
-extern "C" int hlynr_internal_fail(const char* fmt, ...);  // hlynr_capi.cu: sets the thread's hlynr_last_error()
-#define fail hlynr_internal_fail
-#define CK(call)                                                                                      \
-    do {                                                                                              \
-        cudaError_t _e = (call);                                                                      \
-        if (_e != cudaSuccess) return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
-    } while (0)
+#include "hlynr_host.cuh"
 
 namespace {
 
@@ -46,12 +38,6 @@ struct PostStats {
     double ret_mean, ret_var, ret_count;    // ret_rms
     double chk_S[KMAX][OD], chk_Q[KMAX][OD];  // check_sums scratch
     double inv_std[DMAX];                   // 1 / sqrt(var + eps): the normalise kernels compute in float64 like SB3 (obs f32 - mean f64)
-};
-
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && prev != dev) cudaSetDevice(dev); }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
 __device__ __forceinline__ int ring_slot(int newest, int lag, int k) { int s = newest - lag; return s < 0 ? s + k : s; }
@@ -359,6 +345,13 @@ struct hlynr_post {
     int64_t launches = 0;
 };
 
+// Calls f(std::integral_constant<int, F>{}) for the handle's frame width F, 26 or 17: the one place the width picks the
+// instantiations of the ring kernels.
+template <class Fn> static auto with_width(const hlynr_post* p, Fn&& f) {
+    if (p->fw == OD) return f(std::integral_constant<int, OD>{});
+    return f(std::integral_constant<int, 17>{});
+}
+
 static int blocks_for(const hlynr_post* p, int64_t items, int per_block) {
     int64_t b = (items + per_block - 1) / per_block;
     const int64_t cap = (int64_t)p->sm_count * 8;
@@ -385,7 +378,7 @@ static int launch_normalize_t(hlynr_post* p, float* out, int raw, cudaStream_t s
 }
 
 static int launch_normalize(hlynr_post* p, float* out, int raw, cudaStream_t st) {
-    return p->fw == OD ? launch_normalize_t<OD>(p, out, raw, st) : launch_normalize_t<17>(p, out, raw, st);
+    return with_width(p, [&](auto F) { return launch_normalize_t<F>(p, out, raw, st); });
 }
 
 template <int F>
@@ -516,7 +509,7 @@ int hlynr_post_reset(hlynr_post_t* p, float* out_dev, int training, void* stream
     if (!p || !out_dev) return fail("hlynr_post_reset: null argument");
     DeviceGuard g(p->device);
     cudaStream_t st = (cudaStream_t)stream;
-    return p->fw == OD ? reset_t<OD>(p, out_dev, training, st) : reset_t<17>(p, out_dev, training, st);
+    return with_width(p, [&](auto F) { return reset_t<F>(p, out_dev, training, st); });
 }
 
 int hlynr_post_step(hlynr_post_t* p, const float* reward_dev, const uint8_t* terminated_dev, const uint8_t* truncated_dev,
@@ -531,10 +524,10 @@ int hlynr_post_step(hlynr_post_t* p, const float* reward_dev, const uint8_t* ter
     if (terminal_out_dev && (!records_dev || !counter_dev)) return fail("hlynr_post_step: terminal_out_dev needs the done list of the step");
     DeviceGuard g(p->device);
     cudaStream_t st = (cudaStream_t)stream;
-    return p->fw == OD ? step_t<OD>(p, reward_dev, terminated_dev, truncated_dev, records_dev, counter_dev, capacity, out_dev,
-                                    terminal_out_dev, training, can_maintain, st)
-                       : step_t<17>(p, reward_dev, terminated_dev, truncated_dev, records_dev, counter_dev, capacity, out_dev,
-                                    terminal_out_dev, training, can_maintain, st);
+    return with_width(p, [&](auto F) {
+        return step_t<F>(p, reward_dev, terminated_dev, truncated_dev, records_dev, counter_dev, capacity, out_dev, terminal_out_dev,
+                         training, can_maintain, st);
+    });
 }
 
 int hlynr_post_original(hlynr_post_t* p, float* out_dev, void* stream) {
@@ -584,8 +577,7 @@ int hlynr_post_set_stats(hlynr_post_t* p, const double* mean, const double* var,
     const double tail[4] = {count, ret_mean, ret_var, ret_count};
     CK(cudaMemcpyAsync(&p->st->count, &tail[0], sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(&p->st->ret_mean, &tail[1], sizeof(double) * 3, cudaMemcpyHostToDevice, st));
-    if (p->fw == OD) merge_kernel<OD><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps);  // refresh inv_std
-    else merge_kernel<17><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps);
+    with_width(p, [&](auto F) { merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps); });  // refresh inv_std
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));  // `tail` is a stack array
     p->launches += 1;
@@ -600,12 +592,10 @@ int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, voi
     CK(cudaMemsetAsync(p->st->chk_S, 0, sizeof(double) * KMAX * OD * 2, st));
     const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
     const int newest = (int)((p->t - 1) % (uint32_t)p->k);
-    if (p->fw == OD)
-        recompute_sums_kernel<OD><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
-                                                                                      newest, p->st);
-    else
-        recompute_sums_kernel<17><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
-                                                                                      newest, p->st);
+    with_width(p, [&](auto F) {
+        recompute_sums_kernel<F><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
+                                                                                     newest, p->st);
+    });
     CK(cudaGetLastError());
     p->launches += 1;
     PostStats* h = new (std::nothrow) PostStats();

@@ -5,17 +5,9 @@
 #include <cuda_runtime.h>
 
 #include "../../include/hlynr_rollout.h"
-
-extern "C" int hlynr_internal_fail(const char* fmt, ...);
-#define fail hlynr_internal_fail
+#include "hlynr_host.cuh"
 
 namespace {
-
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && prev != dev) cudaSetDevice(dev); }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 __global__ void bootstrap_kernel(float* __restrict__ rewards, const HlynrDoneRecord* __restrict__ recs, const int32_t* __restrict__ counter,
                                  int32_t rows, const float* __restrict__ tv, float gamma, int32_t* overflow) {
@@ -100,8 +92,7 @@ int hlynr_bootstrap_timeouts(float* rewards_dev, const HlynrDoneRecord* records_
     DeviceGuard g(device);
     const int blocks = rows < 256 * 64 ? (rows + 255) / 256 : 64;
     bootstrap_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(rewards_dev, records_dev, counter_dev, rows, terminal_values_dev, (float)gamma, overflow_dev);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail("hlynr_bootstrap_timeouts: %s", cudaGetErrorString(e));
+    CK(cudaGetLastError());
     return 0;
 }
 
@@ -115,8 +106,7 @@ int hlynr_gae(const float* rewards_dev, const float* values_dev, const float* ep
     gae_kernel<<<(unsigned)((N + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rewards_dev, values_dev, episode_starts_dev, last_values_dev,
                                                                             last_dones_dev, T, N, (float)gamma, (float)(gamma * gae_lambda),
                                                                             advantages_dev, returns_dev);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail("hlynr_gae: %s", cudaGetErrorString(e));
+    CK(cudaGetLastError());
     return 0;
 }
 
@@ -132,8 +122,7 @@ int hlynr_eval_record(const HlynrDoneRecord* records_dev, const int32_t* counter
     eval_record_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(records_dev, counter_dev, n_envs, n_episodes / n_envs, n_episodes % n_envs,
                                                                  counts_dev, ticks_dev, results_dev, end_tick_dev,
                                                                  reinterpret_cast<unsigned long long*>(remaining_dev));
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail("hlynr_eval_record: %s", cudaGetErrorString(e));
+    CK(cudaGetLastError());
     return 0;
 }
 
