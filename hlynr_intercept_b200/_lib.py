@@ -25,7 +25,7 @@ EXPORTS = [
     "hlynr_post_step", "hlynr_post_original", "hlynr_post_normalize", "hlynr_post_get_stats", "hlynr_post_set_stats",
     "hlynr_post_check_sums", "hlynr_post_launch_count", "hlynr_post_note_replayed_steps",
     # include/hlynr_rollout.h
-    "hlynr_bootstrap_timeouts", "hlynr_gae", "hlynr_eval_record",
+    "hlynr_bootstrap_timeouts", "hlynr_gae", "hlynr_eval_record", "hlynr_trace_row_size", "hlynr_eval_trace",
     # include/hlynr_policy.h
     "hlynr_policy_create", "hlynr_policy_create_dim", "hlynr_policy_destroy", "hlynr_policy_set_weights", "hlynr_policy_forward", "hlynr_policy_forward_dev",
     "hlynr_policy_set_counter", "hlynr_policy_get_counter", "hlynr_policy_launch_count", "hlynr_policy_set_option", "hlynr_policy_get_timing",
@@ -112,6 +112,8 @@ def load(build_if_missing=True):
     L.hlynr_bootstrap_timeouts.argtypes = [vp, vp, vp, C.c_int32, vp, C.c_double, vp, i32, vp]
     L.hlynr_gae.argtypes = [vp, vp, vp, vp, vp, i64, i64, C.c_double, C.c_double, vp, vp, i32, vp]
     L.hlynr_eval_record.argtypes = [vp, vp, i64, i64, vp, vp, vp, vp, vp, i32, vp]
+    L.hlynr_trace_row_size.restype = C.c_size_t
+    L.hlynr_eval_trace.argtypes = [C.POINTER(abi.HlynrInfoSoA), vp, vp, vp, vp, vp, i64, i64, C.c_int32, vp, i32, vp]
     L.hlynr_policy_create.argtypes = [i32, C.POINTER(vp)]
     L.hlynr_policy_create_dim.argtypes = [i32, i32, C.POINTER(vp)]
     L.hlynr_policy_destroy.argtypes = [vp]
@@ -133,6 +135,8 @@ def load(build_if_missing=True):
     if L.hlynr_curriculum_schedule_size() != C.sizeof(abi.HlynrCurriculumSchedule):
         raise HlynrError(f"HlynrCurriculumSchedule layout mismatch: C {L.hlynr_curriculum_schedule_size()} vs ctypes "
                          f"{C.sizeof(abi.HlynrCurriculumSchedule)}")
+    if L.hlynr_trace_row_size() != abi.trace_row_numpy_dtype().itemsize:
+        raise HlynrError(f"HlynrTraceRow layout mismatch: C {L.hlynr_trace_row_size()} vs numpy {abi.trace_row_numpy_dtype().itemsize}")
     _LIB = L
     return L
 

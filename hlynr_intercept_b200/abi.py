@@ -100,6 +100,21 @@ def done_record_numpy_dtype():
     return dt
 
 
+def trace_row_numpy_dtype():
+    """numpy structured dtype with the exact memory layout of HlynrTraceRow (include/hlynr_rollout.h, 18 words)."""
+    import numpy as np
+
+    dt = np.dtype([("interceptor_pos", np.float32, (3,)), ("missile_pos", np.float32, (3,)), ("action", np.float32, (ACT_DIM,)),
+                   ("reward", np.float32), ("distance", np.float32), ("fuel_remaining", np.float32), ("radar_quality", np.float32),
+                   ("flags", np.uint32), ("step", np.int32)])
+    assert dt.itemsize == 72, dt.itemsize
+    return dt
+
+
+# the info fields a trace row reads (hlynr_eval_trace): the evaluator asks hlynr_step for these only
+TRACE_INFO_FIELDS = ("distance", "fuel_remaining", "steps", "flags", "interceptor_pos", "missile_pos", "radar_quality")
+
+
 STATS_FIELDS = ["episodes", "successes", "return_sum", "length_sum", "min_distance_sum", "final_distance_sum",
                 "hit_target", "interceptor_crash", "fuel_out", "missile_ground", "worsening", "timeouts",
                 "env_steps", "onboard_locks", "reserved0", "reserved1"]

@@ -59,6 +59,45 @@ __global__ void eval_record_kernel(const HlynrDoneRecord* __restrict__ recs, con
     if (taken && (threadIdx.x & 31) == 0) atomicAdd(remaining, (unsigned long long)(-(long long)taken));
 }
 
+static_assert(sizeof(HlynrTraceRow) == 72, "HlynrTraceRow is 18 words");
+
+// the info arrays a trace row reads (hlynr_step writes them; the step kernel skips a NULL field)
+struct TraceInfo {
+    const float *distance, *fuel_remaining, *radar_quality, *interceptor_pos, *missile_pos;
+    const int32_t* steps;
+    const uint8_t* flags;
+};
+
+// One thread per env.  The row is addressed by the env's episode index counts[e] (not yet incremented for the terminal tick:
+// eval_record_kernel runs after this one) and the tick's info['steps'], so no cursor is kept and nothing in the arguments
+// changes from tick to tick: a recorded chunk graph writes the same rows as eager launches.
+__global__ void __launch_bounds__(256) eval_trace_kernel(TraceInfo in, const float* __restrict__ actions, const float* __restrict__ rewards,
+                                                         const uint8_t* __restrict__ terminated, const uint8_t* __restrict__ truncated,
+                                                         const int32_t* __restrict__ counts, int64_t n_envs, int64_t q, int64_t rem,
+                                                         int32_t max_steps, HlynrTraceRow* __restrict__ table) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n_envs) return;
+    const int64_t full = n_envs - rem;   // targets and offsets as in eval_record_kernel
+    const int32_t c = counts[e];
+    if (c >= (e < full ? q : q + 1)) return;   // past the env's quota: SB3 ignores the episode
+    const int32_t s = in.steps[e];
+    if (s < 1 || s > max_steps) return;
+    HlynrTraceRow* r = table + (e * q + (e > full ? e - full : 0) + c) * max_steps + (s - 1);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        r->interceptor_pos[k] = in.interceptor_pos[3 * e + k];
+        r->missile_pos[k] = in.missile_pos[3 * e + k];
+    }
+#pragma unroll
+    for (int k = 0; k < 6; ++k) r->action[k] = actions[6 * e + k];
+    r->reward = rewards[e];
+    r->distance = in.distance[e];
+    r->fuel_remaining = in.fuel_remaining[e];
+    r->radar_quality = in.radar_quality[e];
+    r->flags = (uint32_t)in.flags[e] | (terminated[e] ? HLYNR_DONE_TERMINATED : 0u) | (truncated[e] ? HLYNR_DONE_TRUNCATED : 0u);
+    r->step = s;
+}
+
 // one thread per env, reverse scan over T; every access is coalesced over N
 __global__ void __launch_bounds__(256) gae_kernel(const float* __restrict__ rew, const float* __restrict__ val, const float* __restrict__ starts,
                                                   const float* __restrict__ last_val, const uint8_t* __restrict__ last_done, int64_t T,
@@ -122,6 +161,30 @@ int hlynr_eval_record(const HlynrDoneRecord* records_dev, const int32_t* counter
     eval_record_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(records_dev, counter_dev, n_envs, n_episodes / n_envs, n_episodes % n_envs,
                                                                  counts_dev, ticks_dev, results_dev, end_tick_dev,
                                                                  reinterpret_cast<unsigned long long*>(remaining_dev));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+size_t hlynr_trace_row_size(void) { return sizeof(HlynrTraceRow); }
+
+int hlynr_eval_trace(const HlynrInfoSoA* info, const float* actions_dev, const float* rewards_dev, const uint8_t* terminated_dev,
+                     const uint8_t* truncated_dev, const int32_t* counts_dev, int64_t n_envs, int64_t n_episodes,
+                     int32_t max_steps, HlynrTraceRow* table_dev, int device, void* stream) {
+    if (!info || !actions_dev || !rewards_dev || !terminated_dev || !truncated_dev || !counts_dev || !table_dev)
+        return fail("hlynr_eval_trace: null argument");
+    if (!info->distance || !info->fuel_remaining || !info->steps || !info->flags || !info->interceptor_pos || !info->missile_pos ||
+        !info->radar_quality)
+        return fail("hlynr_eval_trace: null argument (info: distance, fuel_remaining, steps, flags, interceptor_pos, missile_pos "
+                    "and radar_quality are read)");
+    if (n_envs <= 0 || n_envs > INT32_MAX) return fail("hlynr_eval_trace: n_envs must be in [1, INT32_MAX]");
+    if (n_episodes <= 0 || n_episodes > INT32_MAX) return fail("hlynr_eval_trace: n_episodes must be in [1, INT32_MAX]");
+    if (max_steps <= 0) return fail("hlynr_eval_trace: max_steps must be positive");
+    DeviceGuard g(device);
+    const TraceInfo in{info->distance, info->fuel_remaining, info->radar_quality, info->interceptor_pos, info->missile_pos,
+                       info->steps, info->flags};
+    eval_trace_kernel<<<(unsigned)((n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        in, actions_dev, rewards_dev, terminated_dev, truncated_dev, counts_dev, n_envs, n_episodes / n_envs, n_episodes % n_envs,
+        max_steps, table_dev);
     CK(cudaGetLastError());
     return 0;
 }

@@ -6,13 +6,16 @@ The reference writes one `<log_dir>/episodes/<episode_id>.jsonl` per episode thr
 `footer` line with the outcome and the metrics of inference.py:588-606.  When the reference's own scripts drive
 `HlynrVecEnv` they keep using their own logger on the `infos`; this recorder is for callers of the tensor API, where
 nothing per-env ever reaches the host unless asked: it follows ONE env of the batch (lazy: one 400-byte state export per
-tick) and writes the same records.
+tick) and writes the same records.  `write_episodes` writes the same files for every episode of an evaluation traced on the
+device (`DeviceEvaluator.evaluate(..., trace=True)`), which steps every env with auto-reset inside CUDA graphs.
 """
 import json
 import os
 import time
 
 import numpy as np
+
+from . import abi
 
 
 class EpisodeRecorder:
@@ -71,3 +74,52 @@ class EpisodeRecorder:
                                 "outcome": outcome, "metrics": metrics}) + "\n")
         self.file = None
         return True
+
+
+def write_episodes(log_dir, result, dt, metadata=None):
+    """Writes `<log_dir>/episodes/ep_XXXXXX.jsonl` (ep_000001 first) for every episode of an EvalResult of
+    `DeviceEvaluator.evaluate(..., trace=True)`, in SB3's order, with the lines EpisodeRecorder writes: header, per tick an
+    `interceptor` state (position, fuel, action) and a `missile` state (position), footer.  The metrics are EpisodeRecorder's:
+    total_reward is the float64 sum of the rewards in tick order, min_distance the minimum of the ticks' info['distance'],
+    final_distance the last tick's, fuel_used the done record's.
+
+    The ticks ran in batches on the device, not one at a time on the host, so time is simulated time: a state line's
+    `timestamp` is (step - 1) * dt (EpisodeRecorder: wall-clock seconds since the episode began), the footer's `duration` is
+    steps * dt, and `start_time` / `end_time` are the wall clock at writing and that plus the duration.  `fuel` is
+    info['fuel_remaining'] (float32; EpisodeRecorder logs the state's float64).  Returns the paths written."""
+    rows, off = result.trajectories, result.trajectory_offsets
+    if rows is None or off is None:
+        raise ValueError("the result has no trajectories: evaluate with trace=True")
+    if len(off) != len(result.records) + 1:
+        raise ValueError(f"{len(off) - 1} trajectories for {len(result.records)} episodes")
+    dt = float(dt)
+    out_dir = os.path.join(log_dir, "episodes")
+    os.makedirs(out_dir, exist_ok=True)
+    metadata = dict(metadata or {})
+    paths = []
+    for i, rec in enumerate(result.records):
+        ep = rows[off[i]:off[i + 1]]
+        episode_id = f"ep_{i + 1:06d}"
+        t0 = time.time()
+        lines = [{"type": "header", "episode_id": episode_id, "start_time": t0, "metadata": metadata}]
+        total, min_d = 0.0, float("inf")
+        ipos, mpos, act = ep["interceptor_pos"].tolist(), ep["missile_pos"].tolist(), ep["action"].tolist()
+        for k, (step, fuel, reward, dist) in enumerate(zip(ep["step"].tolist(), ep["fuel_remaining"].tolist(), ep["reward"].tolist(),
+                                                            ep["distance"].tolist())):
+            ts = (step - 1) * dt
+            lines.append({"type": "state", "timestamp": ts, "entity_id": "interceptor",
+                          "state": {"position": ipos[k], "fuel": fuel, "action": act[k]}})
+            lines.append({"type": "state", "timestamp": ts, "entity_id": "missile", "state": {"position": mpos[k]}})
+            total += reward
+            min_d = min(min_d, dist)
+        duration = len(ep) * dt
+        outcome = "intercepted" if int(ep["flags"][-1]) & abi.INFO_INTERCEPTED else "failed"     # inference.py:586
+        metrics = {"total_reward": total, "steps": len(ep), "final_distance": float(ep["distance"][-1]),
+                   "min_distance": min_d, "fuel_used": float(rec["fuel_used"])}
+        lines.append({"type": "footer", "episode_id": episode_id, "end_time": t0 + duration, "duration": duration,
+                      "outcome": outcome, "metrics": metrics})
+        path = os.path.join(out_dir, episode_id + ".jsonl")
+        with open(path, "w") as f:
+            f.write("".join(json.dumps(x) + "\n" for x in lines))
+        paths.append(path)
+    return paths

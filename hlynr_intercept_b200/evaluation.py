@@ -11,6 +11,11 @@ as in SB3.
 One tick here is the policy's action clipped to [-1, 1] (the mean with deterministic=True, a sample otherwise), `pipe.step` and
 `hlynr_eval_record` (include/hlynr_rollout.h), which files each counted episode's done record in a table addressed by
 (env, episode index), with the step it ended on.  The host reads one counter per chunk of ticks; with graph=True a chunk is one CUDA graph launch.
+
+evaluate(..., trace=True) also keeps every tick of every counted episode: `pipe.step` writes the tick's info arrays and
+`hlynr_eval_trace`, launched before `hlynr_eval_record`, files each env's row at (episode slot, info['steps']).  The rows are
+what the reference's offline inference logs per tick (inference.py:535-606); episode_log.write_episodes writes them as its
+episode JSONL files.
 """
 import ctypes as C
 import dataclasses
@@ -52,6 +57,8 @@ class EvalResult:
     mean_min_distance: float
     mean_fuel_used: float
     ticks: int                    # ticks run
+    trajectories: np.ndarray = None       # evaluate(trace=True): abi.trace_row_numpy_dtype() rows of every episode, in `records` order
+    trajectory_offsets: np.ndarray = None  # int64 [E+1]: episode i is trajectories[offsets[i]:offsets[i+1]], episode_lengths[i] rows
 
 
 class DeviceEvaluator:
@@ -93,6 +100,8 @@ class DeviceEvaluator:
         self._rec_dtype = abi.done_record_numpy_dtype()
         self._n_episodes, self._results, self._end_tick = 0, None, None
         self._deterministic = True
+        self._trace_dtype = abi.trace_row_numpy_dtype()
+        self._table = self._info = self._info_struct = None   # evaluate(trace=True) only
 
     def _tick(self):
         torch, sim = _torch(), self.sim
@@ -103,23 +112,36 @@ class DeviceEvaluator:
             act = self.policy.mean(self.obs).float().clamp(-1.0, 1.0)
         else:   # SB3's predict(deterministic=False): a sample, clipped to the Box bounds
             act = self.policy(self.obs)[0].float().clamp(-1.0, 1.0)
-        _, _, _, _, (records, counter, _) = self.pipe.step(act, out=self.obs)
         p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
+        stream = C.c_void_p(torch.cuda.current_stream(sim.device).cuda_stream)
+        if self._table is None:
+            _, _, _, _, (records, counter, _) = self.pipe.step(act, out=self.obs)
+        else:
+            _, rew, term, trunc, (records, counter, _) = self.pipe.step(act, out=self.obs, info=self._info_struct)
+            if not act.is_contiguous():
+                act = act.contiguous()
+            # before hlynr_eval_record: the terminal tick's row goes to the episode it ends, not to the next slot
+            _lib.check(sim.L.hlynr_eval_trace(C.byref(self._info_struct), p(act), p(rew), p(term), p(trunc), p(self.counts), sim.n,
+                                              self._n_episodes, self._max_steps, p(self._table), sim.device_index, stream))
         _lib.check(sim.L.hlynr_eval_record(p(records), p(counter), sim.n, self._n_episodes, p(self.counts), p(self.ticks),
-                                           p(self._results), p(self._end_tick), p(self.remaining), sim.device_index,
-                                           C.c_void_p(torch.cuda.current_stream(sim.device).cuda_stream)))
+                                           p(self._results), p(self._end_tick), p(self.remaining), sim.device_index, stream))
 
     def _chunk(self):
         for _ in range(self.chunk):
             self._tick()
 
-    def evaluate(self, n_eval_episodes, graph=True, deterministic=True):
+    def evaluate(self, n_eval_episodes, graph=True, deterministic=True, trace=False):
         """Resets the pipeline and runs until every env has finished its quota.  graph=True: chunks of `chunk` ticks, the
         first one eager, the others as replays of one CUDA graph, so `ticks` is a multiple of `chunk`; graph=False: the
         counter is read after every tick and `ticks` is the step on which the last counted episode ended.
         deterministic=False samples the action, as SB3's evaluate_policy(..., deterministic=False): the fused policy draws at
         its device-side noise counter, one step per tick, so every graph replay draws fresh noise; a torch module draws from
-        torch's generator."""
+        torch's generator.
+        trace=True also records every tick of every counted episode into `trajectories` / `trajectory_offsets` of the result
+        (abi.trace_row_numpy_dtype(): positions, clipped action, reward, distance, fuel, radar quality, info flags | done bits,
+        info['steps']).  It allocates a device table of E x max_steps rows of 72 bytes (E = 4096, max_steps = 1000: 295 MB)
+        and [N]-sized info arrays (41 B per env), and adds one launch and 72 B of writes per env and tick; the evaluation
+        itself is unchanged, bit for bit.  trace=False allocates and launches nothing extra."""
         torch = _torch()
         E = int(n_eval_episodes)
         if not 1 <= E <= INT32_MAX:
@@ -132,12 +154,7 @@ class DeviceEvaluator:
         n = self.sim.n
         # every episode ends within max_steps ticks, and an env needs at most ceil(E / n) of them
         limit = -(-E // n) * int(self.sim.params.max_steps) + self.chunk
-        self._n_episodes = E
-        self._results = torch.empty(E * self._rec_dtype.itemsize, dtype=torch.uint8, device=self.sim.device)
-        self._end_tick = torch.empty(E, dtype=torch.int64, device=self.sim.device)
-        self.counts.zero_()
-        self.ticks.zero_()
-        self.remaining.fill_(E)
+        self._prepare(E, trace)
         ticks = 0
         with torch.no_grad():
             self.pipe.reset(out=self.obs)
@@ -157,6 +174,40 @@ class DeviceEvaluator:
                     ticks += 1
         return self._result(ticks)
 
+    def _prepare(self, E, trace):
+        """The per-evaluation device state: result table, zeroed quota counters, and with trace the row table and info arrays."""
+        torch = _torch()
+        self._n_episodes = E
+        self._results = torch.empty(E * self._rec_dtype.itemsize, dtype=torch.uint8, device=self.sim.device)
+        self._end_tick = torch.empty(E, dtype=torch.int64, device=self.sim.device)
+        self.counts.zero_()
+        self.ticks.zero_()
+        self.remaining.fill_(E)
+        self._max_steps = int(self.sim.params.max_steps)
+        if trace:
+            dev, n = self.sim.device, self.sim.n
+            self._table = torch.empty(E * self._max_steps * self._trace_dtype.itemsize, dtype=torch.uint8, device=dev)
+            dt = {"float32": torch.float32, "int32": torch.int32, "uint8": torch.uint8}
+            self._info = {name: torch.empty((n,) + shp, dtype=dt[d], device=dev) for name, d, shp in abi.INFO_FIELDS
+                          if name in abi.TRACE_INFO_FIELDS}
+            self._info_struct = abi.HlynrInfoSoA(**{k: v.data_ptr() for k, v in self._info.items()})
+        else:
+            self._table = self._info = self._info_struct = None
+
+    def _trajectories(self, order, lengths):
+        """Rows [0, l) of each episode's max_steps slots, episodes in SB3's order; only those rows leave the device."""
+        torch = _torch()
+        lengths = lengths.astype(np.int64)
+        if len(lengths) and lengths.max() > self._max_steps:
+            raise RuntimeError(f"an episode ran {int(lengths.max())} steps, more than the table's max_steps={self._max_steps} rows")
+        offsets = np.zeros(len(lengths) + 1, dtype=np.int64)
+        np.cumsum(lengths, out=offsets[1:])
+        first = order.astype(np.int64) * self._max_steps   # table slot k of the record now at position i is order[i]
+        idx = np.repeat(first - offsets[:-1], lengths) + np.arange(offsets[-1], dtype=np.int64)
+        table = self._table.view(-1, self._trace_dtype.itemsize)
+        rows = table.index_select(0, torch.from_numpy(idx).to(table.device)).cpu().numpy()
+        return rows.reshape(-1).view(self._trace_dtype), offsets
+
     def _check_limit(self, ticks, limit):
         if ticks >= limit:
             raise RuntimeError(f"{int(self.remaining.item())} of {self._n_episodes} episodes still unfinished after {ticks} ticks, "
@@ -168,7 +219,12 @@ class DeviceEvaluator:
         order = np.lexsort((recs["env"], end))   # SB3 appends in step order, and within a step in env order
         recs, end = recs[order], end[order]
         rewards = recs["episode_return"].astype(np.float64).round(6)
+        rows = offsets = None
+        if self._table is not None:
+            rows, offsets = self._trajectories(order, recs["steps"])
+            self._table = self._info = self._info_struct = None
         return EvalResult(records=recs, end_tick=end, episode_rewards=rewards, episode_lengths=recs["steps"].copy(),
+                          trajectories=rows, trajectory_offsets=offsets,
                           mean_reward=float(np.mean(rewards)), std_reward=float(np.std(rewards)),
                           success_rate=float(np.mean((recs["flags"] & abi.INFO_INTERCEPTED) != 0)),
                           mean_min_distance=float(np.mean(recs["min_distance"].astype(np.float64))),

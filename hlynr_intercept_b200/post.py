@@ -83,12 +83,17 @@ class HlynrObsPipeline:
         _lib.check(self.L.hlynr_post_reset(self.h, C.c_void_p(dst.data_ptr()), self._train_flag(), self._stream()))
         return dst
 
-    def step(self, actions, auto_reset=True, out=None, reward_out=None):
+    def step(self, actions, auto_reset=True, out=None, reward_out=None, info=None):
         """One tick + post-processing.  Returns (obs[N, Fk], reward[N], terminated[N], truncated[N], done) where
         `done` = (records uint8 tensor viewable with abi.done_record_numpy_dtype, counter int32[1],
         terminal_obs[capacity, Fk] or None): row r of terminal_obs is the stacked + normalised
-        info['terminal_observation'] of record r.  All tensors are overwritten by the next call."""
+        info['terminal_observation'] of record r.  All tensors are overwritten by the next call.
+        info: None, an abi.HlynrInfoSoA of device pointers, or a dict of device tensors named as in abi.INFO_FIELDS (any
+        subset, each of that field's dtype and shape): hlynr_step writes the tick's info there (for an env reset in this
+        call: its terminal tick's)."""
         t, sim = self._torch, self.sim
+        if isinstance(info, dict):
+            info = self._info_struct(info)
         if not (actions.is_cuda and actions.dtype == t.float32 and actions.shape == (sim.n, 6) and actions.is_contiguous()):
             actions = actions.to(device=sim.device, dtype=t.float32).reshape(sim.n, 6).contiguous()
         o = sim._alloc_out()
@@ -97,14 +102,28 @@ class HlynrObsPipeline:
         self._counter.zero_()
         st = self._stream()
         _lib.check(self.L.hlynr_step(sim.h, C.c_void_p(actions.data_ptr()), self._target(), C.c_void_p(rew.data_ptr()),
-                                     C.c_void_p(o["terminated"].data_ptr()), C.c_void_p(o["truncated"].data_ptr()), None, None,
-                                     int(auto_reset), st))
+                                     C.c_void_p(o["terminated"].data_ptr()), C.c_void_p(o["truncated"].data_ptr()), None,
+                                     None if info is None else C.byref(info), int(auto_reset), st))
         _lib.check(self.L.hlynr_post_step(self.h, C.c_void_p(rew.data_ptr()), C.c_void_p(o["terminated"].data_ptr()),
                                           C.c_void_p(o["truncated"].data_ptr()), C.c_void_p(self._records.data_ptr()),
                                           C.c_void_p(self._counter.data_ptr()), sim.n, C.c_void_p(dst.data_ptr()),
                                           C.c_void_p(self._terminal.data_ptr()) if self._terminal is not None else None,
                                           self._train_flag(), st))
         return dst, rew, o["terminated"], o["truncated"], (self._records, self._counter, self._terminal)
+
+    def _info_struct(self, tensors):
+        t, n = self._torch, self.sim.n
+        fields = {name: (dt, shp) for name, dt, shp in abi.INFO_FIELDS}
+        ptrs = {}
+        for name, x in tensors.items():
+            if name not in fields:
+                raise ValueError(f"unknown info field {name!r}; the fields are {list(fields)}")
+            dt, shp = fields[name]
+            if not (x.is_cuda and x.device == self.sim.device and x.dtype == getattr(t, dt) and tuple(x.shape) == (n,) + shp
+                    and x.is_contiguous()):
+                raise ValueError(f"info[{name!r}] must be a contiguous {dt} tensor of shape {(n,) + shp} on {self.sim.device}")
+            ptrs[name] = x.data_ptr()
+        return abi.HlynrInfoSoA(**ptrs)
 
     def done_records(self):
         """Host copy of the finished episodes of the last step (synchronises)."""

@@ -11,6 +11,7 @@
  *       train_flat_ppo.py:431-448 through model.learn)
  *   evaluate_policy's per-env episode quotas (EvalCallback, train_flat_ppo.py:497-504):          hlynr_eval_record
  *       "if episode_counts[i] < episode_count_targets[i] and dones[i]: append info['episode']"
+ *   inference.py:535-606 logging every tick of each evaluated episode (UnifiedLogger, logger.py:148-273)  hlynr_eval_trace
  *
  * Conventions as in hlynr.h.
  */
@@ -54,6 +55,31 @@ int hlynr_gae(const float* rewards_dev, const float* values_dev, const float* ep
 int hlynr_eval_record(const HlynrDoneRecord* records_dev, const int32_t* counter_dev, int64_t n_envs, int64_t n_episodes,
                       int32_t* counts_dev, int64_t* ticks_dev, HlynrDoneRecord* results_dev, int64_t* end_tick_dev,
                       int64_t* remaining_dev, int device, void* stream);
+
+/* One tick of one evaluated episode: the values of the reference's info dict for that tick (environment.py:829-857) that its
+ * offline inference logs per tick (inference.py:535-548), plus the action, reward and done bits. */
+typedef struct HlynrTraceRow {
+    float interceptor_pos[3], missile_pos[3];   /* info['interceptor_pos'], info['missile_pos'] */
+    float action[6];                            /* the clipped action the env received */
+    float reward, distance, fuel_remaining, radar_quality;
+    uint32_t flags;                             /* HLYNR_INFO_* bits of the tick; | HLYNR_DONE_TERMINATED / _TRUNCATED on the last row */
+    int32_t step;                               /* info['steps'], 1-based */
+} HlynrTraceRow;                                /* 18 words = 72 bytes */
+size_t hlynr_trace_row_size(void);
+
+/* Files the tick's row of every env still inside its evaluate_policy quota (counts_dev[e] < target_e, targets and offset_e as
+ * in hlynr_eval_record) at table_dev[(offset_e + counts_dev[e]) * max_steps + steps[e] - 1]; a row whose steps[e] lies outside
+ * [1, max_steps] is not written.  Launch once per tick after hlynr_step (+ hlynr_post_step) and BEFORE hlynr_eval_record of the
+ * same tick, which increments counts_dev: the terminal tick is then still addressed to the episode it ends.  No argument changes
+ * between ticks, so a CUDA graph of the tick replays correctly.
+ *   info: host struct of the tick's device info arrays (what hlynr_step wrote); distance, fuel_remaining, steps, flags,
+ *         interceptor_pos, missile_pos and radar_quality must be set, the other fields are not read
+ *   actions_dev float[n_envs, 6], rewards_dev float[n_envs], terminated_dev / truncated_dev uint8[n_envs] (the step's outputs)
+ *   table_dev: n_episodes * max_steps rows; rows past an episode's length are left untouched
+ * n_envs and n_episodes must be in [1, INT32_MAX], max_steps positive. */
+int hlynr_eval_trace(const HlynrInfoSoA* info, const float* actions_dev, const float* rewards_dev, const uint8_t* terminated_dev,
+                     const uint8_t* truncated_dev, const int32_t* counts_dev, int64_t n_envs, int64_t n_episodes,
+                     int32_t max_steps, HlynrTraceRow* table_dev, int device, void* stream);
 
 #ifdef __cplusplus
 }
