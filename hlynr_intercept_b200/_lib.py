@@ -19,11 +19,12 @@ EXPORTS = [
     "hlynr_debug_draws", "hlynr_launch_count", "hlynr_set_option", "hlynr_set_done_list", "hlynr_done_records_host",
     "hlynr_ring_period", "hlynr_note_replayed_ticks", "hlynr_tick_count", "hlynr_pinned_done", "hlynr_host_done_buffer",
     "hlynr_curriculum_schedule_size", "hlynr_attach_curriculum", "hlynr_detach_curriculum", "hlynr_set_timesteps", "hlynr_get_timesteps",
-    "hlynr_debug_curriculum_at",
+    "hlynr_debug_curriculum_at", "hlynr_snapshot_info_size", "hlynr_snapshot_layout", "hlynr_snapshot_save", "hlynr_snapshot_load",
     # include/hlynr_post.h
     "hlynr_post_create", "hlynr_post_create_frames", "hlynr_post_destroy", "hlynr_post_obs_dim", "hlynr_post_obs_target", "hlynr_post_reset",
     "hlynr_post_step", "hlynr_post_original", "hlynr_post_normalize", "hlynr_post_get_stats", "hlynr_post_set_stats",
-    "hlynr_post_check_sums", "hlynr_post_launch_count", "hlynr_post_note_replayed_steps",
+    "hlynr_post_check_sums", "hlynr_post_launch_count", "hlynr_post_note_replayed_steps", "hlynr_post_snapshot_info_size",
+    "hlynr_post_snapshot_layout", "hlynr_post_snapshot_save", "hlynr_post_snapshot_load",
     # include/hlynr_rollout.h
     "hlynr_bootstrap_timeouts", "hlynr_gae", "hlynr_eval_record", "hlynr_trace_row_size", "hlynr_eval_trace",
     # include/hlynr_policy.h
@@ -70,6 +71,14 @@ def load(build_if_missing=True):
     L.hlynr_set_timesteps.argtypes = [vp, u64, vp]
     L.hlynr_get_timesteps.argtypes = [vp, C.POINTER(u64), vp]
     L.hlynr_debug_curriculum_at.argtypes = [vp, u64, C.POINTER(C.c_double)]
+    L.hlynr_snapshot_info_size.restype = C.c_size_t
+    L.hlynr_snapshot_layout.argtypes = [vp, C.POINTER(abi.HlynrSnapshotInfo), C.POINTER(C.c_size_t)]
+    L.hlynr_snapshot_save.argtypes = [vp, vp, C.POINTER(abi.HlynrSnapshotInfo), vp]
+    L.hlynr_snapshot_load.argtypes = [vp, C.POINTER(abi.HlynrSnapshotInfo), vp, vp]
+    L.hlynr_post_snapshot_info_size.restype = C.c_size_t
+    L.hlynr_post_snapshot_layout.argtypes = [vp, C.POINTER(abi.HlynrPostSnapshotInfo), C.POINTER(C.c_size_t)]
+    L.hlynr_post_snapshot_save.argtypes = [vp, vp, C.POINTER(abi.HlynrPostSnapshotInfo), vp]
+    L.hlynr_post_snapshot_load.argtypes = [vp, C.POINTER(abi.HlynrPostSnapshotInfo), vp, vp]
     L.hlynr_seed.argtypes = [vp, u64]
     L.hlynr_reset.argtypes = [vp, vp, vp, vp]
     L.hlynr_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(abi.HlynrInfoSoA), i32, vp]
@@ -135,6 +144,9 @@ def load(build_if_missing=True):
     if L.hlynr_curriculum_schedule_size() != C.sizeof(abi.HlynrCurriculumSchedule):
         raise HlynrError(f"HlynrCurriculumSchedule layout mismatch: C {L.hlynr_curriculum_schedule_size()} vs ctypes "
                          f"{C.sizeof(abi.HlynrCurriculumSchedule)}")
+    for name, cls in (("hlynr_snapshot_info_size", abi.HlynrSnapshotInfo), ("hlynr_post_snapshot_info_size", abi.HlynrPostSnapshotInfo)):
+        if getattr(L, name)() != C.sizeof(cls):
+            raise HlynrError(f"{cls.__name__} layout mismatch: C {getattr(L, name)()} vs ctypes {C.sizeof(cls)}")
     if L.hlynr_trace_row_size() != abi.trace_row_numpy_dtype().itemsize:
         raise HlynrError(f"HlynrTraceRow layout mismatch: C {L.hlynr_trace_row_size()} vs numpy {abi.trace_row_numpy_dtype().itemsize}")
     _LIB = L

@@ -1,5 +1,5 @@
 """ctypes mirror of include/hlynr.h (the C ABI).  Field order and types must match the header exactly;
-`hlynr_params_size()` / `hlynr_env_state_size()` are checked at load time."""
+`hlynr_params_size()` / `hlynr_env_state_size()` / `hlynr_snapshot_info_size()` are checked at load time."""
 import ctypes as C
 
 ABI_VERSION = 1
@@ -161,3 +161,59 @@ def env_state_numpy_dtype():
     dt = np.dtype(fields, align=True)
     assert dt.itemsize == C.sizeof(HlynrEnvState), (dt.itemsize, C.sizeof(HlynrEnvState))
     return dt
+
+
+# ---- snapshots (include/hlynr.h hlynr_snapshot_*, include/hlynr_post.h hlynr_post_snapshot_*) ----
+SNAPSHOT_VERSION = 1
+SNAP_SECTIONS = ("real", "int", "onboard_ring", "ground_ring", "stats", "curriculum")
+
+
+class HlynrSnapshotInfo(C.Structure):
+    _fields_ = [("format_version", C.c_int32), ("abi_version", C.c_int32), ("precision", C.c_int32), ("obs_dim", C.c_int32),
+                ("n_envs", C.c_int64), ("env_id_offset", C.c_int64), ("seed", C.c_uint64),
+                ("volley_k", C.c_int32), ("onboard_ring_len", C.c_int32), ("ground_ring_len", C.c_int32),
+                ("curriculum_attached", C.c_int32), ("tick", C.c_uint64), ("env_steps", C.c_double),
+                ("curriculum_increment", C.c_int64), ("params", HlynrParams), ("curriculum", HlynrCurriculum),
+                ("schedule", HlynrCurriculumSchedule), ("section_offset", C.c_uint64 * len(SNAP_SECTIONS)), ("device_bytes", C.c_uint64)]
+
+
+POST_SNAPSHOT_VERSION = 1
+POST_SNAP_SECTIONS = ("frames", "age", "returns", "stats")
+
+
+class HlynrPostSnapshotInfo(C.Structure):
+    _fields_ = [("format_version", C.c_int32), ("frame_dim", C.c_int32), ("n_stack", C.c_int32), ("sums_valid", C.c_int32),
+                ("n_envs", C.c_int64), ("t", C.c_uint64), ("clip_obs", C.c_double), ("epsilon", C.c_double), ("gamma", C.c_double),
+                ("stats_bytes", C.c_uint64), ("section_offset", C.c_uint64 * len(POST_SNAP_SECTIONS)), ("device_bytes", C.c_uint64)]
+
+
+def struct_to_dict(s):
+    """A ctypes structure as plain Python values (nested structures as dicts, arrays as lists): JSON-serialisable, and exact
+    for every double (json writes the shortest repr that reads back to the same bits)."""
+    def val(v):
+        if isinstance(v, C.Structure):
+            return struct_to_dict(v)
+        if isinstance(v, C.Array):
+            return [val(x) for x in v]
+        return v
+
+    return {name: val(getattr(s, name)) for name, _ in s._fields_}
+
+
+def struct_from_dict(cls, d):
+    """The inverse of struct_to_dict; refuses a missing or unknown field."""
+    names = [name for name, _ in cls._fields_]
+    if set(d) != set(names):
+        raise ValueError(f"{cls.__name__}: fields {sorted(set(d) ^ set(names))} are missing or unknown")
+    s = cls()
+    for name, ctype in cls._fields_:
+        v = d[name]
+        if isinstance(ctype, type) and issubclass(ctype, C.Structure):
+            setattr(s, name, struct_from_dict(ctype, v))
+        elif isinstance(ctype, type) and issubclass(ctype, C.Array):
+            if len(v) != ctype._length_:
+                raise ValueError(f"{cls.__name__}.{name}: {len(v)} values, expected {ctype._length_}")
+            setattr(s, name, ctype(*v))
+        else:
+            setattr(s, name, v)
+    return s

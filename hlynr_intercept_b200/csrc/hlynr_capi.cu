@@ -215,6 +215,14 @@ template <class F> static auto with_planes(hlynr_sim* s, F&& f) {
 template <class P> struct PlanesReal;
 template <class R> struct PlanesReal<StatePlanes<R>> { using type = R; };
 template <class P> using real_of = typename PlanesReal<std::decay_t<P>>::type;
+// with_planes plus the handle's plane layout as std::integral_constant<int, C>, C = s->compact (0 wide, 1 compact, 2 DR-compact;
+// the compact layouts exist in the fp32 build only): the instantiations of the snapshot kernels.
+template <class F> static void with_layout(hlynr_sim* s, F&& f) {
+    if (s->precision != HLYNR_FP32) f(s->pd, std::integral_constant<int, 0>{});
+    else if (s->compact == 1) f(s->pf, std::integral_constant<int, 1>{});
+    else if (s->compact == 2) f(s->pf, std::integral_constant<int, 2>{});
+    else f(s->pf, std::integral_constant<int, 0>{});
+}
 
 // ------------------------------------------------------------------------------------------------
 // parameter conversion
@@ -426,6 +434,88 @@ template <typename R> __global__ void import_kernel(KernelArgs<R> A, int64_t fir
     KernelArgs<R> B = A;
     B.P.thrust_dyn = 1; B.P.dr = 1;
     store_env(B, first + j, e);
+}
+
+// ---- snapshots (include/hlynr.h): the canonical image <-> the state planes ----------------------------------------------------
+// Columns of the image (the section list of hlynr.h), n envs each.
+template <typename R> struct SnapImage {
+    R* real;
+    int32_t* ints;
+    R* onb;
+    R* gnd;
+    int64_t n;
+};
+// pack: column <- state; unpack: state <- column.  Every value round-trips exactly (float state is widened to R).
+template <bool kPack, typename T, typename U> __device__ __forceinline__ void snap_move(T& v, U* col) {
+    if constexpr (kPack) *col = (U)v; else v = (T)*col;
+}
+// The one list of the image's columns, walked in both directions.  The per-env planes go through load_env / store_env, which know
+// where each field sits in the handle's layout (Compact = KernelArgs::compact: 0 wide, 1 compact, 2 DR-compact); the volley and
+// ring planes are addressed as the step, export and import kernels address them.
+template <bool kPack, typename R, int Compact> __device__ void snapshot_env(const KernelArgs<R>& A, const SnapImage<R>& S, int64_t i) {
+    KernelArgs<R> B = A;
+    B.P.thrust_dyn = 1; B.P.dr = 1;   // the optional planes are always allocated and initialised: move them unconditionally
+    B.compact = Compact;
+    const int64_t n = S.n, stride = A.ring_stride;
+    Env<R> e;
+    if constexpr (kPack) load_env(B, i, e); else e.flags = 0;
+    R* rc = S.real + i;
+    auto mr = [&](auto& v) { snap_move<kPack>(v, rc); rc += n; };
+    mr(e.ipx); mr(e.ipy); mr(e.ipz); mr(e.fuel); mr(e.ivx); mr(e.ivy); mr(e.ivz); mr(e.fuel_used);
+    mr(e.mpx); mr(e.mpy); mr(e.mpz); mr(e.prev_d); mr(e.mvx); mr(e.mvy); mr(e.mvz); mr(e.last_d);
+    mr(e.kpx); mr(e.kpy); mr(e.kpz); mr(e.min_d); mr(e.kvx); mr(e.kvy); mr(e.kvz); mr(e.ep_ret);
+    mr(e.thx); mr(e.thy); mr(e.thz); mr(e.T0); mr(e.qw); mr(e.qx); mr(e.qy); mr(e.qz);
+    mr(e.wx); mr(e.wy); mr(e.wz); mr(e.Ppp); mr(e.Ppv); mr(e.Pvp); mr(e.Pvv); mr(e.base_cd); mr(e.peak);
+    int32_t* ic = S.ints + i;
+    auto mi = [&](int& v) { snap_move<kPack>(v, ic); ic += n; };
+    int crossed = e.flags & FLAG_CROSSED ? 1 : 0, kf_init = e.flags & FLAG_KF_INIT ? 1 : 0, kf_f64 = e.flags & FLAG_KF_F64 ? 1 : 0;
+    int odelay = FLAG_ODELAY(e.flags), vcur = FLAG_VCUR(e.flags), vcount = FLAG_VCOUNT(e.flags);
+    mi(e.steps); mi(e.worsen); mi(e.episode); mi(crossed); mi(kf_init); mi(kf_f64); mi(odelay); mi(vcur); mi(vcount);
+    for (int m = 0; m < A.P.volley_k; ++m) {
+        Vec4<R>* pa = A.st.vm + (int64_t)(2 * m) * stride + i;
+        Vec4<R>* pb = A.st.vm + (int64_t)(2 * m + 1) * stride + i;
+        Vec4<R> a{R(0), R(0), R(0), R(0)}, b = a;
+        if constexpr (kPack) { a = *pa; b = *pb; }
+        int act = b.w != R(0) ? 1 : 0;
+        mr(a.x); mr(a.y); mr(a.z); mr(a.w); mr(b.x); mr(b.y); mr(b.z); mi(act);
+        if constexpr (!kPack) { b.w = act ? R(1) : R(0); *pa = a; *pb = b; }
+    }
+    const int ol = A.P.onb_ring_len, gl = A.P.gnd_ring_len;
+    R* oc = S.onb + i;
+    for (int j = 0; j < ol; ++j) {   // age j = the sample written j ticks before the snapshot; A.o_row = the last tick's row
+        const int row = A.o_row - j < 0 ? A.o_row - j + ol : A.o_row - j;
+        float4* p = A.st.oring + (int64_t)row * stride + i;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if constexpr (kPack) v = *p;
+        snap_move<kPack>(v.x, oc); snap_move<kPack>(v.y, oc + n); snap_move<kPack>(v.z, oc + 2 * n); snap_move<kPack>(v.w, oc + 3 * n);
+        if constexpr (!kPack) *p = v;
+        oc += 4 * n;
+    }
+    R* gc = S.gnd + i;
+    for (int j = 0; j < gl; ++j) {
+        const int row = A.g_row - j < 0 ? A.g_row - j + gl : A.g_row - j;
+        Vec4<R>* p = A.st.gring + (int64_t)row * 2 * stride + i;
+        for (int h = 0; h < 2; ++h) {
+            Vec4<R> v{R(0), R(0), R(0), R(0)};
+            if constexpr (kPack) v = p[h * stride];
+            snap_move<kPack>(v.x, gc); snap_move<kPack>(v.y, gc + n); snap_move<kPack>(v.z, gc + 2 * n); snap_move<kPack>(v.w, gc + 3 * n);
+            if constexpr (!kPack) p[h * stride] = v;
+            gc += 4 * n;
+        }
+    }
+    if constexpr (!kPack) {
+        e.flags = (crossed ? FLAG_CROSSED : 0) | (kf_init ? FLAG_KF_INIT : 0) | (kf_f64 ? FLAG_KF_F64 : 0) | ((odelay & 0xf) << 8) |
+                  ((vcur & 0x7) << 12) | ((vcount & 0xf) << 16);
+        store_env(B, i, e);
+    }
+}
+template <typename R, int Compact> __global__ void snapshot_pack_kernel(const KernelArgs<R> A, const SnapImage<R> S) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < S.n; i += (int64_t)gridDim.x * blockDim.x)
+        snapshot_env<true, R, Compact>(A, S, i);
+}
+template <typename R, int Compact> __global__ void snapshot_unpack_kernel(const KernelArgs<R> A, const SnapImage<R> S) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < S.n; i += (int64_t)gridDim.x * blockDim.x)
+        snapshot_env<false, R, Compact>(A, S, i);
 }
 
 __global__ void debug_draw_kernel(const __grid_constant__ RoundKeys rk, int64_t env, uint32_t episode, uint32_t step,
@@ -759,15 +849,20 @@ int hlynr_step(hlynr_t* s, const float* actions_dev, float* obs_dev, float* rewa
                       auto_reset, (cudaStream_t)stream);
 }
 
-int hlynr_attach_curriculum(hlynr_t* s, const HlynrCurriculumSchedule* c, uint64_t num_timesteps, int64_t increment) {
-    if (!s || !c) return fail("hlynr_attach_curriculum: null argument");
+// The schedules hlynr_attach_curriculum (and hlynr_snapshot_load, which re-attaches one) accept.
+static int check_schedule(const HlynrCurriculumSchedule* c, int64_t increment, const char* who) {
     const double f[] = {c->initial_radius, c->final_radius, c->curriculum_steps, c->beam_initial, c->beam_final, c->beam_start,
                         c->beam_end, c->onboard_initial, c->onboard_final, c->onboard_start, c->onboard_end, c->ground_initial,
                         c->ground_final, c->ground_start, c->ground_end};
     for (double v : f)
-        if (!std::isfinite(v)) return fail("hlynr_attach_curriculum: every field of the schedule must be finite");
-    if (c->enabled && !(c->curriculum_steps > 0.0)) return fail("hlynr_attach_curriculum: curriculum_steps must be positive while the curriculum is enabled");
-    if (increment < 0) return fail("hlynr_attach_curriculum: increment must not be negative");
+        if (!std::isfinite(v)) return fail("%s: every field of the schedule must be finite", who);
+    if (c->enabled && !(c->curriculum_steps > 0.0)) return fail("%s: curriculum_steps must be positive while the curriculum is enabled", who);
+    if (increment < 0) return fail("%s: increment must not be negative", who);
+    return 0;
+}
+int hlynr_attach_curriculum(hlynr_t* s, const HlynrCurriculumSchedule* c, uint64_t num_timesteps, int64_t increment) {
+    if (!s || !c) return fail("hlynr_attach_curriculum: null argument");
+    if (check_schedule(c, increment, "hlynr_attach_curriculum")) return 1;
     DeviceGuard g(s->device);
     if (!s->cur_block) CK(cudaMalloc(&s->cur_block, sizeof(CurBlock<double>)));
     CK(cudaDeviceSynchronize());   // no launch of an earlier attachment still reads or writes the block
@@ -936,6 +1031,142 @@ int hlynr_debug_draws(hlynr_t* s, int64_t env_global_id, uint32_t episode, uint3
     s->launches += 1;
     return 0;
 }
+
+}  // extern "C"
+
+// ---- snapshots ---------------------------------------------------------------------------------------------------------------
+static_assert(HLYNR_STAT_ROWS == HLYNR_STAT_SLOTS + 1, "the image's statistics section is the whole statistics block");
+static_assert(sizeof(HlynrSnapshotInfo) == 952, "HlynrSnapshotInfo is mirrored by abi.HlynrSnapshotInfo");
+// every field of HlynrParams, compared one by one so that a refused load names the field
+#define HLYNR_PARAMS_FIELDS(X) \
+    X(abi_version) X(max_steps) X(dt) X(max_range) X(max_velocity) X(target) X(m_spawn_spherical) X(i_vel_toward_missile) \
+    X(m_pos_lo) X(m_pos_hi) X(m_speed_lo) X(m_speed_hi) X(m_radius_lo) X(m_radius_hi) X(m_az_lo) X(m_az_hi) X(m_el_lo) \
+    X(m_el_hi) X(i_pos_lo) X(i_pos_hi) X(i_vel_lo) X(i_vel_hi) X(i_speed_lo) X(i_speed_hi) X(base_wind) X(wind_variability) \
+    X(isa_enabled) X(mach_enabled) X(enh_wind_enabled) X(thrust_dyn_enabled) X(dr_enabled) X(validate_enabled) \
+    X(evasion_enabled) X(onboard_delay) X(sub_mach) X(sup_mach) X(peak_mult) X(sup_mult) X(blh) X(turb_intensity) \
+    X(gust_scale) X(thrust_tau) X(dr_variation) X(radar_range) X(radar_quality) X(ground_enabled) X(ground_delay) \
+    X(ground_pos) X(g_max_range) X(g_min_el) X(g_max_el) X(g_sigma_r) X(g_sigma_v) X(g_base_quality) X(max_datalink_range) \
+    X(datalink_packet_loss) X(obs_mode) X(precision_mode) X(fuze_enabled) X(volley_size) X(kill_radius)
+
+// The descriptor of the handle's current state, with the byte offsets of the image's sections (256-byte aligned).
+static void snapshot_describe(const hlynr_sim* s, HlynrSnapshotInfo* info) {
+    memset(info, 0, sizeof(*info));
+    const KParams<float> k = make_kparams<float>(s->params);
+    info->format_version = HLYNR_SNAPSHOT_VERSION; info->abi_version = HLYNR_ABI_VERSION;
+    info->precision = s->precision; info->obs_dim = s->obs_dim;
+    info->n_envs = s->n; info->env_id_offset = s->env_offset; info->seed = s->seed;
+    info->volley_k = s->params.volley_size; info->onboard_ring_len = k.onb_ring_len; info->ground_ring_len = k.gnd_ring_len;
+    info->curriculum_attached = s->cur_attached ? 1 : 0;
+    info->tick = s->tick; info->env_steps = s->env_steps;
+    info->params = s->params; info->curriculum = s->cur;
+    if (s->cur_attached) { info->schedule = s->sched; info->curriculum_increment = s->cur_increment; }
+    const size_t rs = s->precision == HLYNR_FP32 ? sizeof(float) : sizeof(double), n = (size_t)s->n, K = (size_t)s->params.volley_size;
+    const size_t bytes[HLYNR_SNAP_SECTIONS] = {(HLYNR_SNAP_REAL_COLS + 7 * K) * n * rs, (HLYNR_SNAP_INT_COLS + K) * n * sizeof(int32_t),
+                                               (size_t)k.onb_ring_len * 4 * n * rs, (size_t)k.gnd_ring_len * 8 * n * rs,
+                                               sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS, sizeof(uint64_t)};
+    size_t off = 0;
+    for (int j = 0; j < HLYNR_SNAP_SECTIONS; ++j) { info->section_offset[j] = off; off += (bytes[j] + 255) & ~size_t(255); }
+    info->device_bytes = off;
+}
+template <typename R> static SnapImage<R> snap_image(const HlynrSnapshotInfo& info, char* base) {
+    SnapImage<R> S;
+    S.real = (R*)(base + info.section_offset[HLYNR_SNAP_REAL]); S.ints = (int32_t*)(base + info.section_offset[HLYNR_SNAP_INT]);
+    S.onb = (R*)(base + info.section_offset[HLYNR_SNAP_ONBOARD]); S.gnd = (R*)(base + info.section_offset[HLYNR_SNAP_GROUND]);
+    S.n = info.n_envs;
+    return S;
+}
+// Launches the pack or unpack kernel of the handle's precision and layout; the ring rows of the last executed tick come from the
+// handle's tick (set_tick), so load restores the tick first.
+static int snapshot_kernels(hlynr_sim* s, const HlynrSnapshotInfo& info, char* base, bool pack, cudaStream_t st) {
+    const int grid = (int)std::min<int64_t>(grid_for(s->n, 256), (int64_t)s->sm_count * 8);
+    with_layout(s, [&](auto& planes, auto compact) {
+        using R = real_of<decltype(planes)>;
+        constexpr int C = decltype(compact)::value;
+        const KernelArgs<R> A = base_args(s, planes);
+        const SnapImage<R> S = snap_image<R>(info, base);
+        if (pack) snapshot_pack_kernel<R, C><<<grid, 256, 0, st>>>(A, S);
+        else snapshot_unpack_kernel<R, C><<<grid, 256, 0, st>>>(A, S);
+    });
+    CK(cudaGetLastError());
+    s->launches += 1;
+    return 0;
+}
+
+extern "C" {
+
+size_t hlynr_snapshot_info_size(void) { return sizeof(HlynrSnapshotInfo); }
+
+int hlynr_snapshot_layout(const hlynr_t* s, HlynrSnapshotInfo* info, size_t* device_bytes) {
+    if (!s || !info || !device_bytes) return fail("hlynr_snapshot_layout: null argument");
+    snapshot_describe(s, info);
+    *device_bytes = (size_t)info->device_bytes;
+    return 0;
+}
+
+int hlynr_snapshot_save(hlynr_t* s, void* dev_out, HlynrSnapshotInfo* info, void* stream) {
+    if (!s || !dev_out || !info) return fail("hlynr_snapshot_save: null argument");
+    DeviceGuard g(s->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (refuse_capture(st, "hlynr_snapshot_save")) return 1;
+    snapshot_describe(s, info);
+    char* base = (char*)dev_out;
+    if (snapshot_kernels(s, *info, base, true, st)) return 1;
+    CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_STATS], s->stats, sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
+                       cudaMemcpyDeviceToDevice, st));
+    if (s->cur_attached)   // CurBlock::num_timesteps is the block's first member
+        CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_CURRICULUM], s->cur_block, sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+    else
+        CK(cudaMemsetAsync(base + info->section_offset[HLYNR_SNAP_CURRICULUM], 0, sizeof(uint64_t), st));
+    return 0;
+}
+
+int hlynr_snapshot_load(hlynr_t* s, const HlynrSnapshotInfo* info, const void* dev_in, void* stream) {
+    if (!s || !info || !dev_in) return fail("hlynr_snapshot_load: null argument");
+    HlynrSnapshotInfo mine;
+    snapshot_describe(s, &mine);
+    const HlynrSnapshotInfo& in = *info;
+#define HLYNR_SNAP_REFUSE(cond, what, ...) if (cond) return fail("hlynr_snapshot_load: the snapshot's " what " differs from the handle's: " __VA_ARGS__)
+    HLYNR_SNAP_REFUSE(in.format_version != mine.format_version, "format version", "%d, expected %d", in.format_version, mine.format_version);
+    HLYNR_SNAP_REFUSE(in.abi_version != mine.abi_version, "ABI version", "%d, expected %d", in.abi_version, mine.abi_version);
+    HLYNR_SNAP_REFUSE(in.precision != mine.precision, "precision", "fp%d into an fp%d handle", in.precision, mine.precision);
+    HLYNR_SNAP_REFUSE(in.n_envs != mine.n_envs, "n_envs", "%lld, the handle has %lld", (long long)in.n_envs, (long long)mine.n_envs);
+    HLYNR_SNAP_REFUSE(in.env_id_offset != mine.env_id_offset, "env_id_offset", "%lld, the handle has %lld", (long long)in.env_id_offset,
+                      (long long)mine.env_id_offset);
+    HLYNR_SNAP_REFUSE(in.obs_dim != mine.obs_dim, "obs_dim", "%d, the handle has %d", in.obs_dim, mine.obs_dim);
+    HLYNR_SNAP_REFUSE(in.volley_k != mine.volley_k, "volley size K", "%d, the handle has %d", in.volley_k, mine.volley_k);
+    HLYNR_SNAP_REFUSE(in.onboard_ring_len != mine.onboard_ring_len, "onboard ring length", "%d, the handle has %d", in.onboard_ring_len,
+                      mine.onboard_ring_len);
+    HLYNR_SNAP_REFUSE(in.ground_ring_len != mine.ground_ring_len, "ground ring length", "%d, the handle has %d", in.ground_ring_len,
+                      mine.ground_ring_len);
+#define X(f) HLYNR_SNAP_REFUSE(memcmp(&in.params.f, &mine.params.f, sizeof(in.params.f)) != 0, "configuration", "field HlynrParams." #f);
+    HLYNR_PARAMS_FIELDS(X)
+#undef X
+    for (int j = 0; j < HLYNR_SNAP_SECTIONS; ++j)
+        HLYNR_SNAP_REFUSE(in.section_offset[j] != mine.section_offset[j], "image layout", "offset of section %d", j);
+    HLYNR_SNAP_REFUSE(in.device_bytes != mine.device_bytes, "image size", "%llu bytes, expected %llu", (unsigned long long)in.device_bytes,
+                      (unsigned long long)mine.device_bytes);
+#undef HLYNR_SNAP_REFUSE
+    if (in.curriculum_attached && check_schedule(&in.schedule, in.curriculum_increment, "hlynr_snapshot_load")) return 1;
+    DeviceGuard g(s->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (refuse_capture(st, "hlynr_snapshot_load")) return 1;
+    if (in.curriculum_attached && !s->cur_block) CK(cudaMalloc(&s->cur_block, sizeof(CurBlock<double>)));
+    // the host state first: the unpack kernel's ring rows follow the restored tick
+    s->tick = in.tick; s->env_steps = in.env_steps; s->seed = in.seed; s->cur = in.curriculum;
+    s->cur_attached = in.curriculum_attached != 0;
+    if (s->cur_attached) { s->sched = in.schedule; s->cur_increment = in.curriculum_increment; }
+    char* base = (char*)dev_in;
+    if (snapshot_kernels(s, in, base, false, st)) return 1;
+    CK(cudaMemcpyAsync(s->stats, base + in.section_offset[HLYNR_SNAP_STATS], sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
+                       cudaMemcpyDeviceToDevice, st));
+    if (s->cur_attached)
+        CK(cudaMemcpyAsync(s->cur_block, base + in.section_offset[HLYNR_SNAP_CURRICULUM], sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+}  // extern "C"
+
+extern "C" {
 
 // ---- host-buffer entry points ----------------------------------------------------------------
 static int make_pool(hlynr_sim* s) {

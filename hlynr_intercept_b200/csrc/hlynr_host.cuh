@@ -14,6 +14,15 @@ inline constexpr int (&fail)(const char*, ...) = hlynr_internal_fail;
         if (_e != cudaSuccess) return fail("%s: %s failed: %s (%s:%d)", __func__, #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
     } while (0)
 
+// Fails (`who` names the entry point) if `st` is capturing a CUDA graph: for the calls that must not be recorded into one.
+inline int refuse_capture(cudaStream_t st, const char* who) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    const cudaError_t e = cudaStreamIsCapturing(st, &cs);
+    if (e != cudaSuccess) return fail("%s: cudaStreamIsCapturing failed: %s", who, cudaGetErrorString(e));
+    if (cs != cudaStreamCaptureStatusNone) return fail("%s: refused while the stream is capturing a CUDA graph", who);
+    return 0;
+}
+
 // Makes `dev` the current device for the scope and restores the caller's device on exit; ok is false if it could not be selected.
 struct DeviceGuard {
     int prev = -1;

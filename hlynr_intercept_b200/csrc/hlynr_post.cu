@@ -584,6 +584,91 @@ int hlynr_post_set_stats(hlynr_post_t* p, const double* mean, const double* var,
     return 0;
 }
 
+static_assert(sizeof(HlynrPostSnapshotInfo) == 104, "HlynrPostSnapshotInfo is mirrored by abi.HlynrPostSnapshotInfo");
+size_t hlynr_post_snapshot_info_size(void) { return sizeof(HlynrPostSnapshotInfo); }
+
+static void post_snapshot_describe(const hlynr_post* p, HlynrPostSnapshotInfo* info) {
+    memset(info, 0, sizeof(*info));
+    info->format_version = HLYNR_POST_SNAPSHOT_VERSION;
+    info->frame_dim = p->fw; info->n_stack = p->k; info->sums_valid = p->sums_valid ? 1 : 0;
+    info->n_envs = p->n; info->t = p->t;
+    info->clip_obs = p->clip; info->epsilon = p->eps; info->gamma = p->gamma;
+    info->stats_bytes = sizeof(PostStats);
+    const size_t n = (size_t)p->n;
+    const size_t bytes[HLYNR_POST_SNAP_SECTIONS] = {sizeof(float) * n * p->fw * p->k, n, sizeof(double) * n, sizeof(PostStats)};
+    size_t off = 0;
+    for (int j = 0; j < HLYNR_POST_SNAP_SECTIONS; ++j) { info->section_offset[j] = off; off += (bytes[j] + 255) & ~size_t(255); }
+    info->device_bytes = off;
+}
+// Copies the frame ring between the handle (slot t % k is written next) and the image (oldest frame first), in either direction.
+static int post_snapshot_copy(hlynr_post* p, const HlynrPostSnapshotInfo& info, char* base, bool save, cudaStream_t st) {
+    const size_t slot = sizeof(float) * (size_t)p->n * p->fw;
+    const int newest = (int)((p->t - 1) % (uint32_t)p->k);
+    for (int j = 0; j < p->k; ++j) {
+        float* ring = p->frames + (int64_t)((newest - (p->k - 1 - j) + p->k) % p->k) * p->plane;
+        char* img = base + info.section_offset[HLYNR_POST_SNAP_FRAMES] + (size_t)j * slot;
+        CK(cudaMemcpyAsync(save ? (void*)img : (void*)ring, save ? (const void*)ring : (const void*)img, slot, cudaMemcpyDeviceToDevice, st));
+    }
+    uint8_t* age = p->age[p->age_cur];
+    char* img_age = base + info.section_offset[HLYNR_POST_SNAP_AGE];
+    char* img_ret = base + info.section_offset[HLYNR_POST_SNAP_RETURNS];
+    char* img_st = base + info.section_offset[HLYNR_POST_SNAP_STATS];
+    if (save) {
+        CK(cudaMemcpyAsync(img_age, age, (size_t)p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(img_ret, p->returns, sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(img_st, p->st, sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
+    } else {
+        CK(cudaMemcpyAsync(age, img_age, (size_t)p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(p->returns, img_ret, sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(p->st, img_st, sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
+    }
+    return 0;
+}
+
+int hlynr_post_snapshot_layout(const hlynr_post_t* p, HlynrPostSnapshotInfo* info, size_t* device_bytes) {
+    if (!p || !info || !device_bytes) return fail("hlynr_post_snapshot_layout: null argument");
+    post_snapshot_describe(p, info);
+    *device_bytes = (size_t)info->device_bytes;
+    return 0;
+}
+
+int hlynr_post_snapshot_save(hlynr_post_t* p, void* dev_out, HlynrPostSnapshotInfo* info, void* stream) {
+    if (!p || !dev_out || !info) return fail("hlynr_post_snapshot_save: null argument");
+    DeviceGuard g(p->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (refuse_capture(st, "hlynr_post_snapshot_save")) return 1;
+    post_snapshot_describe(p, info);
+    return post_snapshot_copy(p, *info, (char*)dev_out, true, st);
+}
+
+int hlynr_post_snapshot_load(hlynr_post_t* p, const HlynrPostSnapshotInfo* info, const void* dev_in, void* stream) {
+    if (!p || !info || !dev_in) return fail("hlynr_post_snapshot_load: null argument");
+    HlynrPostSnapshotInfo mine;
+    post_snapshot_describe(p, &mine);
+    const HlynrPostSnapshotInfo& in = *info;
+#define HLYNR_POST_REFUSE(cond, what, ...) \
+    if (cond) return fail("hlynr_post_snapshot_load: the snapshot's " what " differs from the pipeline's: " __VA_ARGS__)
+    HLYNR_POST_REFUSE(in.format_version != mine.format_version, "format version", "%d, expected %d", in.format_version, mine.format_version);
+    HLYNR_POST_REFUSE(in.n_envs != mine.n_envs, "n_envs", "%lld, the pipeline has %lld", (long long)in.n_envs, (long long)mine.n_envs);
+    HLYNR_POST_REFUSE(in.frame_dim != mine.frame_dim, "frame width", "%d, the pipeline has %d", in.frame_dim, mine.frame_dim);
+    HLYNR_POST_REFUSE(in.n_stack != mine.n_stack, "n_stack", "%d, the pipeline has %d", in.n_stack, mine.n_stack);
+    HLYNR_POST_REFUSE(memcmp(&in.clip_obs, &mine.clip_obs, sizeof(double)) != 0, "clip_obs", "%g, the pipeline has %g", in.clip_obs, mine.clip_obs);
+    HLYNR_POST_REFUSE(memcmp(&in.epsilon, &mine.epsilon, sizeof(double)) != 0, "epsilon", "%g, the pipeline has %g", in.epsilon, mine.epsilon);
+    HLYNR_POST_REFUSE(memcmp(&in.gamma, &mine.gamma, sizeof(double)) != 0, "gamma", "%g, the pipeline has %g", in.gamma, mine.gamma);
+    HLYNR_POST_REFUSE(in.stats_bytes != mine.stats_bytes, "statistics block", "%llu bytes, expected %llu", (unsigned long long)in.stats_bytes,
+                      (unsigned long long)mine.stats_bytes);
+    for (int j = 0; j < HLYNR_POST_SNAP_SECTIONS; ++j)
+        HLYNR_POST_REFUSE(in.section_offset[j] != mine.section_offset[j], "image layout", "offset of section %d", j);
+    HLYNR_POST_REFUSE(in.device_bytes != mine.device_bytes, "image size", "%llu bytes, expected %llu", (unsigned long long)in.device_bytes,
+                      (unsigned long long)mine.device_bytes);
+#undef HLYNR_POST_REFUSE
+    DeviceGuard g(p->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (refuse_capture(st, "hlynr_post_snapshot_load")) return 1;
+    p->t = (uint32_t)in.t; p->sums_valid = in.sums_valid != 0;   // the ring slots follow the restored t
+    return post_snapshot_copy(p, in, (char*)dev_in, false, st);
+}
+
 int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, void* stream) {
     if (!p || !max_abs_diff) return fail("hlynr_post_check_sums: null argument");
     if (p->t == 0) return fail("hlynr_post_check_sums: no observation yet");

@@ -120,6 +120,15 @@ class FusedActorCritic:
     def calls(self, value):
         _lib.check(self.L.hlynr_policy_set_counter(self.h, int(value), self._stream()))
 
+    def state_dict(self):
+        """The noise counter and seed, what a resumed run needs to draw the same noise; the weights and the optimiser stay with
+        torch's own state_dict.  Synchronises the current stream."""
+        return {"calls": self.calls, "seed": self.seed}
+
+    def load_state_dict(self, state):
+        self.calls = int(state["calls"])
+        self.seed = int(state["seed"])
+
     def _modules(self):
         net = self.net
         seq = net.network if hasattr(net, "network") else net.features_extractor.network

@@ -211,6 +211,27 @@ class HlynrObsPipeline:
             raise ValueError("clip_obs / epsilon of the pickle differ from this pipeline's")
         self.set_stats(d["mean"], d["var"], d["count"], d["ret_mean"], d["ret_var"], d["ret_count"])
 
+    # ---- snapshots (include/hlynr_post.h hlynr_post_snapshot_*, DESIGN.md section 17) ----
+    def state_dict(self):
+        """{'info': descriptor dict, 'image': uint8 CPU tensor, 'training': the training flag}: the frame ring, the per-env ages
+        and discounted returns, obs_rms / ret_rms and the running column sums.  Synchronises the current stream."""
+        from .sim import image_to_host
+
+        info, nbytes = abi.HlynrPostSnapshotInfo(), C.c_size_t()
+        _lib.check(self.L.hlynr_post_snapshot_layout(self.h, C.byref(info), C.byref(nbytes)))
+        dev = self._torch.empty(nbytes.value, dtype=self._torch.uint8, device=self.sim.device)
+        _lib.check(self.L.hlynr_post_snapshot_save(self.h, C.c_void_p(dev.data_ptr()), C.byref(info), self._stream()))
+        return {"info": abi.struct_to_dict(info), "image": image_to_host(self._torch, dev), "training": self.training}
+
+    def load_state_dict(self, state):
+        """Restores a state_dict() into a pipeline of the same n_envs, frame width, n_stack, clip_obs, epsilon and gamma."""
+        from .sim import image_to_device
+
+        info = abi.struct_from_dict(abi.HlynrPostSnapshotInfo, state["info"])
+        dev = image_to_device(self._torch, state["image"], info.device_bytes, self.sim.device)
+        _lib.check(self.L.hlynr_post_snapshot_load(self.h, C.byref(info), C.c_void_p(dev.data_ptr()), self._stream()))
+        self.training = bool(state["training"])
+
     def check_sums(self, resync=False):
         d = C.c_double()
         _lib.check(self.L.hlynr_post_check_sums(self.h, int(resync), C.byref(d), self._stream()))

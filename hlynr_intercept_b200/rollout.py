@@ -148,6 +148,24 @@ class DeviceRolloutCollector:
                                    f"gamma * V(terminal_observation): create the collector with bootstrap_rows=None (all envs)")
         return self
 
+    # ---- checkpoints ------------------------------------------------------------------------------------------------------
+    def state_dict(self):
+        """What the next collect() continues from: obs[T] (its first row), last_dones, whether reset() has run, and the
+        bootstrap overflow count, as CPU tensors.  The sim, the pipeline and the policy keep their own state_dict()."""
+        return {"next_obs": self.obs[self.T].cpu(), "last_dones": self.last_dones.cpu(), "started": self._started,
+                "overflow": self.overflow.cpu()}
+
+    def load_state_dict(self, state):
+        """Restores a state_dict() into a collector of the same n_envs and observation width.  A graph captured before the load
+        is dropped: capture() again (its warm-up collect is then the first rollout after the resume)."""
+        for name, dst in (("next_obs", self.obs[self.T]), ("last_dones", self.last_dones), ("overflow", self.overflow)):
+            src = _torch().as_tensor(state[name])
+            if tuple(src.shape) != tuple(dst.shape) or src.dtype != dst.dtype:
+                raise ValueError(f"collector state {name!r} is {src.dtype} {tuple(src.shape)}, this collector needs {dst.dtype} {tuple(dst.shape)}")
+            dst.copy_(src)
+        self._started = bool(state["started"])
+        self._graph = None
+
     # ---- CUDA graph: the whole collect() (T x ~20 launches) as one graph launch --------------------------------------
     def graph_period(self):
         """collect() can be captured once and replayed iff n_steps is a multiple of this (see graph_period())."""
@@ -168,7 +186,7 @@ class DeviceRolloutCollector:
     def replay(self):
         """One collect() as a single graph launch."""
         if self._graph is None:
-            raise RuntimeError("capture() first")
+            raise RuntimeError("capture() first (after load_state_dict() too)")
         self._graph.replay()
         return self
 

@@ -200,6 +200,32 @@ class HlynrSim:
             arr[k] = state[k]
         _lib.check(self.L.hlynr_import_state(self.h, first, count, arr.ctypes.data_as(C.c_void_p)))
 
+    # ---- snapshots (include/hlynr.h hlynr_snapshot_*, DESIGN.md section 17) ------------------------------------------------
+    def state_dict(self):
+        """The whole shard's state: {'info': the descriptor as a dict, 'image': its canonical device image as a uint8 CPU tensor,
+        'training_step_count': the host curriculum's count}.  Every env (episodes in flight, delay rings, Kalman tracks,
+        domain-randomised draws), the statistics block, the tick, the seed, the curriculum and an attached schedule with its device
+        count.  Synchronises the current stream."""
+        info, nbytes = abi.HlynrSnapshotInfo(), C.c_size_t()
+        _lib.check(self.L.hlynr_snapshot_layout(self.h, C.byref(info), C.byref(nbytes)))
+        dev = self._torch.empty(nbytes.value, dtype=self._torch.uint8, device=self.device)
+        _lib.check(self.L.hlynr_snapshot_save(self.h, C.c_void_p(dev.data_ptr()), C.byref(info), self._stream()))
+        return {"info": abi.struct_to_dict(info), "image": image_to_host(self._torch, dev),
+                "training_step_count": self.curriculum.training_step_count}
+
+    def load_state_dict(self, state):
+        """Restores a state_dict() into this sim, which must have been created with the same configuration, precision, n_envs,
+        env_id_offset and obs_dim (refused otherwise, naming the first difference).  Options are kept.  A StepGraph or collector
+        graph captured before the load must be captured again."""
+        info = abi.struct_from_dict(abi.HlynrSnapshotInfo, state["info"])
+        dev = image_to_device(self._torch, state["image"], info.device_bytes, self.device)
+        _lib.check(self.L.hlynr_snapshot_load(self.h, C.byref(info), C.c_void_p(dev.data_ptr()), self._stream()))
+        self.seed_value = int(info.seed)
+        self.curriculum.set_training_step_count(state["training_step_count"])
+        self.tracking = bool(info.curriculum_attached)
+        if self.tracking:
+            self.increment = int(info.curriculum_increment)
+
     def debug_draws(self, env_global_id, episode, step, block):
         raw, uni, nrm = np.zeros(4, np.uint32), np.zeros(4, np.float32), np.zeros(4, np.float32)
         _lib.check(self.L.hlynr_debug_draws(self.h, env_global_id, episode, step, block, raw.ctypes.data_as(C.c_void_p),
@@ -271,6 +297,24 @@ class StepGraph:
         self.graph.replay()
         _lib.check(self.sim.L.hlynr_note_replayed_ticks(self.sim.h, self.T, self.launches))
         return self.out
+
+
+def image_to_host(torch, dev):
+    """A snapshot's device image as a CPU tensor, copied through pinned memory (synchronises the current stream)."""
+    host = torch.empty(dev.numel(), dtype=torch.uint8, pin_memory=True)
+    host.copy_(dev, non_blocking=True)
+    torch.cuda.current_stream(dev.device).synchronize()
+    return host
+
+
+def image_to_device(torch, image, nbytes, device):
+    """A snapshot's image (CPU tensor or numpy array of bytes) on the device, through pinned memory, ordered on the current stream."""
+    image = torch.as_tensor(image).reshape(-1).view(torch.uint8)
+    if image.numel() != nbytes:
+        raise ValueError(f"the snapshot image has {image.numel()} bytes, its descriptor says {nbytes}")
+    host = torch.empty(image.numel(), dtype=torch.uint8, pin_memory=True)
+    host.copy_(image)
+    return host.to(device, non_blocking=True)
 
 
 def _tensor_from_ptr(torch, ptr, shape, dtype, device):

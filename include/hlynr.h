@@ -395,6 +395,69 @@ int hlynr_tick_count(const hlynr_t* sim, int64_t* out);
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int hlynr_launch_count(const hlynr_t* sim, int64_t* out);
 
+/*
+ * Snapshots: checkpoint and resume a run bit for bit.  A snapshot is a descriptor (HlynrSnapshotInfo, host) plus one device
+ * image in a CANONICAL layout that does not depend on the handle's plane layout (compact or wide), on the tick phase of the delay
+ * rings or on the ring-row convention, so a checkpoint stays readable when the internal layout changes.  The image holds, each
+ * section starting at section_offset[] (256-byte aligned):
+ *   HLYNR_SNAP_REAL       R[HLYNR_SNAP_REAL_COLS + 7 K][n_envs], R = the handle's precision: per env, in this order, ipos[3], fuel,
+ *                         ivel[3], fuel_used, mpos[3], prev_d, mvel[3], last_d, kf_x[0:3], min_d, kf_x[3:6], episode_return,
+ *                         thrust[3], T0, quat[4], wind[3], kf_P pp, kf_P pv, vp, vv, base_cd, peak; then per volley missile m < K
+ *                         vpos[3], vmin, vvel[3]
+ *   HLYNR_SNAP_INT        int32[HLYNR_SNAP_INT_COLS + K][n_envs]: steps, worsen_count, episode, crossed, kf_init, kf_f64,
+ *                         onboard_delay, vcur, vcount; then vactive[m] per volley missile
+ *   HLYNR_SNAP_ONBOARD    R[onboard_ring_len][4][n_envs]: onboard delay ring in AGE order, row j = the sample written j ticks
+ *                         before the snapshot (relative position xyz, detected)
+ *   HLYNR_SNAP_GROUND     R[ground_ring_len][8][n_envs]: ground delay ring in age order (relative position xyz, quality,
+ *                         relative velocity xyz, detection flag)
+ *   HLYNR_SNAP_STATS      double[HLYNR_STAT_SLOTS + 1][HLYNR_STATS_WORDS]: the statistics block, raw (hlynr_get_stats after a load
+ *                         returns the same bits)
+ *   HLYNR_SNAP_CURRICULUM uint64: the attached schedule's training-step count (0 when none is attached)
+ * Options ("pdl", "specialise", "prefetch_waves", ...) and the attached done list are not part of a snapshot: they do not change
+ * results, and the done list belongs to the caller.  A CUDA graph captured before a load bakes in the host counters of its
+ * capture: re-capture after loading.
+ */
+#define HLYNR_SNAPSHOT_VERSION 1
+#define HLYNR_SNAP_REAL_COLS 41
+#define HLYNR_SNAP_INT_COLS 9
+#define HLYNR_STAT_ROWS 65   /* per-block slots + the reduced row */
+enum { HLYNR_SNAP_REAL = 0, HLYNR_SNAP_INT = 1, HLYNR_SNAP_ONBOARD = 2, HLYNR_SNAP_GROUND = 3, HLYNR_SNAP_STATS = 4,
+       HLYNR_SNAP_CURRICULUM = 5, HLYNR_SNAP_SECTIONS = 6 };
+
+typedef struct HlynrSnapshotInfo {
+    int32_t format_version;       /* HLYNR_SNAPSHOT_VERSION */
+    int32_t abi_version;          /* HLYNR_ABI_VERSION */
+    int32_t precision;            /* HLYNR_FP32 / HLYNR_FP64 */
+    int32_t obs_dim;              /* option "obs_dim" */
+    int64_t n_envs, env_id_offset;
+    uint64_t seed;
+    int32_t volley_k;             /* params.volley_size */
+    int32_t onboard_ring_len, ground_ring_len;   /* rows of the delay rings (0 = no ring) */
+    int32_t curriculum_attached;  /* a schedule was attached (hlynr_attach_curriculum) */
+    uint64_t tick;                /* hlynr_tick_count */
+    double env_steps;             /* ticks x envs since the statistics were last zeroed (word 12 of hlynr_get_stats) */
+    int64_t curriculum_increment; /* of the attached schedule */
+    HlynrParams params;
+    HlynrCurriculum curriculum;          /* the host-pushed curriculum (hlynr_set_curriculum) */
+    HlynrCurriculumSchedule schedule;    /* valid when curriculum_attached */
+    uint64_t section_offset[HLYNR_SNAP_SECTIONS];   /* byte offset of each section of the device image */
+    uint64_t device_bytes;                          /* size of the device image */
+} HlynrSnapshotInfo;
+
+size_t hlynr_snapshot_info_size(void);
+/* Fills the descriptor of the handle's current state (format, shape, offsets) and the size of the device image. */
+int hlynr_snapshot_layout(const hlynr_t* sim, HlynrSnapshotInfo* info, size_t* device_bytes);
+/* Writes the device image to dev_out (device_bytes of hlynr_snapshot_layout) and fills `info`; ordered on `stream`, no host
+ * synchronisation.  The host counters in `info` are those of the work enqueued so far.  Refused while `stream` is capturing. */
+int hlynr_snapshot_save(hlynr_t* sim, void* dev_out, HlynrSnapshotInfo* info, void* stream);
+/* Restores a snapshot into a handle created with the same params, precision, n_envs, env_id_offset, obs_dim: the state of every
+ * env, the delay rings, the statistics block, the tick and env_steps counters, the seed, the host-pushed curriculum, and the
+ * curriculum schedule (re-attached with its count and increment, or detached, as it was).  Refuses, naming the first mismatch, a
+ * descriptor of another format version, precision, shape or configuration, and refuses while `stream` is capturing.  Ordered on
+ * `stream`; dev_in may be reused once the stream has passed the load.  A compact-layout snapshot loads into a wide-layout handle
+ * and the reverse. */
+int hlynr_snapshot_load(hlynr_t* sim, const HlynrSnapshotInfo* info, const void* dev_in, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

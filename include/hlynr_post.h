@@ -81,6 +81,39 @@ int hlynr_post_launch_count(const hlynr_post_t* post, int64_t* out);
  * multiple of n_stack; after each replay call hlynr_post_note_replayed_steps(post, T). */
 int hlynr_post_note_replayed_steps(hlynr_post_t* post, int64_t steps, int64_t launches);
 
+/*
+ * Snapshots (see hlynr_snapshot_save in hlynr.h): a descriptor plus one device image in a canonical layout that does not depend
+ * on the ring phase t % n_stack.  Sections, each 256-byte aligned:
+ *   HLYNR_POST_SNAP_FRAMES   float[n_stack][N][F]: the frame ring from the oldest frame to the newest
+ *   HLYNR_POST_SNAP_AGE      uint8[N]: how many older frames belong to each env's episode
+ *   HLYNR_POST_SNAP_RETURNS  double[N]: VecNormalize's discounted returns
+ *   HLYNR_POST_SNAP_STATS    the device statistics block, stats_bytes long: obs_rms, ret_rms and the per-lag column sums that
+ *                            later updates start from
+ */
+#define HLYNR_POST_SNAPSHOT_VERSION 1
+enum { HLYNR_POST_SNAP_FRAMES = 0, HLYNR_POST_SNAP_AGE = 1, HLYNR_POST_SNAP_RETURNS = 2, HLYNR_POST_SNAP_STATS = 3,
+       HLYNR_POST_SNAP_SECTIONS = 4 };
+
+typedef struct HlynrPostSnapshotInfo {
+    int32_t format_version;   /* HLYNR_POST_SNAPSHOT_VERSION */
+    int32_t frame_dim, n_stack;
+    int32_t sums_valid;       /* the per-lag column sums describe the ring (hlynr_post_step can train) */
+    int64_t n_envs;
+    uint64_t t;               /* frames written so far (every reset and step writes one) */
+    double clip_obs, epsilon, gamma;
+    uint64_t stats_bytes;
+    uint64_t section_offset[HLYNR_POST_SNAP_SECTIONS];
+    uint64_t device_bytes;
+} HlynrPostSnapshotInfo;
+
+size_t hlynr_post_snapshot_info_size(void);
+int hlynr_post_snapshot_layout(const hlynr_post_t* post, HlynrPostSnapshotInfo* info, size_t* device_bytes);
+/* Writes the image to dev_out and fills `info`; ordered on `stream`.  Refused while `stream` is capturing. */
+int hlynr_post_snapshot_save(hlynr_post_t* post, void* dev_out, HlynrPostSnapshotInfo* info, void* stream);
+/* Restores a snapshot into a pipeline created with the same n_envs, frame_dim, n_stack, clip_obs, epsilon and gamma (refuses
+ * another, naming the first mismatch, and a capturing stream).  Ordered on `stream`. */
+int hlynr_post_snapshot_load(hlynr_post_t* post, const HlynrPostSnapshotInfo* info, const void* dev_in, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
