@@ -103,7 +103,8 @@ __global__ void __launch_bounds__(256) returns_kernel(double* __restrict__ ret, 
     double s = 0.0, q = 0.0;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
         double r = ret[e];
-        if (training) { r = r * gamma + (double)rew[e]; s += r; q += r * r; }
+        // SB3's `returns * gamma + rewards` rounds twice: _rn keeps nvcc from contracting it into one DFMA
+        if (training) { r = __dadd_rn(__dmul_rn(r, gamma), (double)rew[e]); s += r; q += r * r; }
         const bool done = (term[e] | trunc[e]) != 0;
         ret[e] = done ? 0.0 : r;  // returns[dones] = 0 happens whether or not the statistics move
         const int a = (int)age_in[e] + 1;
@@ -156,6 +157,15 @@ __global__ void __launch_bounds__(512) done_corr_kernel(const HlynrDoneRecord* _
 }
 
 // ---- shift the per-lag sums, merge the batch moments into obs_rms / ret_rms (RunningMeanStd.update_from_moments) ----
+// The merge rounds every product and sum on its own in numpy's order (_rn: no contraction into DFMA), so batch moments that
+// are exact (e.g. dyadic frames) give obs_rms bit for bit as numpy does.
+__device__ __forceinline__ void rms_merge(double& mean, double& var, double count, double bm, double bv, double n) {
+    const double delta = bm - mean, tot = count + n;
+    const double m2 = __dadd_rn(__dadd_rn(__dmul_rn(var, count), __dmul_rn(bv, n)), __dmul_rn(__dmul_rn(__dmul_rn(delta, delta), count), n) / tot);
+    mean = __dadd_rn(mean, __dmul_rn(delta, n) / tot);
+    var = m2 / tot;
+}
+
 template <int F>
 __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int training, int reset_all, int with_returns, double eps) {
     const int f = threadIdx.x, D = k * F;
@@ -175,12 +185,9 @@ __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int trai
         if (training) {
             const int j = f / F, c = f % F, d = k - 1 - j;
             const double bm = st->S[d][c] / n;
-            double bv = st->Q[d][c] / n - bm * bm;
+            double bv = __dsub_rn(st->Q[d][c] / n, __dmul_rn(bm, bm));
             if (bv < 0.0) bv = 0.0;
-            const double delta = bm - st->mean[f], tot = count + n;
-            const double m2 = st->var[f] * count + bv * n + delta * delta * count * n / tot;
-            st->mean[f] = st->mean[f] + delta * n / tot;
-            st->var[f] = m2 / tot;
+            rms_merge(st->mean[f], st->var[f], count, bm, bv, n);
         }
         st->inv_std[f] = 1.0 / sqrt(st->var[f] + eps);
     }
@@ -189,13 +196,10 @@ __global__ void merge_kernel(PostStats* st, int k, double n, int shift, int trai
         st->count = count + n;
         if (with_returns) {
             const double bm = st->ret_sum / n;
-            double bv = st->ret_sq / n - bm * bm;
+            double bv = __dsub_rn(st->ret_sq / n, __dmul_rn(bm, bm));
             if (bv < 0.0) bv = 0.0;
-            const double c0 = st->ret_count, delta = bm - st->ret_mean, tot = c0 + n;
-            const double m2 = st->ret_var * c0 + bv * n + delta * delta * c0 * n / tot;
-            st->ret_mean = st->ret_mean + delta * n / tot;
-            st->ret_var = m2 / tot;
-            st->ret_count = tot;
+            rms_merge(st->ret_mean, st->ret_var, st->ret_count, bm, bv, n);
+            st->ret_count = st->ret_count + n;
         }
         st->ret_sum = 0.0; st->ret_sq = 0.0;
     }
@@ -212,7 +216,8 @@ __global__ void __launch_bounds__(512) normalize_kernel(const float* __restrict_
     const int r = t / P, p = t % P, f = 2 * p, j = f / OD, c = f % OD, lag = k - 1 - j;
     // SB3 evaluates (obs_f32 - mean_f64) / sqrt(var + eps) in float64 and rounds the result to float32.  Here the mean is
     // split into a float pair (hi + lo), so the cancellation obs - mean keeps ~48 bits; the product and the clip are float:
-    // the result is within 2 float ulps of SB3's, without touching the FP64 pipe.
+    // the result is within 3 float ulps of SB3's, without touching the FP64 pipe (3, not 2: obs - m_hi rounds in the operands'
+    // binade, and the result can land one binade lower, where that rounding error is 2 ulps).
     const float m0h = (float)st->mean[f], m0l = (float)(st->mean[f] - (double)m0h), i0 = (float)st->inv_std[f];
     const float m1h = (float)st->mean[f + 1], m1l = (float)(st->mean[f + 1] - (double)m1h), i1 = (float)st->inv_std[f + 1];
     const float* src = frames + (int64_t)ring_slot(newest, lag, k) * plane + c;

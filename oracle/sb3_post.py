@@ -93,20 +93,25 @@ class VecNormalize:
             self.obs_rms.update(obs)
         return self.normalize_obs(obs)
 
-    def step(self, obs, rewards, dones, infos):
+    def update(self, obs, rewards, dones):
+        """The statistics half of step: obs_rms, the discounted returns and ret_rms, returns[dones] = 0.  Nothing in step
+        reads returns between SB3's update and its reset of the finished envs' returns, so the two can sit together here."""
         self.old_obs = obs
         if self.training and self.norm_obs:
             self.obs_rms.update(obs)
-        obs = self.normalize_obs(obs)
         if self.training:
             self.returns = self.returns * self.gamma + rewards
             self.ret_rms.update(self.returns)
+        self.returns[dones.astype(bool)] = 0
+
+    def step(self, obs, rewards, dones, infos):
+        self.update(obs, rewards, dones)
+        obs = self.normalize_obs(obs)
         rewards = self.normalize_reward(rewards)
         for idx in np.nonzero(dones)[0]:
             info = infos.get(int(idx))
             if info is not None and "terminal_observation" in info:
                 info["terminal_observation"] = self.normalize_obs(info["terminal_observation"])
-        self.returns[dones.astype(bool)] = 0
         return obs, rewards, dones, infos
 
 
