@@ -63,16 +63,7 @@ class HlynrCurriculumSchedule(C.Structure):
         (f"{ramp}_{k}", C.c_double) for ramp in ("beam", "onboard", "ground") for k in ("initial", "final", "start", "end")]
 
 
-class HlynrInfoSoA(C.Structure):
-    _fields_ = [("distance", C.c_void_p), ("min_distance", C.c_void_p), ("fuel_remaining", C.c_void_p),
-                ("fuel_used", C.c_void_p), ("steps", C.c_void_p), ("flags", C.c_void_p),
-                ("interceptor_pos", C.c_void_p), ("missile_pos", C.c_void_p),
-                ("episode_return", C.c_void_p), ("episode_length", C.c_void_p),
-                ("missiles_intercepted", C.c_void_p), ("missiles_remaining", C.c_void_p), ("missile_min_distances", C.c_void_p),
-                ("radar_quality", C.c_void_p)]
-
-
-INFO_FIELDS = [  # name, numpy dtype, trailing shape
+INFO_FIELDS = [  # name, numpy dtype, trailing shape: the fields of HlynrInfoSoA, in order
     ("distance", "float32", ()), ("min_distance", "float32", ()), ("fuel_remaining", "float32", ()),
     ("fuel_used", "float32", ()), ("steps", "int32", ()), ("flags", "uint8", ()),
     ("interceptor_pos", "float32", (3,)), ("missile_pos", "float32", (3,)),
@@ -80,6 +71,10 @@ INFO_FIELDS = [  # name, numpy dtype, trailing shape
     ("missiles_intercepted", "int32", ()), ("missiles_remaining", "int32", ()), ("missile_min_distances", "float32", (MAX_VOLLEY,)),
     ("radar_quality", "float32", ()),
 ]
+
+
+class HlynrInfoSoA(C.Structure):   # one device or host pointer per field
+    _fields_ = [(name, C.c_void_p) for name, _, _ in INFO_FIELDS]
 
 INFO_INTERCEPTED, INFO_HIT_TARGET, INFO_CLAMPED, INFO_RADAR_DETECTED = 0x01, 0x02, 0x04, 0x08
 INFO_GROUND_DETECTED, INFO_CROSSED, INFO_FUZE, INFO_KF_INIT = 0x10, 0x20, 0x40, 0x80

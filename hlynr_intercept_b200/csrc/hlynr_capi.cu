@@ -150,22 +150,42 @@ class CopyPool {
 #define HLYNR_HOST_STREAMS 3
 #define HLYNR_DONE_PREFIX 4096  // records fetched together with the count; the rest (rare) in a second copy
 
+// The fields of HlynrInfoSoA (include/hlynr.h): X(name, element type, elements per env).
+#define HLYNR_INFO_FIELDS(X)                                                                                                       \
+    X(distance, float, 1) X(min_distance, float, 1) X(fuel_remaining, float, 1) X(fuel_used, float, 1) X(steps, int32_t, 1)        \
+    X(flags, uint8_t, 1) X(interceptor_pos, float, 3) X(missile_pos, float, 3) X(episode_return, float, 1)                          \
+    X(episode_length, int32_t, 1) X(missiles_intercepted, int32_t, 1) X(missiles_remaining, int32_t, 1)                             \
+    X(missile_min_distances, float, HLYNR_MAX_VOLLEY) X(radar_quality, float, 1)
+#define X(name, type, per_env) +1
+static_assert(sizeof(HlynrInfoSoA) == (0 HLYNR_INFO_FIELDS(X)) * sizeof(void*), "every field of HlynrInfoSoA is in HLYNR_INFO_FIELDS");
+#undef X
+
 struct HostIO {  // pinned host + device staging for the *_host entry points
-    float *h_actions = nullptr, *h_obs = nullptr, *h_reward = nullptr;
-    uint8_t *h_term = nullptr, *h_trunc = nullptr, *h_mask = nullptr;
-    float *d_actions = nullptr, *d_obs = nullptr;
-    uint8_t* d_mask = nullptr;
-    HlynrInfoSoA d_info;
-    HlynrDoneRecord *d_records = nullptr, *h_records = nullptr;  // capacity n; h_records = h_records_ab[call parity]
-    HlynrDoneRecord* h_records_ab[2] = {nullptr, nullptr};       // two host buffers: the records of a call survive the next call
-    uint8_t* h_done = nullptr;                                   // terminated | truncated, written by the kernel
+    PinnedPtr<float> h_actions, h_obs, h_reward;
+    PinnedPtr<uint8_t> h_term, h_trunc, h_mask;
+    DevPtr<float> d_actions, d_obs;
+    DevPtr<uint8_t> d_mask;
+#define X(name, type, per_env) DevPtr<type> info_##name;
+    HLYNR_INFO_FIELDS(X)
+#undef X
+    HlynrInfoSoA d_info{};   // the info_* arrays
+    DevPtr<HlynrDoneRecord> d_records;                // capacity n
+    PinnedPtr<HlynrDoneRecord> h_records_ab[2];       // two host buffers: the records of a call survive the next call
+    HlynrDoneRecord* h_records = nullptr;             // not owned: h_records_ab[call parity]
+    PinnedPtr<uint8_t> h_done;                        // terminated | truncated, written by the kernel
     uint32_t calls = 0;
-    int32_t *d_counter = nullptr, *h_count = nullptr;
+    DevPtr<int32_t> d_counter;
+    PinnedPtr<int32_t> h_count;
     int32_t last_count = 0;
-    cudaStream_t streams[HLYNR_HOST_STREAMS] = {nullptr, nullptr, nullptr};
-    cudaEvent_t ev_start = nullptr, ev_done[HLYNR_HOST_STREAMS] = {nullptr, nullptr, nullptr};
-    CopyPool* pool = nullptr;
+    StreamOwner streams[HLYNR_HOST_STREAMS];
+    EventOwner ev_start, ev_done[HLYNR_HOST_STREAMS];
+    std::unique_ptr<CopyPool> pool;
     bool ready = false, info_ready = false;
+};
+
+template <typename R> struct CurBlock {
+    unsigned long long num_timesteps;
+    KCurriculum<R> slot;
 };
 
 struct hlynr_sim {
@@ -179,14 +199,12 @@ struct hlynr_sim {
     double env_steps = 0.0;
     int specialise = 1;      // use the feature-specialised instantiations when the configuration matches one
     int sm_count = 148;  // ticks simulated since the statistics were last zeroed (n per launch tick)
-    void* state_mem = nullptr;
-    size_t state_bytes = 0;
+    DevPtr<char> state_mem;
     StatePlanes<float> pf;
     StatePlanes<double> pd;
-    double* stats = nullptr;        // [HLYNR_STAT_SLOTS + 1][HLYNR_STATS_WORDS]; last row = reduced block
-    HlynrEnvState* xchg = nullptr;  // device staging for export/import
+    DevPtr<double> stats;          // [HLYNR_STAT_SLOTS + 1][HLYNR_STATS_WORDS]; last row = reduced block
+    DevPtr<HlynrEnvState> xchg;    // device staging for export/import
     int64_t xchg_cap = 0;
-    cudaStream_t own_stream = nullptr;
     HostIO hio;
     int host_info = 1, host_chunks = 0, host_threads = 0;
     int host_chunk_growth = 12;   // geometric chunk schedule of the host path, x1.5 per chunk (measured best on B200: 2.43 -> 2.35 ms at 2^20 envs, 26-D)
@@ -194,13 +212,13 @@ struct hlynr_sim {
     int pdl = 1;   // step kernels are launched with programmatic stream serialization (option "pdl"; -1.5 us per launch on B200)
     int obs_dim = HLYNR_OBS_DIM;  // row pitch of every observation array of the API: 26, or 17 (option "obs_dim")
     int prefetch_waves = 1;  // CTAs per SM the step kernel looks ahead when it prefetches upcoming planes into L2 (0 = off)
-    HlynrDoneRecord* done_records = nullptr;  // attached compact done list (hlynr_set_done_list)
-    int32_t* done_counter = nullptr;
+    HlynrDoneRecord* done_records = nullptr;  // not owned: the caller's compact done list (hlynr_set_done_list)
+    int32_t* done_counter = nullptr;          // not owned: its counter
     int32_t done_cap = 0;
-    uint8_t* io_done = nullptr;   // set by hlynr_step_host for the duration of the call
-    uint8_t* host_done = nullptr; // caller's page-locked `dones` buffer (hlynr_host_done_buffer), NULL = the handle's own
-    // attached curriculum schedule (hlynr_attach_curriculum): a CurBlock<R> allocated on first attach and kept until hlynr_destroy
-    void* cur_block = nullptr;
+    uint8_t* io_done = nullptr;   // not owned: set by hlynr_step_host for the duration of the call
+    uint8_t* host_done = nullptr; // not owned: caller's page-locked `dones` buffer (hlynr_host_done_buffer), NULL = the handle's own
+    // attached curriculum schedule (hlynr_attach_curriculum): a CurBlock<R>, sized for R = double, allocated on first attach
+    DevPtr<CurBlock<double>> cur_block;
     bool cur_attached = false;
     HlynrCurriculumSchedule sched;
     int64_t cur_increment = 0;
@@ -317,10 +335,6 @@ template <typename R> __device__ KCurriculum<R> kcur_at(const HlynrCurriculumSch
     k.onboard_rel = (float)onb; k.ground_rel = (float)gnd;
     return k;
 }
-template <typename R> struct CurBlock {
-    unsigned long long num_timesteps;
-    KCurriculum<R> slot;
-};
 // Launched by hlynr_step before the step kernel (increment = the run's env count) and by hlynr_reset before the reset kernel
 // (increment 0), always WITHOUT programmatic serialization: it starts only once the previous kernel of the stream, which may be a
 // step kernel still reading the slot, has completed.  It lets the next launch be scheduled at once; that launch reads the slot
@@ -575,12 +589,12 @@ template <typename R> static KernelArgs<R> base_args(hlynr_sim* s, const StatePl
     A.env_offset = s->env_offset;
     A.rk = make_round_keys(s->seed);
     set_tick(A, s->tick);
-    A.io.stats = s->stats;
+    A.io.stats = s->stats.get();
     A.k_steps = 1;
     A.prefetch_ahead = s->sm_count * s->prefetch_waves * HLYNR_BLOCK;
     A.obs_dim = s->obs_dim;
     A.compact = s->compact;
-    A.cur_dev = s->cur_attached ? &((CurBlock<R>*)s->cur_block)->slot : nullptr;
+    A.cur_dev = s->cur_attached ? &((CurBlock<R>*)s->cur_block.get())->slot : nullptr;
     return A;
 }
 // Before a step (increment = the attached increment) or a reset (0): the slot the next launch reads, and the count advanced.
@@ -588,7 +602,7 @@ static int curriculum_tick(hlynr_sim* s, int64_t increment, cudaStream_t st) {
     if (!s->cur_attached) return 0;
     with_planes(s, [&](auto& planes) {
         using R = real_of<decltype(planes)>;
-        curriculum_tick_kernel<R><<<1, 1, 0, st>>>((CurBlock<R>*)s->cur_block, s->sched, (unsigned long long)increment);
+        curriculum_tick_kernel<R><<<1, 1, 0, st>>>((CurBlock<R>*)s->cur_block.get(), s->sched, (unsigned long long)increment);
     });
     CK(cudaGetLastError());
     s->launches += 1;
@@ -667,24 +681,6 @@ size_t hlynr_curriculum_schedule_size(void) { return sizeof(HlynrCurriculumSched
 void hlynr_destroy(hlynr_t* s) {
     if (!s) return;
     DeviceGuard g(s->device);
-    cudaFree(s->state_mem); cudaFree(s->stats); cudaFree(s->xchg); cudaFree(s->cur_block);
-    HostIO& h = s->hio;
-    delete h.pool;
-    cudaFreeHost(h.h_actions); cudaFreeHost(h.h_obs); cudaFreeHost(h.h_reward); cudaFreeHost(h.h_records_ab[0]); cudaFreeHost(h.h_records_ab[1]); cudaFreeHost(h.h_count);
-    cudaFreeHost(h.h_done);
-    cudaFreeHost(h.h_term); cudaFreeHost(h.h_trunc); cudaFreeHost(h.h_mask);
-    cudaFree(h.d_actions); cudaFree(h.d_obs); cudaFree(h.d_records); cudaFree(h.d_counter); cudaFree(h.d_mask);
-    for (int k = 0; k < HLYNR_HOST_STREAMS; ++k) {
-        if (h.streams[k]) cudaStreamDestroy(h.streams[k]);
-        if (h.ev_done[k]) cudaEventDestroy(h.ev_done[k]);
-    }
-    if (h.ev_start) cudaEventDestroy(h.ev_start);
-    cudaFree(h.d_info.distance); cudaFree(h.d_info.min_distance); cudaFree(h.d_info.fuel_remaining); cudaFree(h.d_info.fuel_used);
-    cudaFree(h.d_info.steps); cudaFree(h.d_info.flags); cudaFree(h.d_info.interceptor_pos); cudaFree(h.d_info.missile_pos);
-    cudaFree(h.d_info.episode_return); cudaFree(h.d_info.episode_length);
-    cudaFree(h.d_info.missiles_intercepted); cudaFree(h.d_info.missiles_remaining); cudaFree(h.d_info.missile_min_distances);
-    cudaFree(h.d_info.radar_quality);
-    if (s->own_stream) cudaStreamDestroy(s->own_stream);
     delete s;
 }
 
@@ -704,7 +700,7 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
     if (device < 0 || device >= ndev) return fail("hlynr_create: device %d not available (%d devices)", device, ndev);
     DeviceGuard g(device);
     if (!g.ok) return fail("hlynr_create: cannot select device %d", device);
-    hlynr_sim* s = new (std::nothrow) hlynr_sim();
+    std::unique_ptr<hlynr_sim> s(new (std::nothrow) hlynr_sim());
     if (!s) return fail("hlynr_create: out of host memory");
     s->params = *p;
     s->cur = HlynrCurriculum{200.0, 60.0, 1.0, 1.0};
@@ -712,19 +708,17 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
     s->device = device; s->precision = precision; s->seed = seed; s->env_offset = env_id_offset;
     KParams<float> kp = make_kparams<float>(*p);
     const int gl = kp.gnd_ring_len, ol = kp.onb_ring_len;
-    s->state_bytes = with_planes(s, [&](auto& planes) { return carve(planes, nullptr, s->n_pad, gl, ol, p->volley_size); });
-    cudaError_t e = cudaMalloc(&s->state_mem, s->state_bytes);
-    if (e != cudaSuccess) { int r = fail("hlynr_create: cudaMalloc(%zu bytes) failed: %s", s->state_bytes, cudaGetErrorString(e)); delete s; return r; }
-    e = cudaMalloc(&s->stats, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS);
-    if (e != cudaSuccess) { int r = fail("hlynr_create: cudaMalloc(stats) failed: %s", cudaGetErrorString(e)); cudaFree(s->state_mem); delete s; return r; }
-    cudaMemset(s->state_mem, 0, s->state_bytes);
-    cudaMemset(s->stats, 0, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS);
-    cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking);
-    cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device);
+    const size_t state_bytes = with_planes(s.get(), [&](auto& planes) { return carve(planes, nullptr, s->n_pad, gl, ol, p->volley_size); });
+    const cudaError_t e = alloc(s->state_mem, state_bytes);
+    if (e != cudaSuccess) return fail("hlynr_create: cudaMalloc(%zu bytes) failed: %s", state_bytes, cudaGetErrorString(e));
+    CK(alloc(s->stats, (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS));
+    CK(cudaMemset(s->state_mem.get(), 0, state_bytes));
+    CK(cudaMemset(s->stats.get(), 0, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS));
+    CK(cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device));
     const int blk = 256;
-    with_planes(s, [&](auto& planes) {
+    with_planes(s.get(), [&](auto& planes) {
         using R = real_of<decltype(planes)>;
-        carve(planes, (char*)s->state_mem, s->n_pad, gl, ol, p->volley_size);
+        carve(planes, s->state_mem.get(), s->n_pad, gl, ol, p->volley_size);
         // compact plane layout (fp32 build only; hlynr_device.cuh load_env): fixed for the life of the handle, whichever kernel
         // instantiation runs
         s->compact = 0;
@@ -732,10 +726,10 @@ int hlynr_create(const HlynrParams* p, int64_t n_envs, int device, uint64_t seed
             s->compact = feature_set(*p) == FT_V2ON ? 1 : (feature_set(*p) == FT_V2ON_DR ? 2 : 0);
         init_kernel<R><<<grid_for(s->n_pad, blk), blk>>>(planes, s->n_pad, (float)p->peak_mult, s->compact);
     });
-    e = cudaDeviceSynchronize();
-    if (e != cudaSuccess) { int r = fail("hlynr_create: init kernel failed: %s", cudaGetErrorString(e)); hlynr_destroy(s); return r; }
+    CK(cudaGetLastError());
+    CK(cudaDeviceSynchronize());
     s->launches += 1;
-    *out = s;
+    *out = s.release();
     return 0;
 }
 
@@ -864,10 +858,10 @@ int hlynr_attach_curriculum(hlynr_t* s, const HlynrCurriculumSchedule* c, uint64
     if (!s || !c) return fail("hlynr_attach_curriculum: null argument");
     if (check_schedule(c, increment, "hlynr_attach_curriculum")) return 1;
     DeviceGuard g(s->device);
-    if (!s->cur_block) CK(cudaMalloc(&s->cur_block, sizeof(CurBlock<double>)));
+    if (!s->cur_block) CK(alloc(s->cur_block, 1));
     CK(cudaDeviceSynchronize());   // no launch of an earlier attachment still reads or writes the block
     const unsigned long long v = num_timesteps;
-    CK(cudaMemcpy(s->cur_block, &v, sizeof(v), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s->cur_block.get(), &v, sizeof(v), cudaMemcpyHostToDevice));
     s->sched = *c; s->cur_increment = increment; s->cur_attached = true;
     return 0;
 }
@@ -880,7 +874,7 @@ int hlynr_set_timesteps(hlynr_t* s, uint64_t num_timesteps, void* stream) {
     if (!s) return fail("hlynr_set_timesteps: null handle");
     if (!s->cur_attached) return fail("hlynr_set_timesteps: no curriculum schedule is attached (hlynr_attach_curriculum)");
     DeviceGuard g(s->device);
-    set_timesteps_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((unsigned long long*)s->cur_block, (unsigned long long)num_timesteps);
+    set_timesteps_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((unsigned long long*)s->cur_block.get(), (unsigned long long)num_timesteps);
     CK(cudaGetLastError());
     s->launches += 1;
     return 0;
@@ -892,7 +886,7 @@ int hlynr_get_timesteps(hlynr_t* s, uint64_t* out, void* stream) {
     const cudaStream_t st = (cudaStream_t)stream;
     CK(cudaStreamSynchronize(st));
     unsigned long long v = 0;
-    CK(cudaMemcpyAsync(&v, s->cur_block, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&v, s->cur_block.get(), sizeof(v), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     *out = (uint64_t)v;
     return 0;
@@ -901,13 +895,11 @@ int hlynr_debug_curriculum_at(hlynr_t* s, uint64_t count, double out[4]) {
     if (!s || !out) return fail("hlynr_debug_curriculum_at: null argument");
     if (!s->cur_attached) return fail("hlynr_debug_curriculum_at: no curriculum schedule is attached (hlynr_attach_curriculum)");
     DeviceGuard g(s->device);
-    double* buf = nullptr;
-    CK(cudaMalloc(&buf, 4 * sizeof(double)));
-    with_planes(s, [&](auto& planes) { curriculum_probe_kernel<real_of<decltype(planes)>><<<1, 1>>>(s->sched, (unsigned long long)count, buf); });
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpy(out, buf, 4 * sizeof(double), cudaMemcpyDeviceToHost);
-    cudaFree(buf);
-    if (e != cudaSuccess) return fail("hlynr_debug_curriculum_at: %s", cudaGetErrorString(e));
+    DevPtr<double> buf;
+    CK(alloc(buf, 4));
+    with_planes(s, [&](auto& planes) { curriculum_probe_kernel<real_of<decltype(planes)>><<<1, 1>>>(s->sched, (unsigned long long)count, buf.get()); });
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(out, buf.get(), 4 * sizeof(double), cudaMemcpyDeviceToHost));
     s->launches += 1;
     return 0;
 }
@@ -944,7 +936,7 @@ int hlynr_rollout(hlynr_t* s, int k_steps, const float* actions_dev, float* obs_
 
 int hlynr_stats_device_ptr(hlynr_t* s, double** out) {
     if (!s || !out) return fail("null argument");
-    *out = s->stats + HLYNR_STAT_SLOTS * HLYNR_STATS_WORDS;
+    *out = s->stats.get() + HLYNR_STAT_SLOTS * HLYNR_STATS_WORDS;
     return 0;
 }
 
@@ -952,7 +944,7 @@ int hlynr_stats_device_ptr(hlynr_t* s, double** out) {
 int hlynr_stats_reduce(hlynr_t* s, void* stream) {
     if (!s) return fail("null handle");
     DeviceGuard g(s->device);
-    stats_reduce_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(s->stats, s->env_steps);
+    stats_reduce_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(s->stats.get(), s->env_steps);
     CK(cudaGetLastError());
     s->launches += 1;
     return 0;
@@ -963,10 +955,10 @@ int hlynr_get_stats(hlynr_t* s, HlynrStats* host_out, int zero_after, void* stre
     DeviceGuard g(s->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (hlynr_stats_reduce(s, stream)) return 1;
-    CK(cudaMemcpyAsync(host_out, s->stats + HLYNR_STAT_SLOTS * HLYNR_STATS_WORDS, sizeof(double) * HLYNR_STATS_WORDS,
+    CK(cudaMemcpyAsync(host_out, s->stats.get() + HLYNR_STAT_SLOTS * HLYNR_STATS_WORDS, sizeof(double) * HLYNR_STATS_WORDS,
                        cudaMemcpyDeviceToHost, st));
     if (zero_after) {
-        CK(cudaMemsetAsync(s->stats, 0, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS, st));
+        CK(cudaMemsetAsync(s->stats.get(), 0, sizeof(double) * (HLYNR_STAT_SLOTS + 1) * HLYNR_STATS_WORDS, st));
         s->env_steps = 0.0;
     }
     CK(cudaStreamSynchronize(st));
@@ -975,9 +967,8 @@ int hlynr_get_stats(hlynr_t* s, HlynrStats* host_out, int zero_after, void* stre
 
 static int ensure_xchg(hlynr_sim* s, int64_t count) {
     if (s->xchg_cap >= count) return 0;
-    cudaFree(s->xchg);
-    s->xchg = nullptr; s->xchg_cap = 0;
-    CK(cudaMalloc(&s->xchg, sizeof(HlynrEnvState) * count));
+    s->xchg_cap = 0;
+    CK(alloc(s->xchg, count));
     s->xchg_cap = count;
     return 0;
 }
@@ -990,10 +981,10 @@ int hlynr_export_state(hlynr_t* s, int64_t first, int64_t count, HlynrEnvState* 
     CK(cudaDeviceSynchronize());
     if (ensure_xchg(s, count)) return 1;
     with_planes(s, [&](auto& planes) {
-        export_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg);
+        export_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg.get());
     });
     CK(cudaGetLastError());
-    CK(cudaMemcpy(host_out, s->xchg, sizeof(HlynrEnvState) * count, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(host_out, s->xchg.get(), sizeof(HlynrEnvState) * count, cudaMemcpyDeviceToHost));
     s->launches += 1;
     return 0;
 }
@@ -1005,9 +996,9 @@ int hlynr_import_state(hlynr_t* s, int64_t first, int64_t count, const HlynrEnvS
     DeviceGuard g(s->device);
     CK(cudaDeviceSynchronize());
     if (ensure_xchg(s, count)) return 1;
-    CK(cudaMemcpy(s->xchg, host_in, sizeof(HlynrEnvState) * count, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s->xchg.get(), host_in, sizeof(HlynrEnvState) * count, cudaMemcpyHostToDevice));
     with_planes(s, [&](auto& planes) {
-        import_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg);
+        import_kernel<real_of<decltype(planes)>><<<grid_for(count, 128), 128>>>(base_args(s, planes), first, count, s->xchg.get());
     });
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
@@ -1019,14 +1010,12 @@ int hlynr_debug_draws(hlynr_t* s, int64_t env_global_id, uint32_t episode, uint3
                       float uniform_out[4], float normal_out[4]) {
     if (!s) return fail("null handle");
     DeviceGuard g(s->device);
-    void* buf = nullptr;
-    CK(cudaMalloc(&buf, 48));
+    DevPtr<char> buf;
+    CK(alloc(buf, 48));
     debug_draw_kernel<<<1, 1>>>(make_round_keys(s->seed), env_global_id, episode, step, block,
-                                (uint32_t*)buf, (float*)((char*)buf + 16), (float*)((char*)buf + 32));
+                                (uint32_t*)buf.get(), (float*)(buf.get() + 16), (float*)(buf.get() + 32));
     char host[48];
-    cudaError_t e = cudaMemcpy(host, buf, 48, cudaMemcpyDeviceToHost);
-    cudaFree(buf);
-    if (e != cudaSuccess) return fail("hlynr_debug_draws: %s", cudaGetErrorString(e));
+    CK(cudaMemcpy(host, buf.get(), 48, cudaMemcpyDeviceToHost));
     memcpy(raw_out, host, 16); memcpy(uniform_out, host + 16, 16); memcpy(normal_out, host + 32, 16);
     s->launches += 1;
     return 0;
@@ -1111,10 +1100,10 @@ int hlynr_snapshot_save(hlynr_t* s, void* dev_out, HlynrSnapshotInfo* info, void
     snapshot_describe(s, info);
     char* base = (char*)dev_out;
     if (snapshot_kernels(s, *info, base, true, st)) return 1;
-    CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_STATS], s->stats, sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
+    CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_STATS], s->stats.get(), sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
                        cudaMemcpyDeviceToDevice, st));
     if (s->cur_attached)   // CurBlock::num_timesteps is the block's first member
-        CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_CURRICULUM], s->cur_block, sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(base + info->section_offset[HLYNR_SNAP_CURRICULUM], s->cur_block.get(), sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
     else
         CK(cudaMemsetAsync(base + info->section_offset[HLYNR_SNAP_CURRICULUM], 0, sizeof(uint64_t), st));
     return 0;
@@ -1150,17 +1139,17 @@ int hlynr_snapshot_load(hlynr_t* s, const HlynrSnapshotInfo* info, const void* d
     DeviceGuard g(s->device);
     const cudaStream_t st = (cudaStream_t)stream;
     if (refuse_capture(st, "hlynr_snapshot_load")) return 1;
-    if (in.curriculum_attached && !s->cur_block) CK(cudaMalloc(&s->cur_block, sizeof(CurBlock<double>)));
+    if (in.curriculum_attached && !s->cur_block) CK(alloc(s->cur_block, 1));
     // the host state first: the unpack kernel's ring rows follow the restored tick
     s->tick = in.tick; s->env_steps = in.env_steps; s->seed = in.seed; s->cur = in.curriculum;
     s->cur_attached = in.curriculum_attached != 0;
     if (s->cur_attached) { s->sched = in.schedule; s->cur_increment = in.curriculum_increment; }
     char* base = (char*)dev_in;
     if (snapshot_kernels(s, in, base, false, st)) return 1;
-    CK(cudaMemcpyAsync(s->stats, base + in.section_offset[HLYNR_SNAP_STATS], sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
+    CK(cudaMemcpyAsync(s->stats.get(), base + in.section_offset[HLYNR_SNAP_STATS], sizeof(double) * HLYNR_STAT_ROWS * HLYNR_STATS_WORDS,
                        cudaMemcpyDeviceToDevice, st));
     if (s->cur_attached)
-        CK(cudaMemcpyAsync(s->cur_block, base + in.section_offset[HLYNR_SNAP_CURRICULUM], sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(s->cur_block.get(), base + in.section_offset[HLYNR_SNAP_CURRICULUM], sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
     return 0;
 }
 
@@ -1171,13 +1160,12 @@ extern "C" {
 // ---- host-buffer entry points ----------------------------------------------------------------
 static int make_pool(hlynr_sim* s) {
     HostIO& h = s->hio;
-    delete h.pool;
-    h.pool = nullptr;
+    h.pool.reset();
     int helpers = s->host_threads > 0 ? s->host_threads - 1 : 3;
     const int hw = (int)std::thread::hardware_concurrency();
     if (hw > 0 && helpers > hw - 1) helpers = hw - 1;
     if ((size_t)s->n * 26 * sizeof(float) < (size_t(4) << 20)) helpers = 0;  // small shards never reach the pool's threshold
-    h.pool = new (std::nothrow) CopyPool(helpers);
+    h.pool.reset(new (std::nothrow) CopyPool(helpers));
     if (!h.pool) return fail("out of host memory");
     return 0;
 }
@@ -1200,27 +1188,26 @@ static int ensure_hostio(hlynr_sim* s) {
     HostIO& h = s->hio;
     if (h.ready) return 0;
     const size_t n = (size_t)s->n;
-    CK(cudaMallocHost(&h.h_actions, n * 6 * sizeof(float)));
-    CK(cudaMallocHost(&h.h_obs, n * 26 * sizeof(float)));
-    CK(cudaMallocHost(&h.h_reward, n * sizeof(float)));
-    CK(cudaMallocHost(&h.h_term, n)); CK(cudaMallocHost(&h.h_trunc, n)); CK(cudaMallocHost(&h.h_mask, n));
-    CK(cudaMallocHost(&h.h_records_ab[0], n * sizeof(HlynrDoneRecord)));
-    CK(cudaMallocHost(&h.h_records_ab[1], n * sizeof(HlynrDoneRecord)));
-    h.h_records = h.h_records_ab[0];
-    CK(cudaMallocHost(&h.h_done, n));
-    CK(cudaMallocHost(&h.h_count, sizeof(int32_t)));
-    CK(cudaMalloc(&h.d_actions, n * 6 * sizeof(float)));
-    CK(cudaMalloc(&h.d_obs, n * 26 * sizeof(float)));
-    CK(cudaMalloc(&h.d_mask, n));
-    CK(cudaMalloc(&h.d_records, n * sizeof(HlynrDoneRecord)));
-    CK(cudaMalloc(&h.d_counter, sizeof(int32_t)));
-    CK(cudaMemset(h.d_counter, 0, sizeof(int32_t)));
-    memset(&h.d_info, 0, sizeof(h.d_info));
+    CK(alloc(h.h_actions, n * 6));
+    CK(alloc(h.h_obs, n * 26));
+    CK(alloc(h.h_reward, n));
+    CK(alloc(h.h_term, n)); CK(alloc(h.h_trunc, n)); CK(alloc(h.h_mask, n));
+    CK(alloc(h.h_records_ab[0], n));
+    CK(alloc(h.h_records_ab[1], n));
+    h.h_records = h.h_records_ab[0].get();
+    CK(alloc(h.h_done, n));
+    CK(alloc(h.h_count, 1));
+    CK(alloc(h.d_actions, n * 6));
+    CK(alloc(h.d_obs, n * 26));
+    CK(alloc(h.d_mask, n));
+    CK(alloc(h.d_records, n));
+    CK(alloc(h.d_counter, 1));
+    CK(cudaMemset(h.d_counter.get(), 0, sizeof(int32_t)));
     for (int k = 0; k < HLYNR_HOST_STREAMS; ++k) {
-        CK(cudaStreamCreateWithFlags(&h.streams[k], cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&h.ev_done[k], cudaEventDisableTiming));
+        CK(stream_create(h.streams[k]));
+        CK(event_create(h.ev_done[k]));
     }
-    CK(cudaEventCreateWithFlags(&h.ev_start, cudaEventDisableTiming));
+    CK(event_create(h.ev_start));
     if (make_pool(s)) return 1;
     h.ready = true;
     return 0;
@@ -1230,22 +1217,17 @@ static int ensure_hostio(hlynr_sim* s) {
 // Work queued on other caller streams must be synchronised by the caller.
 static int host_streams_begin(hlynr_sim* s) {
     HostIO& h = s->hio;
-    CK(cudaEventRecord(h.ev_start, cudaStreamLegacy));
-    for (int k = 0; k < HLYNR_HOST_STREAMS; ++k) CK(cudaStreamWaitEvent(h.streams[k], h.ev_start, 0));
+    CK(cudaEventRecord(h.ev_start.get(), cudaStreamLegacy));
+    for (int k = 0; k < HLYNR_HOST_STREAMS; ++k) CK(cudaStreamWaitEvent(h.streams[k].get(), h.ev_start.get(), 0));
     return 0;
 }
 static int ensure_host_info(hlynr_sim* s) {
     HostIO& h = s->hio;
     if (h.info_ready) return 0;
     const size_t n = (size_t)s->n;
-    CK(cudaMalloc(&h.d_info.distance, n * 4)); CK(cudaMalloc(&h.d_info.min_distance, n * 4));
-    CK(cudaMalloc(&h.d_info.fuel_remaining, n * 4)); CK(cudaMalloc(&h.d_info.fuel_used, n * 4));
-    CK(cudaMalloc(&h.d_info.steps, n * 4)); CK(cudaMalloc(&h.d_info.flags, n));
-    CK(cudaMalloc(&h.d_info.interceptor_pos, n * 12)); CK(cudaMalloc(&h.d_info.missile_pos, n * 12));
-    CK(cudaMalloc(&h.d_info.episode_return, n * 4)); CK(cudaMalloc(&h.d_info.episode_length, n * 4));
-    CK(cudaMalloc(&h.d_info.missiles_intercepted, n * 4)); CK(cudaMalloc(&h.d_info.missiles_remaining, n * 4));
-    CK(cudaMalloc(&h.d_info.missile_min_distances, n * 4 * HLYNR_MAX_VOLLEY));
-    CK(cudaMalloc(&h.d_info.radar_quality, n * 4));
+#define X(name, type, per_env) CK(alloc(h.info_##name, n * (per_env))); h.d_info.name = h.info_##name.get();
+    HLYNR_INFO_FIELDS(X)
+#undef X
     h.info_ready = true;
     return 0;
 }
@@ -1255,20 +1237,20 @@ int hlynr_reset_host(hlynr_t* s, const uint8_t* mask_host, float* obs_host) {
     DeviceGuard g(s->device);
     if (ensure_hostio(s)) return 1;
     HostIO& h = s->hio;
-    cudaStream_t st = h.streams[0];
+    cudaStream_t st = h.streams[0].get();
     const size_t n = (size_t)s->n, ob = (size_t)s->obs_dim * sizeof(float);
     if (host_streams_begin(s)) return 1;
     if (mask_host) {
-        memcpy(h.h_mask, mask_host, n);
-        CK(cudaMemcpyAsync(h.d_mask, h.h_mask, n, cudaMemcpyHostToDevice, st));
+        memcpy(h.h_mask.get(), mask_host, n);
+        CK(cudaMemcpyAsync(h.d_mask.get(), h.h_mask.get(), n, cudaMemcpyHostToDevice, st));
         // rows of envs that are not reset keep the caller's content
-        if (obs_host != h.h_obs) h.pool->copy(h.h_obs, obs_host, n * ob);
-        CK(cudaMemcpyAsync(h.d_obs, h.h_obs, n * ob, cudaMemcpyHostToDevice, st));
+        if (obs_host != h.h_obs.get()) h.pool->copy(h.h_obs.get(), obs_host, n * ob);
+        CK(cudaMemcpyAsync(h.d_obs.get(), h.h_obs.get(), n * ob, cudaMemcpyHostToDevice, st));
     }
-    if (hlynr_reset(s, mask_host ? h.d_mask : nullptr, h.d_obs, st)) return 1;
-    CK(cudaMemcpyAsync(h.h_obs, h.d_obs, n * ob, cudaMemcpyDeviceToHost, st));
+    if (hlynr_reset(s, mask_host ? h.d_mask.get() : nullptr, h.d_obs.get(), st)) return 1;
+    CK(cudaMemcpyAsync(h.h_obs.get(), h.d_obs.get(), n * ob, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    if (obs_host != h.h_obs) h.pool->copy(obs_host, h.h_obs, n * ob);
+    if (obs_host != h.h_obs.get()) h.pool->copy(obs_host, h.h_obs.get(), n * ob);
     return 0;
 }
 
@@ -1314,18 +1296,18 @@ int hlynr_step_host(hlynr_t* s, const float* actions_host, float* obs_host, floa
     }
     // the handle's own done list for this call (a caller-attached list is restored afterwards)
     HlynrDoneRecord* keep_r = s->done_records; int32_t* keep_c = s->done_counter; const int32_t keep_cap = s->done_cap;
-    s->done_records = h.d_records; s->done_counter = h.d_counter; s->done_cap = (int32_t)(n < INT32_MAX ? n : INT32_MAX);
-    s->io_done = s->host_done ? s->host_done : h.h_done;
+    s->done_records = h.d_records.get(); s->done_counter = h.d_counter.get(); s->done_cap = (int32_t)(n < INT32_MAX ? n : INT32_MAX);
+    s->io_done = s->host_done ? s->host_done : h.h_done.get();
     // caller buffers that are page-locked are used in place; pageable ones go through the handle's pinned staging buffers
-    const bool stage = !(actions_host == h.h_actions || is_pinned_host(actions_host));
-    const float* act_src = stage ? h.h_actions : actions_host;
-    const bool out_direct = (obs_host == h.h_obs || is_pinned_host(obs_host)) && (reward_host == h.h_reward || is_pinned_host(reward_host)) &&
-                            (terminated_host == h.h_term || is_pinned_host(terminated_host)) &&
-                            (truncated_host == h.h_trunc || is_pinned_host(truncated_host));
-    float* obs_dst = out_direct ? obs_host : h.h_obs;
-    float* reward_dst = out_direct ? reward_host : h.h_reward;
-    uint8_t* term_dst = out_direct ? terminated_host : h.h_term;
-    uint8_t* trunc_dst = out_direct ? truncated_host : h.h_trunc;
+    const bool stage = !(actions_host == h.h_actions.get() || is_pinned_host(actions_host));
+    const float* act_src = stage ? h.h_actions.get() : actions_host;
+    const bool out_direct = (obs_host == h.h_obs.get() || is_pinned_host(obs_host)) && (reward_host == h.h_reward.get() || is_pinned_host(reward_host)) &&
+                            (terminated_host == h.h_term.get() || is_pinned_host(terminated_host)) &&
+                            (truncated_host == h.h_trunc.get() || is_pinned_host(truncated_host));
+    float* obs_dst = out_direct ? obs_host : h.h_obs.get();
+    float* reward_dst = out_direct ? reward_host : h.h_reward.get();
+    uint8_t* term_dst = out_direct ? terminated_host : h.h_term.get();
+    uint8_t* trunc_dst = out_direct ? truncated_host : h.h_trunc.get();
     struct Restore { hlynr_sim* s; HlynrDoneRecord* r; int32_t* c; int32_t cap;
                      ~Restore() { s->done_records = r; s->done_counter = c; s->done_cap = cap; s->io_done = nullptr; } }
         restore{s, keep_r, keep_c, keep_cap};
@@ -1339,37 +1321,37 @@ int hlynr_step_host(hlynr_t* s, const float* actions_host, float* obs_host, floa
     auto since = [&] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
     double t_staged[64] = {0}, t_issued = 0, t_synced = 0;
     if (host_streams_begin(s)) return 1;
-    CK(cudaMemsetAsync(h.d_counter, 0, sizeof(int32_t), h.streams[0]));
-    CK(cudaEventRecord(h.ev_start, h.streams[0]));
-    for (int k = 1; k < HLYNR_HOST_STREAMS; ++k) CK(cudaStreamWaitEvent(h.streams[k], h.ev_start, 0));
+    CK(cudaMemsetAsync(h.d_counter.get(), 0, sizeof(int32_t), h.streams[0].get()));
+    CK(cudaEventRecord(h.ev_start.get(), h.streams[0].get()));
+    for (int k = 1; k < HLYNR_HOST_STREAMS; ++k) CK(cudaStreamWaitEvent(h.streams[k].get(), h.ev_start.get(), 0));
     s->tick += 1;
     const HlynrInfoSoA* info = s->host_info ? &h.d_info : nullptr;
-    struct StageGuard { CopyPool* p; ~StageGuard() { if (p) p->finish(); } } stage_guard{stage ? h.pool : nullptr};
-    if (stage) h.pool->start(h.h_actions, actions_host, (size_t)n * 24);
+    struct StageGuard { CopyPool* p; ~StageGuard() { if (p) p->finish(); } } stage_guard{stage ? h.pool.get() : nullptr};
+    if (stage) h.pool->start(h.h_actions.get(), actions_host, (size_t)n * 24);
     for (int64_t c = 0; c < chunks; ++c) {
         const int64_t first = bounds[c], lim = bounds[c + 1], cnt = lim - first;
-        cudaStream_t st = h.streams[c % HLYNR_HOST_STREAMS];
+        cudaStream_t st = h.streams[c % HLYNR_HOST_STREAMS].get();
         if (stage) h.pool->wait_prefix((size_t)lim * 24);
         if (trace && c < 64) t_staged[c] = since();
-        CK(cudaMemcpyAsync(h.d_actions + first * 6, act_src + first * 6, (size_t)cnt * 24, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(h.d_actions.get() + first * 6, act_src + first * 6, (size_t)cnt * 24, cudaMemcpyHostToDevice, st));
         // reward / terminated / truncated (6 B per env) are written by the kernel STRAIGHT into the pinned host buffers
         // (cudaMallocHost memory is device-accessible under unified addressing; coalesced posted PCIe writes, +26 us per
         // 2^20 envs): three small copy-engine transfers per chunk, each with its own fixed latency, disappear and only the
         // observation (104 B per env) rides the copy engine
-        if (step_range(s, first, lim, h.d_actions, h.d_obs, reward_k, term_k, trunc_k, nullptr, info, auto_reset, st)) return 1;
-        CK(cudaMemcpyAsync(obs_dst + first * od, h.d_obs + first * od, (size_t)(cnt * od) * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (step_range(s, first, lim, h.d_actions.get(), h.d_obs.get(), reward_k, term_k, trunc_k, nullptr, info, auto_reset, st)) return 1;
+        CK(cudaMemcpyAsync(obs_dst + first * od, h.d_obs.get() + first * od, (size_t)(cnt * od) * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
     // done list: after every chunk's kernel; count + the first records in one go on stream 0
     for (int k = 1; k < HLYNR_HOST_STREAMS; ++k) {
-        CK(cudaEventRecord(h.ev_done[k], h.streams[k]));
-        CK(cudaStreamWaitEvent(h.streams[0], h.ev_done[k], 0));
+        CK(cudaEventRecord(h.ev_done[k].get(), h.streams[k].get()));
+        CK(cudaStreamWaitEvent(h.streams[0].get(), h.ev_done[k].get(), 0));
     }
     const size_t prefix = (size_t)(n < HLYNR_DONE_PREFIX ? n : HLYNR_DONE_PREFIX);
-    h.h_records = h.h_records_ab[(h.calls++) & 1u];
-    CK(cudaMemcpyAsync(h.h_count, h.d_counter, sizeof(int32_t), cudaMemcpyDeviceToHost, h.streams[0]));
-    CK(cudaMemcpyAsync(h.h_records, h.d_records, prefix * sizeof(HlynrDoneRecord), cudaMemcpyDeviceToHost, h.streams[0]));
+    h.h_records = h.h_records_ab[(h.calls++) & 1u].get();
+    CK(cudaMemcpyAsync(h.h_count.get(), h.d_counter.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, h.streams[0].get()));
+    CK(cudaMemcpyAsync(h.h_records, h.d_records.get(), prefix * sizeof(HlynrDoneRecord), cudaMemcpyDeviceToHost, h.streams[0].get()));
     if (trace) t_issued = since();
-    for (int k = HLYNR_HOST_STREAMS - 1; k >= 0; --k) CK(cudaStreamSynchronize(h.streams[k]));
+    for (int k = HLYNR_HOST_STREAMS - 1; k >= 0; --k) CK(cudaStreamSynchronize(h.streams[k].get()));
     if (trace) {
         t_synced = since();
         fprintf(stderr, "hlynr_step_host: staged");
@@ -1383,9 +1365,9 @@ int hlynr_step_host(hlynr_t* s, const float* actions_host, float* obs_host, floa
     int32_t count = *h.h_count;
     if (count > s->done_cap) count = s->done_cap;
     if ((size_t)count > prefix) {
-        CK(cudaMemcpyAsync(h.h_records + prefix, h.d_records + prefix, ((size_t)count - prefix) * sizeof(HlynrDoneRecord),
-                           cudaMemcpyDeviceToHost, h.streams[0]));
-        CK(cudaStreamSynchronize(h.streams[0]));
+        CK(cudaMemcpyAsync(h.h_records + prefix, h.d_records.get() + prefix, ((size_t)count - prefix) * sizeof(HlynrDoneRecord),
+                           cudaMemcpyDeviceToHost, h.streams[0].get()));
+        CK(cudaStreamSynchronize(h.streams[0].get()));
     }
     h.last_count = count;
     if (terminal_obs_host)  // only rows of finished envs are written (info['terminal_observation'])
@@ -1407,22 +1389,10 @@ int hlynr_info_host(hlynr_t* s, HlynrInfoSoA* o) {
     DeviceGuard g(s->device);
     const HlynrInfoSoA& d = s->hio.d_info;
     const size_t n = (size_t)s->n;
-    cudaStream_t st = s->hio.streams[0];
-    if (o->distance) CK(cudaMemcpyAsync(o->distance, d.distance, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->min_distance) CK(cudaMemcpyAsync(o->min_distance, d.min_distance, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->fuel_remaining) CK(cudaMemcpyAsync(o->fuel_remaining, d.fuel_remaining, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->fuel_used) CK(cudaMemcpyAsync(o->fuel_used, d.fuel_used, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->steps) CK(cudaMemcpyAsync(o->steps, d.steps, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->flags) CK(cudaMemcpyAsync(o->flags, d.flags, n, cudaMemcpyDeviceToHost, st));
-    if (o->interceptor_pos) CK(cudaMemcpyAsync(o->interceptor_pos, d.interceptor_pos, n * 12, cudaMemcpyDeviceToHost, st));
-    if (o->missile_pos) CK(cudaMemcpyAsync(o->missile_pos, d.missile_pos, n * 12, cudaMemcpyDeviceToHost, st));
-    if (o->episode_return) CK(cudaMemcpyAsync(o->episode_return, d.episode_return, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->episode_length) CK(cudaMemcpyAsync(o->episode_length, d.episode_length, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->missiles_intercepted) CK(cudaMemcpyAsync(o->missiles_intercepted, d.missiles_intercepted, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->missiles_remaining) CK(cudaMemcpyAsync(o->missiles_remaining, d.missiles_remaining, n * 4, cudaMemcpyDeviceToHost, st));
-    if (o->missile_min_distances)
-        CK(cudaMemcpyAsync(o->missile_min_distances, d.missile_min_distances, n * 4 * HLYNR_MAX_VOLLEY, cudaMemcpyDeviceToHost, st));
-    if (o->radar_quality) CK(cudaMemcpyAsync(o->radar_quality, d.radar_quality, n * 4, cudaMemcpyDeviceToHost, st));
+    cudaStream_t st = s->hio.streams[0].get();
+#define X(name, type, per_env) if (o->name) CK(cudaMemcpyAsync(o->name, d.name, n * (per_env) * sizeof(type), cudaMemcpyDeviceToHost, st));
+    HLYNR_INFO_FIELDS(X)
+#undef X
     CK(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1432,7 +1402,7 @@ int hlynr_pinned_done(hlynr_t* s, uint8_t** done) {
     if (!s || !done) return fail("hlynr_pinned_done: null argument");
     DeviceGuard g(s->device);
     if (ensure_hostio(s)) return 1;
-    *done = s->hio.h_done;
+    *done = s->hio.h_done.get();
     return 0;
 }
 
@@ -1450,11 +1420,11 @@ int hlynr_pinned_buffers(hlynr_t* s, float** actions, float** obs, float** rewar
     if (!s) return fail("null handle");
     DeviceGuard g(s->device);
     if (ensure_hostio(s)) return 1;
-    if (actions) *actions = s->hio.h_actions;
-    if (obs) *obs = s->hio.h_obs;
-    if (reward) *reward = s->hio.h_reward;
-    if (terminated) *terminated = s->hio.h_term;
-    if (truncated) *truncated = s->hio.h_trunc;
+    if (actions) *actions = s->hio.h_actions.get();
+    if (obs) *obs = s->hio.h_obs.get();
+    if (reward) *reward = s->hio.h_reward.get();
+    if (terminated) *terminated = s->hio.h_term.get();
+    if (truncated) *truncated = s->hio.h_trunc.get();
     return 0;
 }
 

@@ -1,6 +1,9 @@
 // hlynr_host.cuh -- host-side helpers shared by the translation units of the library (internal: not part of include/ or the ABI).
 #pragma once
 
+#include <memory>
+#include <type_traits>
+
 #include <cuda_runtime.h>
 
 // Formats the message into the calling thread's hlynr_last_error() and returns 1 (defined in hlynr_capi.cu).
@@ -33,3 +36,40 @@ struct DeviceGuard {
     }
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+// Owners of the CUDA resources a handle allocates: each releases what it holds when it is destroyed or re-assigned, so a
+// handle's destructor frees everything and an allocation repeated after a failure leaks nothing.  The resources belong to the
+// device that was current when they were made; the owner must be destroyed with that device current (a DeviceGuard).
+struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void* p) const { cudaFreeHost(p); } };
+struct CudaStreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct CudaEventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;       // device memory
+template <class T> using PinnedPtr = std::unique_ptr<T, CudaFreeHost>;  // page-locked host memory
+using StreamOwner = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, CudaStreamDestroy>;
+using EventOwner = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, CudaEventDestroy>;
+
+// The helpers below replace what the owner held, and leave it empty if the call fails; use them under CK.
+// `count` elements of device memory (DevPtr) or page-locked host memory (PinnedPtr); the old block is freed first.
+template <class T, class D> cudaError_t alloc(std::unique_ptr<T, D>& p, size_t count) {
+    static_assert(std::is_same<D, CudaFree>::value || std::is_same<D, CudaFreeHost>::value, "a DevPtr or a PinnedPtr");
+    p.reset();
+    void* q = nullptr;
+    const cudaError_t e = std::is_same<D, CudaFree>::value ? cudaMalloc(&q, count * sizeof(T)) : cudaMallocHost(&q, count * sizeof(T));
+    if (e == cudaSuccess) p.reset(static_cast<T*>(q));
+    return e;
+}
+// a stream that does not synchronise with the legacy default stream
+inline cudaError_t stream_create(StreamOwner& s) {
+    cudaStream_t q = nullptr;
+    const cudaError_t e = cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking);
+    s.reset(e == cudaSuccess ? q : nullptr);
+    return e;
+}
+// an event for ordering only (no timing)
+inline cudaError_t event_create(EventOwner& ev) {
+    cudaEvent_t q = nullptr;
+    const cudaError_t e = cudaEventCreateWithFlags(&q, cudaEventDisableTiming);
+    ev.reset(e == cudaSuccess ? q : nullptr);
+    return e;
+}

@@ -647,11 +647,11 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 struct hlynr_policy {
     int device = 0, sm_count = 148;
     int in_dim = IN, kb0 = IN_PAD / BK;   // input width, K blocks of the first GEMM
-    __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wh = nullptr;   // [512,64*kb0], [512,512], [256,512], [16,256]
-    float* vec = nullptr;   // b1 g1 be1 (512 x3) | b2 g2 be2 (512 x3) | b3 g3 be3 (256 x3) | bh (16) | log_std (8)
-    int* error_flag = nullptr;
-    unsigned long long* ctr = nullptr;   // 16 bytes: the device-resident call counter (u64), then the forward's ticket (u32)
-    long long* timing = nullptr;   // debug timestamps (option "timing")
+    DevPtr<__nv_bfloat16> w1, w2, w3, wh;   // [512,64*kb0], [512,512], [256,512], [16,256]
+    DevPtr<float> vec;   // b1 g1 be1 (512 x3) | b2 g2 be2 (512 x3) | b3 g3 be3 (256 x3) | bh (16) | log_std (8)
+    DevPtr<int> error_flag;
+    DevPtr<unsigned long long> ctr;   // 16 bytes: the device-resident call counter (u64), then the forward's ticket (u32)
+    DevPtr<long long> timing;   // debug timestamps (option "timing")
     int timing_on = 0;
     CUtensorMap tm[3][4];   // [log2(cluster size)][layer]: box rows = N / cluster size
     int cluster = 1;        // CTAs per cluster (option "cluster": 1, 2 or 4)
@@ -686,7 +686,6 @@ extern "C" {
 void hlynr_policy_destroy(hlynr_policy_t* p) {
     if (!p) return;
     DeviceGuard g(p->device);
-    cudaFree(p->w1); cudaFree(p->w2); cudaFree(p->w3); cudaFree(p->wh); cudaFree(p->vec); cudaFree(p->error_flag); cudaFree(p->ctr); cudaFree(p->timing);
     delete p;
 }
 
@@ -702,40 +701,33 @@ int hlynr_policy_create_dim(int device, int in_dim, hlynr_policy_t** out) {
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     if (prop.major != 10) return fail("hlynr_policy_create: the fused policy kernel is sm_100a code (tcgen05 / TMEM); device %d is sm_%d%d", device, prop.major, prop.minor);
-    hlynr_policy* p = new (std::nothrow) hlynr_policy();
+    std::unique_ptr<hlynr_policy> p(new (std::nothrow) hlynr_policy());
     if (!p) return fail("hlynr_policy_create: out of host memory");
     p->device = device; p->sm_count = prop.multiProcessorCount;
     p->in_dim = in_dim; p->kb0 = (in_dim + BK - 1) / BK;
-    cudaError_t e = cudaSuccess;
     // the TMA map needs 16-byte row strides: w1 lives in a [512, 64 * kb0] buffer whose columns past in_dim are zero
-    if (e == cudaSuccess) e = cudaMalloc(&p->w1, sizeof(__nv_bfloat16) * H1 * BK * p->kb0);
-    if (e == cudaSuccess) e = cudaMalloc(&p->w2, sizeof(__nv_bfloat16) * H2 * H1);
-    if (e == cudaSuccess) e = cudaMalloc(&p->w3, sizeof(__nv_bfloat16) * H3 * H2);
-    if (e == cudaSuccess) e = cudaMalloc(&p->wh, sizeof(__nv_bfloat16) * HEAD_N * H3);
-    if (e == cudaSuccess) e = cudaMalloc(&p->vec, sizeof(float) * VEC_TOTAL);
-    if (e == cudaSuccess) e = cudaMalloc(&p->error_flag, sizeof(int));
-    if (e == cudaSuccess) e = cudaMemset(p->error_flag, 0, sizeof(int));
-    if (e == cudaSuccess) e = cudaMalloc(&p->ctr, 16);
-    if (e == cudaSuccess) e = cudaMemset(p->ctr, 0, 16);
-    if (e != cudaSuccess) { const int r = fail("hlynr_policy_create: %s", cudaGetErrorString(e)); hlynr_policy_destroy(p); return r; }
+    CK(alloc(p->w1, H1 * BK * p->kb0));
+    CK(alloc(p->w2, H2 * H1));
+    CK(alloc(p->w3, H3 * H2));
+    CK(alloc(p->wh, HEAD_N * H3));
+    CK(alloc(p->vec, VEC_TOTAL));
+    CK(alloc(p->error_flag, 1));
+    CK(cudaMemset(p->error_flag.get(), 0, sizeof(int)));
+    CK(alloc(p->ctr, 2));
+    CK(cudaMemset(p->ctr.get(), 0, 16));
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
-    e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-    if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn) {
-        const int r = fail("hlynr_policy_create: cuTensorMapEncodeTiled is not available from the driver");
-        hlynr_policy_destroy(p);
-        return r;
-    }
+    const cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
+    if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn)
+        return fail("hlynr_policy_create: cuTensorMapEncodeTiled is not available from the driver");
     EncodeTiledFn enc = reinterpret_cast<EncodeTiledFn>(fn);
     for (int c = 0; c < 3; ++c) {
         const int cl = 1 << c;
-        if (make_map(enc, &p->tm[c][0], p->w1, H1, BK * p->kb0, BN / cl) || make_map(enc, &p->tm[c][1], p->w2, H2, H1, BN / cl) ||
-            make_map(enc, &p->tm[c][2], p->w3, H3, H2, BN / cl) || make_map(enc, &p->tm[c][3], p->wh, HEAD_N, H3, HEAD_N / cl)) {
-            hlynr_policy_destroy(p);
+        if (make_map(enc, &p->tm[c][0], p->w1.get(), H1, BK * p->kb0, BN / cl) || make_map(enc, &p->tm[c][1], p->w2.get(), H2, H1, BN / cl) ||
+            make_map(enc, &p->tm[c][2], p->w3.get(), H3, H2, BN / cl) || make_map(enc, &p->tm[c][3], p->wh.get(), HEAD_N, H3, HEAD_N / cl))
             return 1;
-        }
     }
-    *out = p;
+    *out = p.release();
     return 0;
 }
 
@@ -750,18 +742,18 @@ int hlynr_policy_set_weights(hlynr_policy_t* p, const HlynrPolicyWeights* w, voi
         const int n = rows_dst * k_dst;
         pack_bf16_kernel<<<(n + 255) / 256, 256, 0, st>>>(src, rows, k, dst, rows_dst, k_dst);
     };
-    auto vec = [&](const float* src, int n, int off, int n_dst) { copy_f32_kernel<<<(n_dst + 255) / 256, 256, 0, st>>>(src, p->vec + off, n, n_dst); };
-    pack(w->w1, H1, p->in_dim, p->w1, H1, BK * p->kb0);
-    pack(w->w2, H2, H1, p->w2, H2, H1);
-    pack(w->w3, H3, H2, p->w3, H3, H2);
-    CK(cudaMemsetAsync(p->wh, 0, sizeof(__nv_bfloat16) * HEAD_N * H3, st));
-    pack(w->wa, ACT, H3, p->wh, ACT, H3);                 // rows 0-5: action_net
-    pack(w->wv, 1, H3, p->wh + (size_t)ACT * H3, 1, H3);  // row 6: value_net
-    auto centred = [&](const float* src, int n, int off) { copy_centred_f32_kernel<<<1, 256, 0, st>>>(src, p->vec + off, n); };
+    auto vec = [&](const float* src, int n, int off, int n_dst) { copy_f32_kernel<<<(n_dst + 255) / 256, 256, 0, st>>>(src, p->vec.get() + off, n, n_dst); };
+    pack(w->w1, H1, p->in_dim, p->w1.get(), H1, BK * p->kb0);
+    pack(w->w2, H2, H1, p->w2.get(), H2, H1);
+    pack(w->w3, H3, H2, p->w3.get(), H3, H2);
+    CK(cudaMemsetAsync(p->wh.get(), 0, sizeof(__nv_bfloat16) * HEAD_N * H3, st));
+    pack(w->wa, ACT, H3, p->wh.get(), ACT, H3);                 // rows 0-5: action_net
+    pack(w->wv, 1, H3, p->wh.get() + (size_t)ACT * H3, 1, H3);  // row 6: value_net
+    auto centred = [&](const float* src, int n, int off) { copy_centred_f32_kernel<<<1, 256, 0, st>>>(src, p->vec.get() + off, n); };
     centred(w->b1, H1, VEC_B1); vec(w->ln1_g, H1, VEC_G1, H1); vec(w->ln1_b, H1, VEC_BE1, H1);
     centred(w->b2, H2, VEC_B2); vec(w->ln2_g, H2, VEC_G2, H2); vec(w->ln2_b, H2, VEC_BE2, H2);
     centred(w->b3, H3, VEC_B3); vec(w->ln3_g, H3, VEC_G3, H3); vec(w->ln3_b, H3, VEC_BE3, H3);
-    CK(cudaMemsetAsync(p->vec + VEC_BH, 0, sizeof(float) * 16, st));
+    CK(cudaMemsetAsync(p->vec.get() + VEC_BH, 0, sizeof(float) * 16, st));
     vec(w->ba, ACT, VEC_BH, ACT); vec(w->bv, 1, VEC_BH + ACT, 1);
     vec(w->log_std, ACT, VEC_LS, 8);
     CK(cudaGetLastError());
@@ -792,13 +784,13 @@ int launch_forward(const char* fn, hlynr_policy_t* p, const float* obs_dev, int6
     Params P;
     memset(&P, 0, sizeof(P));
     P.obs = obs_dev; P.in_dim = p->in_dim; P.kb0 = p->kb0; P.n_rows = n_rows; P.n_rows_dev = n_rows_dev;
-    P.vec = p->vec;
+    P.vec = p->vec.get();
     P.actions = actions_dev; P.values = values_dev; P.logp = logp_dev; P.mean = mean_dev; P.actions_clipped = actions_clipped_dev;
     P.ln_eps = p->ln_eps;
     P.k0 = (uint32_t)seed; P.k1 = (uint32_t)(seed >> 32); P.ctr_lo = (uint32_t)counter; P.ctr_hi = (uint32_t)(counter >> 32);
-    unsigned long long* ctr_dev = dev_counter ? p->ctr : nullptr;
-    P.deterministic = deterministic; P.error_flag = p->error_flag;
-    P.timing = p->timing_on ? p->timing : nullptr; P.timing_tiles = 8;
+    unsigned long long* ctr_dev = dev_counter ? p->ctr.get() : nullptr;
+    P.deterministic = deterministic; P.error_flag = p->error_flag.get();
+    P.timing = p->timing_on ? p->timing.get() : nullptr; P.timing_tiles = 8;
     const int64_t n_tiles = (n_rows + BM - 1) / BM;
     const int cl = p->cluster, ci = cl == 4 ? 2 : (cl == 2 ? 1 : 0);
     const ForwardKernel kernel = forward_kernel(ci, fixed);
@@ -851,7 +843,7 @@ int hlynr_policy_forward_dev(hlynr_policy_t* p, const float* obs_dev, int64_t n_
 int hlynr_policy_set_counter(hlynr_policy_t* p, uint64_t value, void* stream) {
     if (!p) return fail("hlynr_policy_set_counter: null argument");
     DeviceGuard g(p->device);
-    set_counter_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(p->ctr, (unsigned long long)value);
+    set_counter_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(p->ctr.get(), (unsigned long long)value);
     CK(cudaGetLastError());
     p->launches += 1;
     return 0;
@@ -863,7 +855,7 @@ int hlynr_policy_get_counter(hlynr_policy_t* p, uint64_t* out, void* stream) {
     const cudaStream_t st = (cudaStream_t)stream;
     CK(cudaStreamSynchronize(st));
     unsigned long long v = 0;
-    CK(cudaMemcpyAsync(&v, p->ctr, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&v, p->ctr.get(), sizeof(v), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     *out = (uint64_t)v;
     return 0;
@@ -873,7 +865,12 @@ int hlynr_policy_set_option(hlynr_policy_t* p, const char* name, int64_t value) 
     if (!p || !name) return fail("null argument");
     if (strcmp(name, "timing") == 0) {   // debug: record SM-clock timestamps of the phases of CTA 0's first 8 tiles
         DeviceGuard g(p->device);
-        if (value && !p->timing) { CK(cudaMalloc(&p->timing, sizeof(long long) * 8 * 16)); CK(cudaMemset(p->timing, 0, sizeof(long long) * 8 * 16)); }
+        if (value && !p->timing) {
+            DevPtr<long long> t;   // kept only once it is zeroed
+            CK(alloc(t, 8 * 16));
+            CK(cudaMemset(t.get(), 0, sizeof(long long) * 8 * 16));
+            p->timing = std::move(t);
+        }
         p->timing_on = value != 0;
         return 0;
     }
@@ -891,7 +888,7 @@ int hlynr_policy_get_timing(hlynr_policy_t* p, long long* host_out) {
     if (!p || !host_out || !p->timing) return fail("hlynr_policy_get_timing: option \"timing\" was never enabled");
     DeviceGuard g(p->device);
     CK(cudaDeviceSynchronize());
-    CK(cudaMemcpy(host_out, p->timing, sizeof(long long) * 8 * 16, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(host_out, p->timing.get(), sizeof(long long) * 8 * 16, cudaMemcpyDeviceToHost));
     return 0;
 }
 

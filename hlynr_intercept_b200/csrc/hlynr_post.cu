@@ -338,12 +338,12 @@ struct hlynr_post {
     int64_t n = 0, plane = 0;   // plane = floats per ring slot (n * fw rounded up to 128-byte multiples)
     int device = 0, fw = OD, k = 1, D = OD;   // frame width (26 or 17), n_stack, fw * n_stack
     double clip = 10.0, eps = 1e-8, gamma = 0.99;
-    float* frames = nullptr;
-    uint8_t* age[2] = {nullptr, nullptr};
+    DevPtr<float> frames;
+    DevPtr<uint8_t> age[2];
     int age_cur = 0;
-    double* returns = nullptr;
-    PostStats* st = nullptr;
-    double* partials = nullptr; // [max_blocks][PART_WORDS] first-stage sums
+    DevPtr<double> returns;
+    DevPtr<PostStats> st;
+    DevPtr<double> partials;    // [max_blocks][PART_WORDS] first-stage sums
     uint32_t t = 0;             // frames written so far; target slot = t % k, newest = (t - 1) % k
     bool sums_valid = false;    // the per-lag sums S/Q describe the current ring (maintained by every reset/step that can)
     int sm_count = 148;
@@ -371,11 +371,11 @@ static int launch_normalize_t(hlynr_post* p, float* out, int raw, cudaStream_t s
         const int P = p->D / 2;
         const int lanes = 512 / P > 0 ? 512 / P : 1;
         normalize_kernel<<<blocks_for(p, (p->n + NORM_UNROLL - 1) / NORM_UNROLL, lanes), lanes * P, 0, st>>>(
-            p->frames, p->plane, p->age[p->age_cur], p->st, out, p->n, p->k, newest, (float)p->clip, raw);
+            p->frames.get(), p->plane, p->age[p->age_cur].get(), p->st.get(), out, p->n, p->k, newest, (float)p->clip, raw);
     } else {
         const int lanes = 512 / p->D;
         normalize1_kernel<F><<<blocks_for(p, (p->n + NORM_UNROLL - 1) / NORM_UNROLL, lanes), lanes * p->D, 0, st>>>(
-            p->frames, p->plane, p->age[p->age_cur], p->st, out, p->n, p->k, newest, (float)p->clip, raw);
+            p->frames.get(), p->plane, p->age[p->age_cur].get(), p->st.get(), out, p->n, p->k, newest, (float)p->clip, raw);
     }
     CK(cudaGetLastError());
     p->launches += 1;
@@ -388,17 +388,17 @@ static int launch_normalize(hlynr_post* p, float* out, int raw, cudaStream_t st)
 
 template <int F>
 static int reset_t(hlynr_post* p, float* out_dev, int training, cudaStream_t st) {
-    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
+    const float* frame = p->frames.get() + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
     p->t += 1;
-    CK(cudaMemsetAsync(p->returns, 0, sizeof(double) * p->n, st));  // VecNormalize.reset: returns = zeros
+    CK(cudaMemsetAsync(p->returns.get(), 0, sizeof(double) * p->n, st));  // VecNormalize.reset: returns = zeros
     const int nb_col = blocks_for(p, p->n, 16);
-    colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials);
-    fold_kernel<F><<<2 * F, 256, 0, st>>>(p->partials, nb_col, 0, 0, 0, p->st);
-    merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 1, 0, p->eps);
+    colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials.get());
+    fold_kernel<F><<<2 * F, 256, 0, st>>>(p->partials.get(), nb_col, 0, 0, 0, p->st.get());
+    merge_kernel<F><<<1, 256, 0, st>>>(p->st.get(), p->k, (double)p->n, 1, training, 1, 0, p->eps);
     CK(cudaGetLastError());
     p->launches += 3;
     p->sums_valid = true;
-    CK(cudaMemsetAsync(p->age[p->age_cur], 0, p->n, st));  // VecFrameStack.reset: only the newest frame is valid
+    CK(cudaMemsetAsync(p->age[p->age_cur].get(), 0, p->n, st));  // VecFrameStack.reset: only the newest frame is valid
     return launch_normalize_t<F>(p, out_dev, 0, st);
 }
 
@@ -407,34 +407,34 @@ static int step_t(hlynr_post* p, const float* reward_dev, const uint8_t* termina
                   const HlynrDoneRecord* records_dev, const int32_t* counter_dev, int32_t capacity, float* out_dev,
                   float* terminal_out_dev, int training, bool can_maintain, cudaStream_t st) {
     const int newest_old = (int)((p->t - 1) % (uint32_t)p->k);
-    const float* frame = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
-    const uint8_t* age_old = p->age[p->age_cur];
+    const float* frame = p->frames.get() + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
+    const uint8_t* age_old = p->age[p->age_cur].get();
     p->t += 1;
     const int nb_ret = blocks_for(p, p->n, 256);
-    returns_kernel<F><<<nb_ret, 256, 0, st>>>(p->returns, reward_dev, terminated_dev, truncated_dev, p->n, p->gamma, p->partials, training,
-                                              age_old, p->age[p->age_cur ^ 1], p->k);
+    returns_kernel<F><<<nb_ret, 256, 0, st>>>(p->returns.get(), reward_dev, terminated_dev, truncated_dev, p->n, p->gamma, p->partials.get(), training,
+                                              age_old, p->age[p->age_cur ^ 1].get(), p->k);
     p->launches += 1;
     if (can_maintain && p->sums_valid) {  // the sums follow the ring on every step; obs_rms / ret_rms only move when training
         const int nb_col = blocks_for(p, p->n, 16);
-        colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials);
+        colsum_kernel<F><<<nb_col, 16 * F, 0, st>>>(frame, p->n, p->partials.get());
         p->launches += 1;
         const int per = (p->k - 1) * F;
         if (p->k > 1) {
             const int lanes = 512 / per;
-            done_corr_kernel<F><<<64, lanes * per, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->k, newest_old,
-                                                            p->partials);
+            done_corr_kernel<F><<<64, lanes * per, 0, st>>>(records_dev, counter_dev, capacity, p->frames.get(), p->plane, age_old, p->k, newest_old,
+                                                            p->partials.get());
             p->launches += 1;
         }
-        fold_kernel<F><<<2 * F + 2 + 2 * per, 256, 0, st>>>(p->partials, nb_col, training ? nb_ret : 0, 64, per, p->st);
+        fold_kernel<F><<<2 * F + 2 + 2 * per, 256, 0, st>>>(p->partials.get(), nb_col, training ? nb_ret : 0, 64, per, p->st.get());
         p->launches += 1;
-        merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 1, training, 0, training, p->eps);
+        merge_kernel<F><<<1, 256, 0, st>>>(p->st.get(), p->k, (double)p->n, 1, training, 0, training, p->eps);
         p->launches += 1;
     } else {
         p->sums_valid = false;
     }
     if (terminal_out_dev) {
         const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
-        terminal_kernel<F><<<64, lanes * p->D, 0, st>>>(records_dev, counter_dev, capacity, p->frames, p->plane, age_old, p->st, terminal_out_dev,
+        terminal_kernel<F><<<64, lanes * p->D, 0, st>>>(records_dev, counter_dev, capacity, p->frames.get(), p->plane, age_old, p->st.get(), terminal_out_dev,
                                                         p->k, newest_old, (float)p->clip);
         p->launches += 1;
     }
@@ -459,39 +459,35 @@ int hlynr_post_create_frames(int64_t n_envs, int device, int frame_dim, int n_st
     CK(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail("hlynr_post_create: device %d not available", device);
     DeviceGuard g(device);
-    hlynr_post* p = new (std::nothrow) hlynr_post();
+    std::unique_ptr<hlynr_post> p(new (std::nothrow) hlynr_post());
     if (!p) return fail("hlynr_post_create: out of host memory");
     p->n = n_envs; p->device = device; p->fw = frame_dim; p->k = n_stack; p->D = frame_dim * n_stack;
     p->clip = clip_obs; p->eps = epsilon; p->gamma = gamma;
     p->plane = ((n_envs * frame_dim + 31) / 32) * 32;  // every slot starts 128-byte aligned
-    cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device);
-    cudaError_t e = cudaMalloc(&p->frames, sizeof(float) * p->plane * n_stack);
-    if (e == cudaSuccess) e = cudaMalloc(&p->age[0], n_envs);
-    if (e == cudaSuccess) e = cudaMalloc(&p->age[1], n_envs);
-    if (e == cudaSuccess) e = cudaMalloc(&p->returns, sizeof(double) * n_envs);
-    if (e == cudaSuccess) e = cudaMalloc(&p->st, sizeof(PostStats));
-    if (e == cudaSuccess) e = cudaMalloc(&p->partials, sizeof(double) * PART_WORDS * ((size_t)p->sm_count * 8 + 64));
-    if (e == cudaSuccess) e = cudaMemset(p->partials, 0, sizeof(double) * PART_WORDS * ((size_t)p->sm_count * 8 + 64));
-    if (e != cudaSuccess) { int r = fail("hlynr_post_create: cudaMalloc failed: %s", cudaGetErrorString(e)); hlynr_post_destroy(p); return r; }
-    cudaMemset(p->frames, 0, sizeof(float) * p->plane * n_stack);
-    cudaMemset(p->age[0], 0, n_envs); cudaMemset(p->age[1], 0, n_envs);
-    cudaMemset(p->returns, 0, sizeof(double) * n_envs);
-    PostStats* h = new (std::nothrow) PostStats();
-    if (!h) { hlynr_post_destroy(p); return fail("hlynr_post_create: out of host memory"); }
-    memset(h, 0, sizeof(*h));
+    CK(cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device));
+    const size_t partial_words = PART_WORDS * ((size_t)p->sm_count * 8 + 64);
+    CK(alloc(p->frames, p->plane * n_stack));
+    CK(alloc(p->age[0], n_envs));
+    CK(alloc(p->age[1], n_envs));
+    CK(alloc(p->returns, n_envs));
+    CK(alloc(p->st, 1));
+    CK(alloc(p->partials, partial_words));
+    CK(cudaMemset(p->partials.get(), 0, sizeof(double) * partial_words));
+    CK(cudaMemset(p->frames.get(), 0, sizeof(float) * p->plane * n_stack));
+    CK(cudaMemset(p->age[0].get(), 0, n_envs)); CK(cudaMemset(p->age[1].get(), 0, n_envs));
+    CK(cudaMemset(p->returns.get(), 0, sizeof(double) * n_envs));
+    std::unique_ptr<PostStats> h(new (std::nothrow) PostStats());   // value-initialised: all zeros
+    if (!h) return fail("hlynr_post_create: out of host memory");
     for (int f = 0; f < DMAX; ++f) { h->var[f] = 1.0; h->inv_std[f] = 1.0 / sqrt(1.0 + epsilon); }
     h->count = 1e-4; h->ret_var = 1.0; h->ret_count = 1e-4;  // RunningMeanStd(epsilon=1e-4)
-    e = cudaMemcpy(p->st, h, sizeof(*h), cudaMemcpyHostToDevice);
-    delete h;
-    if (e != cudaSuccess) { int r = fail("hlynr_post_create: %s", cudaGetErrorString(e)); hlynr_post_destroy(p); return r; }
-    *out = p;
+    CK(cudaMemcpy(p->st.get(), h.get(), sizeof(*h), cudaMemcpyHostToDevice));
+    *out = p.release();
     return 0;
 }
 
 void hlynr_post_destroy(hlynr_post_t* p) {
     if (!p) return;
     DeviceGuard g(p->device);
-    cudaFree(p->frames); cudaFree(p->age[0]); cudaFree(p->age[1]); cudaFree(p->returns); cudaFree(p->st); cudaFree(p->partials);
     delete p;
 }
 
@@ -506,7 +502,7 @@ int hlynr_post_note_replayed_steps(hlynr_post_t* p, int64_t steps, int64_t launc
 
 int hlynr_post_obs_target(hlynr_post_t* p, float** obs_dev) {
     if (!p || !obs_dev) return fail("hlynr_post_obs_target: null argument");
-    *obs_dev = p->frames + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
+    *obs_dev = p->frames.get() + (int64_t)(p->t % (uint32_t)p->k) * p->plane;
     return 0;
 }
 
@@ -547,7 +543,7 @@ int hlynr_post_normalize(hlynr_post_t* p, const float* stacked_dev, int64_t rows
     if (rows <= 0) return 0;
     DeviceGuard g(p->device);
     const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
-    normalize_rows_kernel<<<blocks_for(p, rows, lanes), lanes * p->D, 0, (cudaStream_t)stream>>>(stacked_dev, out_dev, rows, p->D, p->st, (float)p->clip);
+    normalize_rows_kernel<<<blocks_for(p, rows, lanes), lanes * p->D, 0, (cudaStream_t)stream>>>(stacked_dev, out_dev, rows, p->D, p->st.get(), (float)p->clip);
     CK(cudaGetLastError());
     p->launches += 1;
     return 0;
@@ -557,18 +553,16 @@ int hlynr_post_get_stats(hlynr_post_t* p, double* mean, double* var, double* cou
                          double* ret_count, void* stream) {
     if (!p) return fail("hlynr_post_get_stats: null handle");
     DeviceGuard g(p->device);
-    PostStats* h = new (std::nothrow) PostStats();
+    std::unique_ptr<PostStats> h(new (std::nothrow) PostStats());
     if (!h) return fail("out of host memory");
-    cudaError_t e = cudaMemcpyAsync(h, p->st, sizeof(*h), cudaMemcpyDeviceToHost, (cudaStream_t)stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
-    if (e != cudaSuccess) { delete h; return fail("hlynr_post_get_stats: %s", cudaGetErrorString(e)); }
+    CK(cudaMemcpyAsync(h.get(), p->st.get(), sizeof(*h), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    CK(cudaStreamSynchronize((cudaStream_t)stream));
     if (mean) memcpy(mean, h->mean, sizeof(double) * p->D);
     if (var) memcpy(var, h->var, sizeof(double) * p->D);
     if (count) *count = h->count;
     if (ret_mean) *ret_mean = h->ret_mean;
     if (ret_var) *ret_var = h->ret_var;
     if (ret_count) *ret_count = h->ret_count;
-    delete h;
     return 0;
 }
 
@@ -582,7 +576,7 @@ int hlynr_post_set_stats(hlynr_post_t* p, const double* mean, const double* var,
     const double tail[4] = {count, ret_mean, ret_var, ret_count};
     CK(cudaMemcpyAsync(&p->st->count, &tail[0], sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(&p->st->ret_mean, &tail[1], sizeof(double) * 3, cudaMemcpyHostToDevice, st));
-    with_width(p, [&](auto F) { merge_kernel<F><<<1, 256, 0, st>>>(p->st, p->k, (double)p->n, 0, 0, 0, 0, p->eps); });  // refresh inv_std
+    with_width(p, [&](auto F) { merge_kernel<F><<<1, 256, 0, st>>>(p->st.get(), p->k, (double)p->n, 0, 0, 0, 0, p->eps); });  // refresh inv_std
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));  // `tail` is a stack array
     p->launches += 1;
@@ -610,22 +604,22 @@ static int post_snapshot_copy(hlynr_post* p, const HlynrPostSnapshotInfo& info, 
     const size_t slot = sizeof(float) * (size_t)p->n * p->fw;
     const int newest = (int)((p->t - 1) % (uint32_t)p->k);
     for (int j = 0; j < p->k; ++j) {
-        float* ring = p->frames + (int64_t)((newest - (p->k - 1 - j) + p->k) % p->k) * p->plane;
+        float* ring = p->frames.get() + (int64_t)((newest - (p->k - 1 - j) + p->k) % p->k) * p->plane;
         char* img = base + info.section_offset[HLYNR_POST_SNAP_FRAMES] + (size_t)j * slot;
         CK(cudaMemcpyAsync(save ? (void*)img : (void*)ring, save ? (const void*)ring : (const void*)img, slot, cudaMemcpyDeviceToDevice, st));
     }
-    uint8_t* age = p->age[p->age_cur];
+    uint8_t* age = p->age[p->age_cur].get();
     char* img_age = base + info.section_offset[HLYNR_POST_SNAP_AGE];
     char* img_ret = base + info.section_offset[HLYNR_POST_SNAP_RETURNS];
     char* img_st = base + info.section_offset[HLYNR_POST_SNAP_STATS];
     if (save) {
         CK(cudaMemcpyAsync(img_age, age, (size_t)p->n, cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(img_ret, p->returns, sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(img_st, p->st, sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(img_ret, p->returns.get(), sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(img_st, p->st.get(), sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
     } else {
         CK(cudaMemcpyAsync(age, img_age, (size_t)p->n, cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(p->returns, img_ret, sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(p->st, img_st, sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(p->returns.get(), img_ret, sizeof(double) * p->n, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(p->st.get(), img_st, sizeof(PostStats), cudaMemcpyDeviceToDevice, st));
     }
     return 0;
 }
@@ -683,16 +677,15 @@ int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, voi
     const int lanes = 512 / p->D > 0 ? 512 / p->D : 1;
     const int newest = (int)((p->t - 1) % (uint32_t)p->k);
     with_width(p, [&](auto F) {
-        recompute_sums_kernel<F><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames, p->plane, p->age[p->age_cur], p->n, p->k,
-                                                                                     newest, p->st);
+        recompute_sums_kernel<F><<<blocks_for(p, p->n, lanes), lanes * p->D, 0, st>>>(p->frames.get(), p->plane, p->age[p->age_cur].get(), p->n, p->k,
+                                                                                     newest, p->st.get());
     });
     CK(cudaGetLastError());
     p->launches += 1;
-    PostStats* h = new (std::nothrow) PostStats();
+    std::unique_ptr<PostStats> h(new (std::nothrow) PostStats());
     if (!h) return fail("out of host memory");
-    cudaError_t e = cudaMemcpyAsync(h, p->st, sizeof(*h), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) { delete h; return fail("hlynr_post_check_sums: %s", cudaGetErrorString(e)); }
+    CK(cudaMemcpyAsync(h.get(), p->st.get(), sizeof(*h), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     double m = 0.0;
     for (int d = 0; d < p->k; ++d)
         for (int c = 0; c < p->fw; ++c) {
@@ -700,7 +693,6 @@ int hlynr_post_check_sums(hlynr_post_t* p, int resync, double* max_abs_diff, voi
             m = fmax(m, fabs(h->Q[d][c] - h->chk_Q[d][c]));
         }
     *max_abs_diff = m;
-    delete h;
     if (resync) {
         CK(cudaMemcpyAsync(p->st->S, p->st->chk_S, sizeof(double) * KMAX * OD, cudaMemcpyDeviceToDevice, st));
         CK(cudaMemcpyAsync(p->st->Q, p->st->chk_Q, sizeof(double) * KMAX * OD, cudaMemcpyDeviceToDevice, st));

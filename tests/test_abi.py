@@ -29,6 +29,15 @@ def test_library_loads_and_exports_everything():
     assert L.hlynr_env_state_size() == ctypes.sizeof(abi.HlynrEnvState)
 
 
+def test_info_fields_match_header():
+    """abi.INFO_FIELDS lists the members of HlynrInfoSoA in the header's order, and abi.HlynrInfoSoA has exactly those."""
+    src = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "hlynr.h")).read(), flags=re.S)
+    body = re.search(r"typedef struct HlynrInfoSoA \{(.*?)\} HlynrInfoSoA;", src, flags=re.S).group(1)
+    header = re.findall(r"\*\s*(\w+)\s*;", body)
+    assert header == [name for name, _, _ in abi.INFO_FIELDS]
+    assert [name for name, _ in abi.HlynrInfoSoA._fields_] == header
+
+
 def test_no_cpu_fallback_in_product():
     """The product package must not import, load or name the oracle."""
     pkg = os.path.join(ROOT, "hlynr_intercept_b200")
