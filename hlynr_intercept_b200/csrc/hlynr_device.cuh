@@ -43,10 +43,12 @@ HD double add(double a, double b) { return __dadd_rn(a, b); }
 HD double sub(double a, double b) { return __dsub_rn(a, b); }
 // fp64 build: a / b as a * (1 / b) with the reciprocal from rcp.approx.ftz.f64 (20 bits) + two Newton steps (80 bits -> full
 // double): ~8 instructions and no slow-path call instead of the ~30 of the correctly rounded IEEE division.  The build's contract
-// is rtol 1e-5 against the float64 reference, not bit-exactness, and the quotient is within 1-2 ulp (1e-16); the profile that
+// is rtol 1e-5 against the float64 reference, not bit-exactness, and the reciprocal and the quotient are within 1 ulp over the
+// normal range (worst measured on a B200, tests/test_device_math.py); the profile that
 // motivated it (profiles/r02_b_fp64_*) shows 3729 instructions per env-step of 165 KB straight-line code with `no_instruction`
 // (instruction-cache misses) as the top stall reason.  Every divisor on the path is positive and finite (guards are at the call
-// sites, as in the reference).  -DHLYNR_F64_EXACT_DIV restores __ddiv_rn.
+// sites, as in the reference).  Outside the normal range the ftz reciprocal is not IEEE: drcp(+-0), drcp(subnormal) and
+// drcp(+-inf) are NaN, drcp(b) is +-0 for |b| > 2^1022.  -DHLYNR_F64_EXACT_DIV restores __ddiv_rn.
 // The final product is __dmul_rn like every operation of this section: a plain `*` may be contracted with an addition that follows
 // it into an FMA, and whether the compiler does so depends on the code around the call: with a plain `*` the FT_V2OFF and the
 // generic step kernels of this build left the missile state of cfg2 different in the last bits (tests/test_kernel_variants.py).
@@ -66,7 +68,10 @@ HD double dvd(double a, double b) { return __dmul_rn(a, drcp(b)); }
 #if defined(HLYNR_F64_EXACT_DIV) || defined(HLYNR_F64_EXACT_SQRT)
 HD double sqr(double a) { return __dsqrt_rn(a); }
 #else
-HD double sqr(double a) {   // sqrt(a) = a * rsqrt(a): rsqrt.approx.ftz.f64 + two Newton steps (1-2 ulp), exact 0 for a == 0 and for denormals
+// sqrt(a) = a * rsqrt(a): rsqrt.approx.ftz.f64 + two Newton steps, within 3 ulp on [2.3e-308, DBL_MAX] (worst measured on a B200).
+// Below 2.3e-308 (zero, subnormals, the smallest normals), for negative a and for NaN it returns +0; sqr(+inf) is NaN.  The
+// arguments on the path are finite sums of squares (the state stays finite: spawns are finite and accelerations bounded or guarded).
+HD double sqr(double a) {
     double y;
     asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(a));
     const double h = 0.5 * a;
@@ -118,11 +123,13 @@ HD float ndot3(float ax, float ay, float az, float bx, float by, float bz) { ret
 HD double ndot3(double ax, double ay, double az, double bx, double by, double bz) { return dot3(ax, ay, az, bx, by, bz); }
 template <typename T> HD T nnorm3(T x, T y, T z) { return nsqrt(ndot3(x, y, z, x, y, z)); }
 HD float npow(float x, float y) { return exp2f(y * __log2f(x)); }
-HD double npow(double x, double y) { return exp(y * log(x)); }   // x > 0 on this path (temperature ratio, altitude / 10 m): within a few ulp of pow() at a third of its code
+HD double npow(double x, double y) { return exp(y * log(x)); }   // x > 0 on this path (temperature ratio, altitude / 10 m): isa_props within 11 ulp (B200) at a third of pow()'s code
 HD float nexp(float x) { return __expf(x); }
 HD double nexp(double x) { return exp(x); }
-// x / c for a constant c with rc = RN(1/c): Markstein's correction yields the correctly rounded quotient
-// in 3 instructions instead of the ~13 of an IEEE division.
+// x / c for a constant c with rc = RN(1/c): Markstein's correction in 3 instructions instead of the ~13 of an IEEE division.
+// It is not correctly rounded for every c; it is, float and double, for the constants the kernel passes (500, 100 and dt = 0.01,
+// the dt of every shipped configuration), checked on a B200 for every normal quotient (tests/test_device_math.py).  A subnormal
+// quotient may be 1 ulp off, and the quotient of -0 is +0.
 HD float cdiv(float x, float c, float rc) {
     float q = __fmul_rn(x, rc);
     float r = __fmaf_rn(-q, c, x);
@@ -138,8 +145,11 @@ HD double cdiv(double x, double c, double rc) {   // division by a constant: Mar
 #endif
 
 // atan2 / asin for the euler-angle channels obs[9:12] (core.py:1103-1121): degree-7 minimax polynomial of atan(a)/a in
-// a^2 on [0,1] (max error 1.9e-7 rad, fitted and checked in float32), one MUFU reciprocal, quadrant fix-up: ~20
-// instructions instead of the ~57 of atan2f.  The channels are observations only (they never feed the dynamics).
+// a^2 on [0,1] (1.9e-7 rad from the polynomial), one MUFU reciprocal, quadrant fix-up: ~20 instructions instead of the ~57
+// of atan2f.  Worst error measured on a B200 over all octants: 3.4e-7 rad for fast_atan2 (the final pi/2 - r, pi - r
+// roundings add to the polynomial's), 2.4e-7 rad for fast_asin.  Domain: 2^-126 <= max(|x|, |y|) < 2^126 or x = y = 0;
+// from 2^126 on the ftz reciprocal is 0 and the angle collapses (fast_atan2(1e38, 2e38) = 0), and x = -0 counts as positive.
+// The kernel's arguments have magnitude <= 2.  The channels are observations only (they never feed the dynamics).
 HD float fast_atan2(float y, float x) {
     const float ax = fabsf(x), ay = fabsf(y);
     const float mx = fmaxf(ax, ay), mn = fminf(ax, ay);
@@ -184,7 +194,7 @@ HD uint4 draw_raw(const RngKey& k, uint32_t episode, uint32_t step, uint32_t blk
 }
 HD float u01(uint32_t x) { return (float)(x >> 8) * 5.9604644775390625e-8f; }
 HD float u01_open(uint32_t x) { return (float)((x >> 8) + 1u) * 5.9604644775390625e-8f; }
-// accurate Box-Muller (reset path: domain-randomization draws, gust direction)
+// accurate Box-Muller (reset path: domain-randomization draws, gust direction): within 1.8e-7 r of float64 (B200)
 HD void box_muller(uint32_t xa, uint32_t xb, float* z0, float* z1) {
     float r = sqrtf(-2.0f * logf(u01_open(xa)));
     float s, c;
@@ -192,7 +202,11 @@ HD void box_muller(uint32_t xa, uint32_t xb, float* z0, float* z1) {
     *z0 = r * c; *z1 = r * s;
 }
 // per-tick draws: the same Box-Muller pairs evaluated with MUFU lg2/sqrt/sin/cos (absolute error ~1e-6 on a
-// standard normal, i.e. ~1e-5 m on the noisiest channel: far below every parity tolerance)
+// standard normal, i.e. ~1e-5 m on the noisiest channel: far below every parity tolerance).  Near u = 1 the absolute error
+// of __log2f (CUDA documents up to 2^-22) dominates the small radius.  Worst measured on a B200 over every radius word and
+// every angle word: |z - z_exact| <= 2.1e-6 for radii >= 0.1, and |z - z_exact| * r <= 7.5e-8 below (2.2e-4 at the smallest
+// nonzero radius, 3.5e-4).  __log2f could in principle make the square root's argument negative there; over all 2^24 radius
+// words it never does on a B200 (tests/test_device_math.py).
 HD void fast_pair(uint32_t xa, uint32_t xb, float* z0, float* z1) {
     float r = nsqrt(-1.3862943611198906f * __log2f(u01_open(xa)));  // sqrt(-2 ln u)
     float t = 2.0f * u01(xb);
@@ -481,10 +495,11 @@ template <typename R> __device__ __noinline__ Pair<R> isa_above_11km(R alt) {  /
     } else {
         R ex = sub(alt, R(20000.0));
         o.a = mul(R(216.65), nexp(ndiv(-ex, R(10000.0))));
-        o.b = mul(R(5474.889421808574), nexp(ndiv(-ex, R(6000.0))));  // get_pressure(20000.0) in python floats
+        o.b = mul(R(5474.790039909648), nexp(ndiv(-ex, R(6000.0))));  // get_pressure(20000.0) in python floats: 22632 exp(-g 9000 / (R 216.65))
     }
     return o;
 }
+// rho and cs within 1.3e-6 relative (fp32 build) / 11 ulp (fp64 build) of the float64 formula, worst measured on a B200
 template <typename R> HD void isa_props(const KParams<R>& P, R T0, R alt, R* rho, R* cs) {
     R T, Pr;
     if (alt <= R(11000.0)) {
@@ -1137,8 +1152,10 @@ __device__ __noinline__ SpawnOut spawn_values(const KernelArgs<R>& A, uint32_t c
         if (al > 1e-6) {
             // h = acos(fz) / 2 without the transcendentals: cos h = sqrt((1 + fz) / 2), sin h = sqrt((1 - fz) / 2), and the
             // cancelling one of the two comes from sin(2h) = al instead (al = |f x z| = sin(acos fz) for the unit vector f).
-            // (f is a float32 vector divided by its float32 norm, so |f| = 1 only to ~1e-7 and the two forms differ by that
-            // much: far below the fp32 build's tolerance, visible at the fp64 build's, which therefore keeps acos / sin / cos.)
+            // (f is a float32 vector divided by its float32 norm, so |f|^2 = 1 + eps with |eps| ~ 1e-7, and the two forms differ
+            // by up to about eps / (2 al): ~1e-7 in general, 2e-4 within 1e-3 rad of +-Z, where the reference's acos of a
+            // float32 fz next to +-1 is itself quantised in steps of ~3.5e-4 rad.  Below the fp32 build's tolerance, visible at
+            // the fp64 build's, which therefore keeps acos / sin / cos.)
             ax /= al; ay /= al;
             const double cz = clip(fz, -1.0, 1.0);
             double sh, ch;
@@ -1226,7 +1243,7 @@ HD void quat_step(Env<float>& e, float wx, float wy, float wz, float dt) {
     float w2 = fmaf(wz, wz, fmaf(wy, wy, wx * wx));
     float wn = nsqrt(w2);
     if (wn * dt > 1e-6f) {
-        float h = 0.5f * wn * dt, h2 = h * h;  // h <= 0.18 rad for |a| <= 1: Taylor to float accuracy
+        float h = 0.5f * wn * dt, h2 = h * h;  // h <= 0.18 rad for |a| <= 1: Taylor to float accuracy (step within 1.8e-7 of float64, B200)
         float sh = h * fmaf(h2, fmaf(h2, fmaf(h2, -1.98412698e-4f, 8.33333333e-3f), -1.66666667e-1f), 1.f);
         float ch = fmaf(h2, fmaf(h2, fmaf(h2, fmaf(h2, 2.48015873e-5f, -1.38888889e-3f), 4.16666667e-2f), -0.5f), 1.f);
         if (h > 0.5f) { const Pair<float> sc = sincos_full(h); sh = sc.a; ch = sc.b; }  // actions outside [-1,1]
